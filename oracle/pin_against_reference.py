@@ -31,6 +31,7 @@ sys.path.insert(0, ROOT)
 REF_SRC = "/root/reference/src"
 
 from oracle import kd_oracle as O  # noqa: E402
+from tests.harness import save_golden  # noqa: E402
 
 
 def load_reference():
@@ -148,11 +149,10 @@ def main():
             got = O.kd_step(params, pparams, batch, a, b, g, temp, use_refinement=refine, dtype=dtype)
             ok &= compare(f"{name}/{str(dtype)[6:]}", got, ref, tol)
             if dtype == torch.float32:
-                torch.save({"meta": dict(B=B, T=T, V=V, E=E, H=H, L=L, refinement=refine, alpha=a, beta=b,
-                                         gamma=g, temperature=temp, torch=torch.__version__,
-                                         generator="oracle/pin_against_reference.py (reference modules, fp32 CPU)"),
-                            "params": params, "proj_params": pparams, "batch": batch, "reference": ref},
-                           os.path.join(ROOT, "tests", "golden", name + ".pt"))
+                save_golden({"meta": dict(B=B, T=T, V=V, E=E, H=H, L=L, refinement=refine, alpha=a, beta=b,
+                                          gamma=g, temperature=temp, torch=torch.__version__,
+                                          generator="oracle/pin_against_reference.py (reference modules, fp32 CPU)"),
+                             "params": params, "proj_params": pparams, "batch": batch, "reference": ref}, name)
         torch.set_default_dtype(torch.float32)
 
     # ---- greedy decode: reference step methods in a batched loop + caption_image at B=1 ----

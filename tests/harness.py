@@ -2,11 +2,40 @@
 dict and replay the reference's KD step structure (src/train_student_kd.py:262-288) on a synthetic batch."""
 from __future__ import annotations
 
+import io
 import os
 
 import torch
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+GOLDEN_PART_BYTES = 900_000      # files in the repository stay below 1 MB: a larger fixture is stored in parts of this size
+
+
+def save_golden(obj, name: str) -> None:
+    """torch.save `obj` as tests/golden/<name>.pt, or, when the stream is larger than GOLDEN_PART_BYTES, as its consecutive
+    byte ranges <name>.pt.0, <name>.pt.1, ... (load_golden joins them back into the same stream)."""
+    buf = io.BytesIO()
+    torch.save(obj, buf)
+    data = buf.getvalue()
+    path = os.path.join(GOLDEN, name + ".pt")
+    chunks = [data] if len(data) <= GOLDEN_PART_BYTES else [data[i:i + GOLDEN_PART_BYTES] for i in range(0, len(data), GOLDEN_PART_BYTES)]
+    for i, chunk in enumerate(chunks):
+        with open(path if len(chunks) == 1 else f"{path}.{i}", "wb") as f:
+            f.write(chunk)
+
+
+def load_golden(name: str):
+    """The fixture save_golden wrote: tests/golden/<name>.pt, or the concatenation of its parts <name>.pt.0, .1, ..."""
+    path = os.path.join(GOLDEN, name + ".pt")
+    if os.path.exists(path):
+        return torch.load(path, weights_only=False)
+    parts = []
+    while os.path.exists(f"{path}.{len(parts)}"):
+        with open(f"{path}.{len(parts)}", "rb") as f:
+            parts.append(f.read())
+    if not parts:
+        raise FileNotFoundError(path)
+    return torch.load(io.BytesIO(b"".join(parts)), weights_only=False)
 
 
 def build_student(params, proj_params, V, E, H, L, refinement, Et, device, dropout=0.0):

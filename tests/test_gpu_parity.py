@@ -6,8 +6,8 @@ import pytest
 import torch
 
 from oracle import kd_oracle as O
-from tests.harness import (GOLDEN, autocast_reference_errors, build_student, compare_step, compare_step_calibrated, relerr, relerr_l2, run_kd_step,
-                           step_errors, to_device)
+from tests.harness import (GOLDEN, autocast_reference_errors, build_student, compare_step, compare_step_calibrated, load_golden, relerr, relerr_l2,
+                           run_kd_step, step_errors, to_device)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -21,7 +21,7 @@ GATED = ("grad:decoder.output_projection.0.weight", "grad:decoder.output_project
 
 
 def _golden_step(name, dtype):
-    g = torch.load(os.path.join(GOLDEN, name + ".pt"), weights_only=False)
+    g = load_golden(name)
     m = g["meta"]
     Et = g["batch"]["teacher_features"].shape[-1]
     model, projector = build_student(g["params"], g["proj_params"], m["V"], m["E"], m["H"], m["L"], m["refinement"], Et, DEV)
@@ -40,7 +40,7 @@ def test_kd_step_bf16_matches_reference(name):
     """bf16 mode against the reference's fp32 golden vectors: every tensor within max(2e-2, 1.2 x the error the REFERENCE's own
     arithmetic shows under torch.autocast(bf16) on the same inputs) -- no hand-set per-tensor factors."""
     got, ref = _golden_step(name, torch.bfloat16)
-    g = torch.load(os.path.join(GOLDEN, name + ".pt"), weights_only=False)
+    g = load_golden(name)
     ref_err = autocast_reference_errors(g["params"], g["proj_params"], g["meta"], g["batch"], ref, DEV, use_refinement=g["meta"]["refinement"])
     compare_step_calibrated(got, ref, ref_err, BF16_TOL)
 

@@ -7,14 +7,14 @@ import torch
 
 from oracle import kd_oracle as O
 from oracle import manual_backward as M
-from tests.harness import GOLDEN, relerr
+from tests.harness import GOLDEN, load_golden, relerr
 
 KD_CASES = ["kd_small_default", "kd_small_large_variant", "kd_small_ce_heavy_nohid"]
 
 
 @pytest.mark.parametrize("name", KD_CASES)
 def test_oracle_matches_reference_golden(name):
-    g = torch.load(os.path.join(GOLDEN, name + ".pt"), weights_only=False)
+    g = load_golden(name)
     m, ref = g["meta"], g["reference"]
     got = O.kd_step(g["params"], g["proj_params"], g["batch"], m["alpha"], m["beta"], m["gamma"], m["temperature"],
                     use_refinement=m["refinement"])
