@@ -95,6 +95,7 @@ SYMBOLS = {
     "b2c_decoder_forward_eval": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp, _vp, _vp, _vp, _sz, ctypes.c_int, _vp]),
     "b2c_decoder_forward_prepared": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _vp, _sz, ctypes.c_int, _DRP, _vp]),
     "b2c_decoder_backward": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _vp, _GRD, _vp, _vp, _sz, ctypes.c_int, _DRP, ctypes.c_int, _vp]),
+    "b2c_decoder_backward_pitched": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _GRD, _vp, _vp, _sz, ctypes.c_int, _DRP, ctypes.c_int, _vp]),
     "b2c_bump_counter": (ctypes.c_int, [_vp, _vp]),
     "b2c_debug_recur_trace": (ctypes.c_int, [_vp, _i64, _vp, _vp]),
     "b2c_join_side_work": (ctypes.c_int, [_vp]),
@@ -108,6 +109,7 @@ SYMBOLS = {
     "b2c_projector_backward": (ctypes.c_int, [_SHP, ctypes.POINTER(B2CProjParams), _vp, ctypes.POINTER(B2CProjGrads), _vp, _sz, ctypes.c_int, _DRP, _vp]),
     "b2c_count_valid": (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp]),
     "b2c_kd_token_loss": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _f, _f, _f, _vp, _vp, _vp, _vp, ctypes.c_int, _vp]),
+    "b2c_kd_token_loss_pitched": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _f, _f, _f, _vp, _vp, _i64, _vp, _vp, ctypes.c_int, _vp]),
     "b2c_kd_token_eval": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _vp, _vp, _vp, _vp, ctypes.c_int, _vp]),
     "b2c_bleu1": (ctypes.c_int, [_vp, _vp, _i32, _i32, _vp, _vp]),
     "b2c_aux_loss": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32, _i32, _f, _f, _vp, _vp, _vp, _vp, _vp, ctypes.c_int, ctypes.c_int, _vp]),
@@ -319,6 +321,18 @@ def compute_copy_of(t: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
     return t.detach().to(dtype).contiguous()
 
 
+def _pitched_rows(g: torch.Tensor, cdt: torch.dtype) -> Optional[int]:
+    """Row pitch of a (T,B,V) bf16 gradient whose rows are padded to a 16-byte pitch (strides (B*ld, ld, 1), ld % 8 == 0, ld > V,
+    16-byte aligned: the view KDLossFunction returns for V % 8 != 0), or None: then the gradient is made contiguous."""
+    if cdt != torch.bfloat16 or g.dtype != cdt or g.dim() != 3:
+        return None
+    T, B, V = g.shape
+    ld = g.stride(1)
+    if ld <= V or ld % 8 or g.stride(2) != 1 or g.stride(0) != B * ld or g.data_ptr() % 16:
+        return None
+    return ld
+
+
 class DecoderFunction(torch.autograd.Function):
     """LSTMDecoder.forward (reference src/student_model.py:205-256) as one C-ABI call each way."""
 
@@ -376,7 +390,9 @@ class DecoderFunction(torch.autograd.Function):
         cdt = f.dtype
         if dlogits is None:
             dlogits = torch.zeros(shape.T, shape.B, shape.V, dtype=cdt, device=f.device)
-        dlogits = dlogits.to(cdt).contiguous()
+        ld = _pitched_rows(dlogits, cdt)
+        if ld is None:
+            dlogits = dlogits.to(cdt).contiguous()
         if dhid is not None:
             dhid = dhid.to(cdt).contiguous()
         grads, all_direct = _grad_buffers(ctx.b2c_params, master, opts)
@@ -386,10 +402,17 @@ class DecoderFunction(torch.autograd.Function):
         dfeats = torch.empty(shape.B, shape.S, shape.E, dtype=torch.float32, device=f.device)
         prm = _fill_struct(B2CParams(), master, L)
         grd = _fill_struct(B2CGrads(), grads, L)
-        _check(lib.b2c_decoder_backward(ctypes.byref(shape), ctypes.byref(prm), f.data_ptr(), cap.data_ptr(), hid.data_ptr(), attw.data_ptr(),
-                                        dlogits.data_ptr(), _ptr(dhid), ctypes.byref(grd), dfeats.data_ptr(), ws.data_ptr(), ws.numel(),
-                                        code, ctypes.byref(drop), B2C_BWD_DEFER_JOIN if defer else 0, _stream()),
-               "b2c_decoder_backward")
+        flags = B2C_BWD_DEFER_JOIN if defer else 0
+        if ld is None:
+            _check(lib.b2c_decoder_backward(ctypes.byref(shape), ctypes.byref(prm), f.data_ptr(), cap.data_ptr(), hid.data_ptr(), attw.data_ptr(),
+                                            dlogits.data_ptr(), _ptr(dhid), ctypes.byref(grd), dfeats.data_ptr(), ws.data_ptr(), ws.numel(),
+                                            code, ctypes.byref(drop), flags, _stream()),
+                   "b2c_decoder_backward")
+        else:
+            _check(lib.b2c_decoder_backward_pitched(ctypes.byref(shape), ctypes.byref(prm), f.data_ptr(), cap.data_ptr(), hid.data_ptr(),
+                                                    attw.data_ptr(), dlogits.data_ptr(), ld, _ptr(dhid), ctypes.byref(grd), dfeats.data_ptr(),
+                                                    ws.data_ptr(), ws.numel(), code, ctypes.byref(drop), flags, _stream()),
+                   "b2c_decoder_backward_pitched")
         if defer:
             opts.join_pending = True                     # the owner of `opts` calls join_side_work() and clears this
         if opts.after_backward is not None:              # GraphedKDStep: the decoder's gradients are enqueued from here on
@@ -475,11 +498,21 @@ class KDLossFunction(torch.autograd.Function):
             nval = count_valid(tg, V)
             if group is not None:                  # data parallel: the CE normaliser is the GLOBAL non-PAD count
                 torch.distributed.all_reduce(nval, group=group)
-        dlogits = torch.empty_like(y)
         rows = torch.empty(2, N, dtype=torch.float32, device=dev)
-        _check(lib.b2c_kd_token_loss(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), float(alpha), float(w_ce),
-                                     float(ce_mult), nval.data_ptr(), dlogits.data_ptr(), rows[0].data_ptr(), rows[1].data_ptr(), code, st),
-               "b2c_kd_token_loss")
+        if cdt == torch.bfloat16 and V % 8 != 0:
+            # the logits gradient lives at row pitch Vp = roundup(V, 8) (columns V..Vp-1 written as zeros) and leaves as the (T,B,V)
+            # view: DecoderFunction.backward hands the pitch on, and the vocabulary head's backward contractions stay on tensor cores
+            Vp = (V + 7) // 8 * 8
+            dlogits_buf = torch.empty(T, B, Vp, dtype=cdt, device=dev)
+            _check(lib.b2c_kd_token_loss_pitched(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), float(alpha), float(w_ce),
+                                                 float(ce_mult), nval.data_ptr(), dlogits_buf.data_ptr(), Vp, rows[0].data_ptr(), rows[1].data_ptr(),
+                                                 code, st), "b2c_kd_token_loss_pitched")
+            dlogits = dlogits_buf[..., :V]
+        else:
+            dlogits = dlogits_buf = torch.empty_like(y)
+            _check(lib.b2c_kd_token_loss(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), float(alpha), float(w_ce),
+                                         float(ce_mult), nval.data_ptr(), dlogits.data_ptr(), rows[0].data_ptr(), rows[1].data_ptr(), code, st),
+                   "b2c_kd_token_loss")
         fs = ft = hs = ht = dfs = dft = dhs = feat_part = hid_part = None
         Ss = St = E = H = Th = 0
         fcode = code
@@ -507,7 +540,7 @@ class KDLossFunction(torch.autograd.Function):
         _check(lib.b2c_loss_finalize(rows[0].data_ptr(), rows[1].data_ptr(), N, nval.data_ptr(), float(ce_mult), _ptr(feat_part), B, E,
                                      _ptr(hid_part), Th, H, float(temperature), float(alpha), float(beta), float(gamma), float(w_ce),
                                      out5.data_ptr(), st), "b2c_loss_finalize")
-        ctx.b2c = dict(dlogits=dlogits, dfs=dfs, dft=dft, dhs=dhs, code=code, used=False, unit_grad=bool(unit_grad),
+        ctx.b2c = dict(dlogits=dlogits, dlogits_buf=dlogits_buf, dfs=dfs, dft=dft, dhs=dhs, code=code, used=False, unit_grad=bool(unit_grad),
                        dtypes=(logits.dtype, None if feats_s is None else feats_s.dtype,
                                None if feats_t is None else feats_t.dtype, None if hid_s is None else hid_s.dtype))
         ctx.mark_non_differentiable(out5)
@@ -523,7 +556,8 @@ class KDLossFunction(torch.autograd.Function):
         if not sv["unit_grad"]:          # unit_grad: the caller guarantees loss.backward() with grad_output == 1 (GraphedKDStep)
             scale = grad_loss.detach().to(torch.float32).reshape(1).contiguous()
             st = _stream()
-            for key, code in (("dlogits", sv["code"]), ("dfs", B2C_F32), ("dft", B2C_F32), ("dhs", sv["code"])):
+            # the whole padded buffer: its padding columns are zeros and stay zeros
+            for key, code in (("dlogits_buf", sv["code"]), ("dfs", B2C_F32), ("dft", B2C_F32), ("dhs", sv["code"])):
                 t = sv[key]
                 if t is not None:
                     _check(lib.b2c_scale_inplace(t.data_ptr(), t.numel(), code, scale.data_ptr(), st), "b2c_scale_inplace")

@@ -233,6 +233,16 @@ int colsum(cudaStream_t st, const T* A, long rows, int cols, long ld, float* par
     B2C_LAUNCH_CHECK("colsum_final_kernel");
     return 0;
   }
+  if (ld != cols && ld % 8 == 0 && cols <= ld && ((uintptr_t)A & 15) == 0 && rows >= 256) {
+    // pitched 16-byte rows (the padded logits gradient): the same vectorised read, padding columns summed but not written
+    const int gx = cdiv(cols, 256);
+    int rs = (int)((rows + 31) / 32); if (rs > 592 / gx) rs = 592 / gx; if (rs > COLSUM_RS) rs = COLSUM_RS; if (rs < 1) rs = 1;
+    colsum_vec_pitched_kernel<T><<<dim3(gx, rs), 256, 0, st>>>(A, rows, cols, ld, partial);
+    B2C_LAUNCH_CHECK("colsum_vec_pitched_kernel");
+    colsum_final_kernel<<<cdiv(cols, 256), 256, 0, st>>>(partial, rs, cols, out, out2, unperm_h);
+    B2C_LAUNCH_CHECK("colsum_final_kernel");
+    return 0;
+  }
   int rs = (int)((rows + 255) / 256); if (rs > COLSUM_RS) rs = COLSUM_RS; if (rs < 1) rs = 1;
   colsum_partial_kernel<T><<<dim3(cdiv(cols, 32), rs), 256, 0, st>>>(A, rows, cols, ld, partial);
   B2C_LAUNCH_CHECK("colsum_partial_kernel");
@@ -576,12 +586,13 @@ inline int wgrad_chunks() { static int v = -1; if (v < 0) { const char* e = gete
 template <typename T>
 int decoder_backward_impl(const B2CShape& s, const B2CParams& p, const T* feats, const int64_t* cap, const T* hid_top,
                           const float* attw, const T* dlogits, const T* dhid, const B2CGrads& g, float* dfeats,
-                          void* ws, size_t ws_bytes, const B2CDropout& dr, cudaStream_t st, int flags) {
+                          void* ws, size_t ws_bytes, const B2CDropout& dr, cudaStream_t st, int flags, long ld_dl = 0 /* 0 = V */) {
   TrainWs<T> W; W.carve(ws, s);
   B2C_CHECK_ARG(ws_bytes >= W.bytes, "workspace too small: %zu < %zu", ws_bytes, W.bytes);
   B2C_CHECK_ARG(g.embedding && g.attn_w && g.attn_b && g.comb_w && g.comb_b && g.out0_w && g.out0_b && g.out3_w && g.out3_b && dfeats, "NULL gradient pointer");
   const int B = s.B, Tn = s.T, S = s.S, E = s.E, H = s.H, L = s.L, V = s.V;
   const long TB = (long)Tn * B;
+  if (ld_dl == 0) ld_dl = V;
   const float inv_keep = dr.p > 0.f ? 1.0f / (1.0f - dr.p) : 1.0f;
   SubStreams* hs = nullptr;
   B2C_TRY(get_substreams(&hs));
@@ -596,15 +607,15 @@ int decoder_backward_impl(const B2CShape& s, const B2CParams& p, const T* feats,
   B2C_CUDA(cudaEventRecord(hs->ev[3], side));
   // ---- output head (time-batched).  Only d(o1) -> dH_ext feeds the time loop; the head's weight gradients run on a side
   // stream underneath the (latency-bound) recurrence and are joined after it.
-  B2C_TRY((gemm<T, T>(st, (int)TB, E, V, dlogits, V, 0, W.w.W2, E, 1, W.do1, E)));
+  B2C_TRY((gemm<T, T>(st, (int)TB, E, V, dlogits, ld_dl, 0, W.w.W2, E, 1, W.do1, E)));
   relu_bwd_inplace_kernel<T><<<ew_grid(TB * E), 256, 0, st>>>(W.do1, W.o1, TB * E, inv_keep);
   B2C_LAUNCH_CHECK("relu_bwd_inplace_kernel");
   B2C_CUDA(cudaEventRecord(hs->fork, st));
   B2C_CUDA(cudaStreamWaitEvent(side, hs->fork, 0));
   {
     GemmCapScope bg(bg_ctas());          // these run under the reverse recurrence: confined to the SMs the chain leaves free
-    B2C_TRY((gemm<T, float>(side, V, E, (int)TB, dlogits, V, 1, W.o1, E, 1, g.out3_w, E)));
-    B2C_TRY(colsum<T>(side, dlogits, TB, V, V, W.partial_side, g.out3_b));
+    B2C_TRY((gemm<T, float>(side, V, E, (int)TB, dlogits, ld_dl, 1, W.o1, E, 1, g.out3_w, E)));
+    B2C_TRY(colsum<T>(side, dlogits, TB, V, ld_dl, W.partial_side, g.out3_b));
     B2C_TRY((gemm<T, float>(side, E, H, (int)TB, W.do1, E, 1, hid_top, H, 1, g.out0_w, H)));
     B2C_TRY(colsum<T>(side, W.do1, TB, E, E, W.partial_side, g.out0_b));
   }
@@ -1067,9 +1078,11 @@ int projector_backward_impl(const B2CShape& s, const B2CProjParams& p, const flo
 
 template <typename TS>
 int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, int V, float temperature, float alpha,
-                       float w_ce_eff, const int* n_valid, TS* dy, float* row_kl, float* row_ce, cudaStream_t st, int* argmax_out = nullptr) {
+                       float w_ce_eff, const int* n_valid, TS* dy, float* row_kl, float* row_ce, cudaStream_t st, int* argmax_out = nullptr,
+                       long ld = 0 /* dy pitch; 0 = V */) {
+  if (ld == 0) ld = V;
   const bool eval = (dy == nullptr) || (argmax_out != nullptr);      // losses only (+ predictions): the row-in-smem kernel
-  const bool vec = (V % 8 == 0) && ((uintptr_t)y % 16 == 0) && ((uintptr_t)z % 16 == 0) && ((uintptr_t)dy % 16 == 0);
+  const bool vec = (V % 8 == 0) && (ld == V) && ((uintptr_t)y % 16 == 0) && ((uintptr_t)z % 16 == 0) && ((uintptr_t)dy % 16 == 0);
   const bool t4 = (temperature == 4.0f);
   const size_t smem = align_up((size_t)V * 4, 16) + align_up((size_t)V * sizeof(TS), 16);
   const float inv_temp = 1.0f / temperature, kd_coef = alpha * temperature / (float)N;
@@ -1096,6 +1109,34 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
     B2C_LAUNCH_CHECK("kd_token_loss_pipe_kernel");
     return 0;
   }
+  // bf16 rows of any length / alignment with a 16-byte-aligned dy of pitch ld % 8 == 0: the same pipeline on the rows'
+  // enclosing 16-byte ranges (slot = the ranges plus one word of read-ahead)
+  const int Vp = (V + 7) & ~7;
+  const size_t usmem = 2 * ((size_t)(Vp + 4) * 4 + (size_t)(Vp + 8) * sizeof(TS));
+  if constexpr (sizeof(TS) == 2) if (!vec && !eval && ld % 8 == 0 && ld >= Vp && (uintptr_t)dy % 16 == 0 && V <= 8 * KDR_THREADS * 8 && usmem <= 200 * 1024) {
+    const int need = cdiv(Vp / 8, KDR_THREADS);
+    int per_sm = (int)((200 * 1024) / (usmem + 1024)); if (per_sm < 1) per_sm = 1;
+    const int reg_cap = need <= 3 ? 3 : (need <= 5 ? 2 : 1);
+    if (per_sm > reg_cap) per_sm = reg_cap;
+    long grid = (long)sm_count() * per_sm; if (grid > N) grid = N;
+    const bf16* yb = reinterpret_cast<const bf16*>(y);
+    bf16* dyb = reinterpret_cast<bf16*>(dy);
+#define B2C_KDU(NCH, T4)                                                                                                   \
+  do {                                                                                                                     \
+    B2C_TRY(set_smem(kd_token_loss_pipe_unaligned_kernel<NCH, T4>, usmem));                                                \
+    kd_token_loss_pipe_unaligned_kernel<NCH, T4><<<(unsigned)grid, KDR_THREADS, usmem, st>>>(yb, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce_eff, n_valid, dyb, row_kl, row_ce); \
+  } while (0)
+#define B2C_KDU2(NCH) do { if (t4) B2C_KDU(NCH, true); else B2C_KDU(NCH, false); } while (0)
+    switch (need) {
+      case 1: B2C_KDU2(1); break; case 2: B2C_KDU2(2); break; case 3: B2C_KDU2(3); break; case 4: B2C_KDU2(4); break;
+      case 5: B2C_KDU2(5); break; case 6: B2C_KDU2(6); break; case 7: B2C_KDU2(7); break; default: B2C_KDU2(8); break;
+    }
+#undef B2C_KDU2
+#undef B2C_KDU
+    B2C_LAUNCH_CHECK("kd_token_loss_pipe_unaligned_kernel");
+    return 0;
+  }
+  B2C_CHECK_ARG(ld == V, "dlogits pitch %ld != V=%d needs bf16, a 16-byte-aligned dlogits with pitch %% 8 == 0 and >= roundup(V, 8), and V <= 16384", ld, V);
 #define B2C_KD_LAUNCH(G, T4)                                                                                             \
   do {                                                                                                                   \
     B2C_TRY(set_smem(kd_token_loss_kernel<TS, G, T4>, smem));                                                            \
@@ -1227,6 +1268,20 @@ int b2c_decoder_backward(const B2CShape* shape, const B2CParams* params, const v
   return set_err(B2C_EINVAL, "bad dtype %d", dtype);
 }
 
+int b2c_decoder_backward_pitched(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                                 const void* hidden_top, const float* attn_w, const void* dlogits, int64_t ld_dlogits, const void* dhidden_top,
+                                 const B2CGrads* grads, float* dfeats, void* workspace, size_t ws_bytes,
+                                 int dtype, const B2CDropout* dropout, int flags, void* stream) {
+  B2C_TRY(check_shape(shape)); B2C_TRY(check_device());
+  B2C_CHECK_ARG(params && feats && captions && hidden_top && attn_w && dlogits && grads && workspace, "NULL argument");
+  B2C_CHECK_ARG(ld_dlogits >= shape->V, "ld_dlogits=%ld < V=%d", (long)ld_dlogits, shape->V);
+  const B2CDropout dr = dropout ? *dropout : B2CDropout{0.f, 0, nullptr};
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == B2C_F32) return decoder_backward_impl<float>(*shape, *params, (const float*)feats, captions, (const float*)hidden_top, attn_w, (const float*)dlogits, (const float*)dhidden_top, *grads, dfeats, workspace, ws_bytes, dr, st, flags, (long)ld_dlogits);
+  if (dtype == B2C_BF16) return decoder_backward_impl<bf16>(*shape, *params, (const bf16*)feats, captions, (const bf16*)hidden_top, attn_w, (const bf16*)dlogits, (const bf16*)dhidden_top, *grads, dfeats, workspace, ws_bytes, dr, st, flags, (long)ld_dlogits);
+  return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+}
+
 int b2c_debug_recur_trace(uint64_t* out_host, int64_t n, int32_t* grid_out, int32_t* steps_out) {
   RecurTrace& t = recur_trace_state();
   B2C_CHECK_ARG(t.dev != nullptr && out_host && n > 0, "no trace recorded (set B2C_RECUR_TRACE=1 before the first forward)");
@@ -1355,6 +1410,19 @@ int b2c_kd_token_loss(const void* student_logits, const float* teacher_logits, c
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == B2C_F32) return kd_token_loss_impl<float>((const float*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (float*)dlogits, row_kl, row_ce, st);
   if (dtype == B2C_BF16) return kd_token_loss_impl<bf16>((const bf16*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (bf16*)dlogits, row_kl, row_ce, st);
+  return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+}
+
+int b2c_kd_token_loss_pitched(const void* student_logits, const float* teacher_logits, const int64_t* targets,
+                              int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
+                              const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype, void* stream) {
+  B2C_TRY(check_device());
+  B2C_CHECK_ARG(student_logits && teacher_logits && targets && n_valid && dlogits && row_kl && row_ce, "NULL argument");
+  B2C_CHECK_ARG(N > 0 && N < 2147483647L && V > 1 && temperature > 0.f, "bad N=%ld V=%d temperature=%f", (long)N, V, temperature);
+  B2C_CHECK_ARG(ld_dlogits >= V, "ld_dlogits=%ld < V=%d", (long)ld_dlogits, V);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == B2C_F32) return kd_token_loss_impl<float>((const float*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (float*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits);
+  if (dtype == B2C_BF16) return kd_token_loss_impl<bf16>((const bf16*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (bf16*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits);
   return set_err(B2C_EINVAL, "bad dtype %d", dtype);
 }
 

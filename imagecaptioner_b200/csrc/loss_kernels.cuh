@@ -243,24 +243,78 @@ template <> struct RowS<float> {
 };
 
 constexpr int KD_SLOTS = 2;              // row slots per CTA: the TMA prefetch runs KD_SLOTS - 1 rows ahead of the math
-template <typename TS, int NCH, bool TEMP4>
-__global__ void __launch_bounds__(KDR_THREADS, (NCH <= 3 ? 3 : (NCH <= 5 ? 2 : 1)))
-kd_token_loss_pipe_kernel(const TS* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
-                          long N, int V, float inv_temp, float temperature, float kd_coef, float w_ce, const int* __restrict__ n_valid_ptr,
-                          TS* __restrict__ dy, float* __restrict__ row_kl, float* __restrict__ row_ce) {
+
+// Unaligned rows (V % 8 != 0): row r of y / z starts anywhere inside a 16-byte word.  The bulk copy takes the enclosing
+// 16-byte-aligned byte range, so element v of the row sits at slot index sh + v with sh = the row start's offset inside its
+// word (0..7 bf16, 0..3 fp32).  These rebuild the 8 elements of column group g from the two (bf16) or three (fp32) 16-byte
+// words that hold them; the shift is uniform over the CTA, so the selects below never diverge.
+__device__ __forceinline__ uint32_t pick_word(const uint32_t (&u)[8], int q, int j) {      // u[q + j], q in 0..3
+  return q == 0 ? u[j] : (q == 1 ? u[j + 1] : (q == 2 ? u[j + 2] : u[j + 3]));
+}
+__device__ __forceinline__ void load_shifted_bf16(const bf16* slot, int sh, int g, float (&v)[8]) {
+  const uint4 a = reinterpret_cast<const uint4*>(slot)[g], b = reinterpret_cast<const uint4*>(slot)[g + 1];
+  const uint32_t u[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+  const int q = sh >> 1, bits = (sh & 1) * 16;
+  uint32_t w[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) w[j] = __funnelshift_r(pick_word(u, q, j), pick_word(u, q, j + 1), bits);
+#pragma unroll
+  for (int j = 0; j < 4; ++j) { v[2 * j] = bf16_lo(w[j]); v[2 * j + 1] = bf16_hi(w[j]); }
+}
+__device__ __forceinline__ void load_shifted_f32(const float* slot, int sh, int g, float (&v)[8]) {
+  const float4 a = reinterpret_cast<const float4*>(slot)[2 * g], b = reinterpret_cast<const float4*>(slot)[2 * g + 1],
+               c = reinterpret_cast<const float4*>(slot)[2 * g + 2];
+  const float f[12] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w};
+#pragma unroll
+  for (int k = 0; k < 8; ++k) v[k] = sh == 0 ? f[k] : (sh == 1 ? f[k + 1] : (sh == 2 ? f[k + 2] : f[k + 3]));
+}
+
+// Body of kernel (3)'s default form.  UNALIGNED = false: V % 8 == 0, 16-byte aligned y / z / dy, dy pitch V (ld == V).
+// UNALIGNED = true (bf16 student logits, any V): y and z keep pitch V and any alignment; each row is fetched by bulk copies of
+// its enclosing 16-byte-aligned ranges, except a row whose enclosing range would reach outside [y, y + N*V) or [z, z + N*V)
+// (the first / last row or two): that one is read with guarded plain loads.  Columns >= V are left out of the maxima, the
+// sums and the CE term.  dy has pitch ld (ld % 8 == 0, 16-byte aligned): 16-byte stores, columns V..roundup(V,8)-1 written
+// as exact zeros.
+template <typename TS, int NCH, bool TEMP4, bool UNALIGNED>
+__device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
+                                                   long N, int V, long ld, float inv_temp, float temperature, float kd_coef, float w_ce,
+                                                   const int* __restrict__ n_valid_ptr, TS* __restrict__ dy, float* __restrict__ row_kl,
+                                                   float* __restrict__ row_ce) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ __align__(8) uint64_t full_bar[KD_SLOTS];
   __shared__ float scratch[KDR_THREADS / 32 * 4];
-  const size_t zbytes = (size_t)V * 4, ybytes = (size_t)V * sizeof(TS), slot = zbytes + ybytes;    // both multiples of 16
+  const int Vp = (V + 7) & ~7;
+  // slot bytes: both multiples of 16; the unaligned form holds the enclosing ranges plus the word the last group reads past them
+  const size_t zbytes = UNALIGNED ? (size_t)(Vp + 4) * 4 : (size_t)V * 4;
+  const size_t ybytes = UNALIGNED ? (size_t)(Vp + 8) * sizeof(TS) : (size_t)V * sizeof(TS);
+  const size_t slot = zbytes + ybytes;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int groups = V >> 3;
+  const int groups = UNALIGNED ? (Vp >> 3) : (V >> 3);
   const int n_valid = *n_valid_ptr;
+  const uintptr_t y_end = (uintptr_t)(y + N * (long)V), z_end = (uintptr_t)(z + N * (long)V);
+  // enclosing 16-byte range [lo, hi) of row `row` of y / z, and whether both lie inside their tensors
+  auto y_lo = [&](long row) { return (uintptr_t)(y + row * (long)V) & ~(uintptr_t)15; };
+  auto z_lo = [&](long row) { return (uintptr_t)(z + row * (long)V) & ~(uintptr_t)15; };
+  auto y_hi = [&](long row) { return ((uintptr_t)(y + (row + 1) * (long)V) + 15) & ~(uintptr_t)15; };
+  auto z_hi = [&](long row) { return ((uintptr_t)(z + (row + 1) * (long)V) + 15) & ~(uintptr_t)15; };
+  auto bulk_row = [&](long row) {
+    return !UNALIGNED || (y_lo(row) >= (uintptr_t)y && y_hi(row) <= y_end && z_lo(row) >= (uintptr_t)z && z_hi(row) <= z_end);
+  };
 
   auto issue = [&](long row, int sidx) {       // thread 0 only
     unsigned char* dst = smem_raw + (size_t)sidx * slot;
-    mbar_arrive_expect_tx(&full_bar[sidx], (uint32_t)slot);
-    bulk_g2s(dst, z + row * (long)V, (uint32_t)zbytes, &full_bar[sidx]);
-    bulk_g2s(dst + zbytes, y + row * (long)V, (uint32_t)ybytes, &full_bar[sidx]);
+    if constexpr (!UNALIGNED) {
+      mbar_arrive_expect_tx(&full_bar[sidx], (uint32_t)slot);
+      bulk_g2s(dst, z + row * (long)V, (uint32_t)zbytes, &full_bar[sidx]);
+      bulk_g2s(dst + zbytes, y + row * (long)V, (uint32_t)ybytes, &full_bar[sidx]);
+    } else if (bulk_row(row)) {
+      const uint32_t zb = (uint32_t)(z_hi(row) - z_lo(row)), yb = (uint32_t)(y_hi(row) - y_lo(row));
+      mbar_arrive_expect_tx(&full_bar[sidx], zb + yb);
+      bulk_g2s(dst, (const void*)z_lo(row), zb, &full_bar[sidx]);
+      bulk_g2s(dst + zbytes, (const void*)y_lo(row), yb, &full_bar[sidx]);
+    } else {
+      mbar_arrive(&full_bar[sidx]);            // guarded row: nothing to copy, but the slot's phase still completes
+    }
   };
   if (tid == 0) { for (int i = 0; i < KD_SLOTS; ++i) mbar_init(&full_bar[i], 1); fence_barrier_init(); }
   __syncthreads();
@@ -276,15 +330,58 @@ kd_token_loss_pipe_kernel(const TS* __restrict__ y, const float* __restrict__ z,
     const TS* ys = reinterpret_cast<const TS*>(smem_raw + (size_t)sidx * slot + zbytes);
     mbar_wait(&full_bar[sidx], ph);
     float yv[NCH][8], zv[NCH][8];
+    bool bulk = true;
+    int sy = 0, sz = 0;
+    if constexpr (!UNALIGNED) {
 #pragma unroll
-    for (int i = 0; i < NCH; ++i) {
-      const int g = tid + i * KDR_THREADS;
-      if (i < NCH - 1 || g < groups) { RowS<TS>::load(ys + g * 8, yv[i]); RowS<float>::load(zs + g * 8, zv[i]); }
+      for (int i = 0; i < NCH; ++i) {
+        const int g = tid + i * KDR_THREADS;
+        if (i < NCH - 1 || g < groups) { RowS<TS>::load(ys + g * 8, yv[i]); RowS<float>::load(zs + g * 8, zv[i]); }
+      }
+    } else {
+      const TS* yr = y + r * (long)V;
+      const float* zr = z + r * (long)V;
+      bulk = bulk_row(r);
+      if (bulk) {
+        sy = (int)(((uintptr_t)yr & 15) / sizeof(TS)); sz = (int)(((uintptr_t)zr & 15) >> 2);
+#pragma unroll
+        for (int i = 0; i < NCH; ++i) {
+          const int g = tid + i * KDR_THREADS;
+          if (i < NCH - 1 || g < groups) { load_shifted_bf16(ys, sy, g, yv[i]); load_shifted_f32(zs, sz, g, zv[i]); }
+        }
+      } else {
+#pragma unroll
+        for (int i = 0; i < NCH; ++i) {
+          const int g = tid + i * KDR_THREADS;
+          if (i < NCH - 1 || g < groups) {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+              const int c = g * 8 + j;
+              yv[i][j] = c < V ? to_f<TS>(yr[c]) : 0.f; zv[i][j] = c < V ? zr[c] : 0.f;
+            }
+          }
+        }
+      }
+      // columns V..Vp-1 (the last group only) hold a neighbouring row or nothing.  A finite sentinel far below any logit keeps
+      // them out of the maxima and gives them e^x = 0 in every sum (and a gradient of exactly 0) without a branch per element;
+      // unlike -inf it never forms inf - inf in the KL term, and (x - max) / Temp stays finite for any Temp > 1e-8.
+#pragma unroll
+      for (int i = 0; i < NCH; ++i) {
+        const int g = tid + i * KDR_THREADS;
+        if (g == groups - 1) {
+#pragma unroll
+          for (int j = 0; j < 8; ++j) if (g * 8 + j >= V) { yv[i][j] = -1.0e30f; zv[i][j] = -1.0e30f; }
+        }
+      }
     }
     const long t64 = tgt[r];
     const bool valid = (t64 > 0) && (t64 < V);
     const int t_idx = valid ? (int)t64 : -1;
-    const float y_tgt = valid ? to_f<TS>(ys[t_idx]) : 0.f, z_tgt = valid ? zs[t_idx] : 0.f;
+    float y_tgt = 0.f, z_tgt = 0.f;
+    if (valid) {
+      if (bulk) { y_tgt = to_f<TS>(ys[sy + t_idx]); z_tgt = zs[sz + t_idx]; }
+      else { y_tgt = to_f<TS>(y[r * (long)V + t_idx]); z_tgt = z[r * (long)V + t_idx]; }
+    }
     __syncthreads();                           // every thread has taken its groups out of the slot ...
     if (tid == 0 && r + KD_SLOTS * stride < N) issue(r + KD_SLOTS * stride, sidx);      // ... so a later row can land in it
 
@@ -341,7 +438,7 @@ kd_token_loss_pipe_kernel(const TS* __restrict__ y, const float* __restrict__ z,
 
     // phase 3: gradient, straight from registers to 128-bit streaming stores.  The one-hot term of the target logit is
     // applied by the thread that owns that logit with one scalar store after its vector store (same thread, same address).
-    TS* dyg = dy + r * (long)V;
+    TS* dyg = dy + r * ld;
     const float a_s = kd_coef * inv_sT, a_t = -kd_coef * inv_sZ, a_c = ce_coef * inv_s1;
     const int t_grp = t_idx >> 3;               // -1 on PAD rows: matches no group
     float g_t = 0.f;
@@ -368,6 +465,24 @@ kd_token_loss_pipe_kernel(const TS* __restrict__ y, const float* __restrict__ z,
       }
     }
   }
+}
+
+template <typename TS, int NCH, bool TEMP4>
+__global__ void __launch_bounds__(KDR_THREADS, (NCH <= 3 ? 3 : (NCH <= 5 ? 2 : 1)))
+kd_token_loss_pipe_kernel(const TS* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
+                          long N, int V, float inv_temp, float temperature, float kd_coef, float w_ce, const int* __restrict__ n_valid_ptr,
+                          TS* __restrict__ dy, float* __restrict__ row_kl, float* __restrict__ row_ce) {
+  kd_token_pipe_body<TS, NCH, TEMP4, false>(y, z, tgt, N, V, V, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce);
+}
+
+// The form for bf16 rows of any length (V % 8 != 0 or unaligned logits) with dlogits of pitch ld (ld % 8 == 0).
+template <int NCH, bool TEMP4>
+__global__ void __launch_bounds__(KDR_THREADS, (NCH <= 3 ? 3 : (NCH <= 5 ? 2 : 1)))
+kd_token_loss_pipe_unaligned_kernel(const bf16* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
+                                    long N, int V, long ld, float inv_temp, float temperature, float kd_coef, float w_ce,
+                                    const int* __restrict__ n_valid_ptr, bf16* __restrict__ dy, float* __restrict__ row_kl,
+                                    float* __restrict__ row_ce) {
+  kd_token_pipe_body<bf16, NCH, TEMP4, true>(y, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce);
 }
 
 // validate_student_model's monitoring metric (reference src/distillation_utils.py:398-409, compute_bleu_score): per sample,

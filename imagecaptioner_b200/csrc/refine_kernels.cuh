@@ -254,14 +254,16 @@ __global__ void __launch_bounds__(256) ln_param_grad_kernel(const float* __restr
 }
 
 // ------------------------------------------------------------------ column sums (bias gradients), optionally fused with the ReLU backward
-// A is (rows, cols), cols % 8 == 0.  Block = 32 chunk lanes x 8 row lanes: a warp reads 32 consecutive 8-element chunks of one row.
+// A is (rows, cols) with pitch ld, ld % 8 == 0 and cols <= ld; nch = ceil(cols / 8).  Block = 32 chunk lanes x 8 row lanes: a warp
+// reads 32 consecutive 8-element chunks of one row.  Columns cols..8*nch-1 of the last chunk are read (they lie inside the pitch)
+// and summed, but never written to `partial`.
 // RELU_BWD: d <- act > 0 ? d * inv_keep : 0 is applied in place first (act = the saved post-ReLU / post-dropout activation).
 template <typename T, bool RELU_BWD>
-__global__ void __launch_bounds__(256)
-colsum_vec_kernel(T* __restrict__ A, const T* __restrict__ act, long rows, int cols, float inv_keep, float* __restrict__ partial) {
+__device__ __forceinline__ void colsum_vec_body(T* __restrict__ A, const T* __restrict__ act, long rows, int cols, long ld, int nch,
+                                                float inv_keep, float* __restrict__ partial) {
   __shared__ float red[8][32 * 8 + 8];
   const int lane = threadIdx.x & 31, ry = threadIdx.x >> 5;
-  const int ch = blockIdx.x * 32 + lane, nch = cols >> 3;
+  const int ch = blockIdx.x * 32 + lane;
   const long per = (rows + gridDim.y - 1) / gridDim.y;
   const long r0 = (long)blockIdx.y * per, r1 = (r0 + per < rows) ? r0 + per : rows;
   float acc[8];
@@ -274,16 +276,16 @@ colsum_vec_kernel(T* __restrict__ A, const T* __restrict__ act, long rows, int c
     for (; r + 24 < r1; r += 32) {
       float v[4][8];
 #pragma unroll
-      for (int u = 0; u < 4; ++u) Vec8<T>::load(A + (r + 8 * u) * cols + ch * 8, v[u]);
+      for (int u = 0; u < 4; ++u) Vec8<T>::load(A + (r + 8 * u) * ld + ch * 8, v[u]);
       if (RELU_BWD) {
         float a[4][8];
 #pragma unroll
-        for (int u = 0; u < 4; ++u) Vec8<T>::load(act + (r + 8 * u) * cols + ch * 8, a[u]);
+        for (int u = 0; u < 4; ++u) Vec8<T>::load(act + (r + 8 * u) * ld + ch * 8, a[u]);
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
 #pragma unroll
           for (int j = 0; j < 8; ++j) v[u][j] = a[u][j] > 0.f ? v[u][j] * inv_keep : 0.f;
-          Vec8<T>::store(A + (r + 8 * u) * cols + ch * 8, v[u]);
+          Vec8<T>::store(A + (r + 8 * u) * ld + ch * 8, v[u]);
         }
       }
 #pragma unroll
@@ -293,12 +295,12 @@ colsum_vec_kernel(T* __restrict__ A, const T* __restrict__ act, long rows, int c
     }
     for (; r < r1; r += 8) {
       float v[8];
-      Vec8<T>::load(A + r * cols + ch * 8, v);
+      Vec8<T>::load(A + r * ld + ch * 8, v);
       if (RELU_BWD) {
-        float a[8]; Vec8<T>::load(act + r * cols + ch * 8, a);
+        float a[8]; Vec8<T>::load(act + r * ld + ch * 8, a);
 #pragma unroll
         for (int j = 0; j < 8; ++j) v[j] = a[j] > 0.f ? v[j] * inv_keep : 0.f;
-        Vec8<T>::store(A + r * cols + ch * 8, v);
+        Vec8<T>::store(A + r * ld + ch * 8, v);
       }
 #pragma unroll
       for (int j = 0; j < 8; ++j) acc[j] += v[j];
@@ -315,6 +317,17 @@ colsum_vec_kernel(T* __restrict__ A, const T* __restrict__ act, long rows, int c
     for (int i = 0; i < 8; ++i) sres += red[i][t];
     partial[(long)blockIdx.y * cols + col] = sres;
   }
+}
+template <typename T, bool RELU_BWD>
+__global__ void __launch_bounds__(256)
+colsum_vec_kernel(T* __restrict__ A, const T* __restrict__ act, long rows, int cols, float inv_keep, float* __restrict__ partial) {
+  colsum_vec_body<T, RELU_BWD>(A, act, rows, cols, cols, cols >> 3, inv_keep, partial);     // contiguous, cols % 8 == 0
+}
+// column sums of a pitched matrix (e.g. the logits gradient with its row pitch rounded up to 8 elements)
+template <typename T>
+__global__ void __launch_bounds__(256)
+colsum_vec_pitched_kernel(const T* __restrict__ A, long rows, int cols, long ld, float* __restrict__ partial) {
+  colsum_vec_body<T, false>(const_cast<T*>(A), (const T*)nullptr, rows, cols, ld, (cols + 7) >> 3, 1.f, partial);
 }
 
 // ------------------------------------------------------------------ multi-head self-attention core over S tokens (S = 49), one CTA per (sample, head)

@@ -244,9 +244,9 @@ class CaptioningStudent(nn.Module):
         return outputs, encoder_features, hidden_states, attention_weights
 
     def supports_fused_validation(self) -> bool:
-        """The logits-free validation forward exists in bf16 mode (autocast, or decoder.compute_dtype = bfloat16) for vocabularies
-        TMA can describe (V % 8 == 0)."""
-        return self.decoder._mode() == torch.bfloat16 and self.vocab_size % 8 == 0
+        """The logits-free validation forward exists in bf16 mode (autocast, or decoder.compute_dtype = bfloat16), for any vocabulary
+        size (the epilogue reads teacher rows that do not start on a 16-byte boundary with plain loads)."""
+        return self.decoder._mode() == torch.bfloat16
 
     @torch.no_grad()
     def forward_validation(self, images, captions, teacher_logits, targets, temperature):

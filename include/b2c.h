@@ -16,6 +16,7 @@
  *   b2c_projector_forward/backward  <- FeatureProjector.forward (+ autograd)      src/distillation_utils.py:203-252
  *   b2c_count_valid       <- CrossEntropyLoss(ignore_index=0) normaliser  src/distillation_utils.py:22
  *   b2c_kd_token_loss     <- token_level_distillation :30-54 + CE term :154 (+ their gradient)
+ *   b2c_kd_token_loss_pitched / b2c_decoder_backward_pitched <- the same two calls with the logits gradient at a padded row pitch
  *   b2c_kd_token_eval     <- validate_student_model: loss without gradients + logits.argmax(-1)   src/train_student_kd.py:29-86
  *   b2c_bleu1             <- compute_bleu_score (per sample, on the device)                       src/distillation_utils.py:398-409
  *   b2c_aux_loss          <- encoder_feature_distillation :56-94 + decoder_hidden_state_distillation :96-136
@@ -144,6 +145,15 @@ int b2c_decoder_backward(const B2CShape* shape, const B2CParams* params, const v
                          const B2CGrads* grads, float* dfeats, void* workspace, size_t ws_bytes,
                          int dtype, const B2CDropout* dropout, int flags, void* stream);
 
+/* b2c_decoder_backward with the logits gradient at row pitch ld_dlogits >= V (elements): row r of dlogits starts at
+ * dlogits + r * ld_dlogits, and only its first V columns are read.  The caller owns the buffer.  In bf16 mode a pitch with
+ * ld_dlogits % 8 == 0 and a 16-byte-aligned dlogits lets the vocabulary head's data-gradient and weight-gradient contractions
+ * run on tensor cores for any V (TMA needs 16-byte row pitches); with ld_dlogits == V this is b2c_decoder_backward. */
+int b2c_decoder_backward_pitched(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                                 const void* hidden_top, const float* attn_w, const void* dlogits, int64_t ld_dlogits, const void* dhidden_top,
+                                 const B2CGrads* grads, float* dfeats, void* workspace, size_t ws_bytes,
+                                 int dtype, const B2CDropout* dropout, int flags, void* stream);
+
 /* b2c_decoder_backward contracts every weight gradient on an internal (per-device) side stream next to the chain that produces
  * dfeats, and by default makes `stream` wait for that branch before it returns ("all work is enqueued on stream").  A caller that
  * does not read parameter gradients until later (an optimizer step after the rest of the backward) passes
@@ -216,6 +226,16 @@ int b2c_count_valid(const int64_t* targets, int64_t n, int32_t V, int32_t* n_val
 int b2c_kd_token_loss(const void* student_logits, const float* teacher_logits, const int64_t* targets,
                       int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
                       const int32_t* n_valid, void* dlogits, float* row_kl, float* row_ce, int dtype, void* stream);
+
+/* b2c_kd_token_loss writing dlogits at row pitch ld_dlogits >= V (elements); the student and teacher logits keep pitch V.  The caller
+ * owns dlogits, (N, ld_dlogits) elements.  In bf16 mode with ld_dlogits % 8 == 0, ld_dlogits >= roundup(V, 8) and a 16-byte-aligned
+ * dlogits (any V <= 16384, any alignment of the logits) the rows are streamed by the TMA-pipelined pass and written with 16-byte
+ * stores; columns V .. roundup(V, 8) - 1 of every row are written as exact zeros, columns beyond that are not written.  Any other
+ * pitched call (fp32 mode, or a pitch that misses those conditions) returns B2C_EINVAL unless ld_dlogits == V, which is
+ * b2c_kd_token_loss. */
+int b2c_kd_token_loss_pitched(const void* student_logits, const float* teacher_logits, const int64_t* targets,
+                              int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
+                              const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype, void* stream);
 
 /* Evaluation form of the token pass (validate_student_model, src/train_student_kd.py:29-86): the same per-row KL and CE partials,
  * NO gradient, plus (argmax_out != NULL) the teacher-forced prediction argmax_v student_logits[r, v] of every row (lowest index on
