@@ -96,6 +96,10 @@ SYMBOLS = {
     "b2c_decoder_forward_prepared": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _vp, _sz, ctypes.c_int, _DRP, _vp]),
     "b2c_decoder_backward": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _vp, _GRD, _vp, _vp, _sz, ctypes.c_int, _DRP, ctypes.c_int, _vp]),
     "b2c_decoder_backward_pitched": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _GRD, _vp, _vp, _sz, ctypes.c_int, _DRP, ctypes.c_int, _vp]),
+    "b2c_decoder_forward_steps": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _vp, _sz, ctypes.c_int, _DRP, _vp, _vp]),
+    "b2c_decoder_forward_prepared_steps": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _vp, _sz, ctypes.c_int, _DRP, _vp, _vp]),
+    "b2c_decoder_backward_steps": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _GRD, _vp, _vp, _sz, ctypes.c_int, _DRP, ctypes.c_int,
+                                                  _vp, _vp]),
     "b2c_bump_counter": (ctypes.c_int, [_vp, _vp]),
     "b2c_debug_recur_trace": (ctypes.c_int, [_vp, _i64, _vp, _vp]),
     "b2c_join_side_work": (ctypes.c_int, [_vp]),
@@ -110,10 +114,14 @@ SYMBOLS = {
     "b2c_count_valid": (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp]),
     "b2c_kd_token_loss": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _f, _f, _f, _vp, _vp, _vp, _vp, ctypes.c_int, _vp]),
     "b2c_kd_token_loss_pitched": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _f, _f, _f, _vp, _vp, _i64, _vp, _vp, ctypes.c_int, _vp]),
+    "b2c_kd_token_loss_steps": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _f, _f, _f, _vp, _vp, _i64, _vp, _vp, ctypes.c_int, _vp, _i64, _vp]),
     "b2c_kd_token_eval": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _vp, _vp, _vp, _vp, ctypes.c_int, _vp]),
     "b2c_bleu1": (ctypes.c_int, [_vp, _vp, _i32, _i32, _vp, _vp]),
     "b2c_aux_loss": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32, _i32, _f, _f, _vp, _vp, _vp, _vp, _vp, ctypes.c_int, ctypes.c_int, _vp]),
+    "b2c_aux_loss_steps": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32, _i32, _f, _f, _vp, _vp, _vp, _vp, _vp, ctypes.c_int, ctypes.c_int,
+                                          _vp, _vp]),
     "b2c_loss_finalize": (ctypes.c_int, [_vp, _vp, _i64, _vp, _f, _vp, _i32, _i32, _vp, _i32, _i32, _f, _f, _f, _f, _f, _vp, _vp]),
+    "b2c_loss_finalize_steps": (ctypes.c_int, [_vp, _vp, _i64, _vp, _f, _vp, _i32, _i32, _vp, _i32, _i32, _f, _f, _f, _f, _f, _vp, _vp, _vp]),
     "b2c_scale_inplace": (ctypes.c_int, [_vp, _i64, ctypes.c_int, _vp, _vp]),
     "b2c_optimizer_step": (ctypes.c_int, [_vp, _vp, _vp, _vp, ctypes.POINTER(B2COptSegment), _i32, ctypes.POINTER(B2COptHyper),
                                           _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -217,10 +225,15 @@ class CallOptions:
                     so the all-reduce of the decoder's gradient segment can start while the refinement backward still runs.
     seed_dev        int64 device tensor (1 element): the per-step dropout counter the kernels mix into the seed (B2CDropout.seed_dev),
                     so CUDA-graph replays draw fresh masks.
-    background_ctas ProjectorFunction.backward only: CTA budget of its contractions when it overlaps the decoder's reverse recurrence."""
+    background_ctas ProjectorFunction.backward only: CTA budget of its contractions when it overlaps the decoder's reverse recurrence.
+    steps_dev       int32 device tensor (1 element), or None: the batch has only its first steps_dev[0] time steps (1 <= value <= T);
+                    the decoder and the KD loss compute the loss and gradients of that shorter batch in their (T, B, ...) buffers, reading
+                    the value at run time (the *_steps entry points of include/b2c.h), so one CUDA graph serves every caption length.
+                    The caller keeps the caption / target rows past it PAD (0) and writes the value on the stream before the call."""
 
-    def __init__(self, grad_dest=None, defer_join=False, after_backward=None, seed_dev=None, background_ctas=0):
+    def __init__(self, grad_dest=None, defer_join=False, after_backward=None, seed_dev=None, background_ctas=0, steps_dev=None):
         self.grad_dest, self.defer_join, self.after_backward, self.seed_dev = grad_dest, defer_join, after_backward, seed_dev
+        self.steps_dev = steps_dev
         # > 0: the projector's backward runs as background work next to a latency-bound chain on another stream: its persistent GEMMs
         # are confined to this many CTAs (b2c_set_gemm_cta_limit) so they cannot starve the chain of SMs
         self.background_ctas = background_ctas
@@ -333,6 +346,15 @@ def _pitched_rows(g: torch.Tensor, cdt: torch.dtype) -> Optional[int]:
     return ld
 
 
+def _steps_arg(sd: Optional[torch.Tensor]) -> Optional[int]:
+    """Device pointer of a CallOptions.steps_dev tensor (validated), or None for a full-length batch."""
+    if sd is None:
+        return None
+    if not (sd.is_cuda and sd.dtype == torch.int32 and sd.numel() == 1):
+        raise ValueError(f"steps_dev must be a 1-element int32 CUDA tensor, got {sd.dtype} {tuple(sd.shape)} on {sd.device}")
+    return sd.data_ptr()
+
+
 class DecoderFunction(torch.autograd.Function):
     """LSTMDecoder.forward (reference src/student_model.py:205-256) as one C-ABI call each way."""
 
@@ -354,11 +376,11 @@ class DecoderFunction(torch.autograd.Function):
                 raise ValueError(f"decoder was prepared for {prepared.key}, forward called with {(B, T, S, E, H, L, V, code)}")
             ws, cap = prepared.ws, prepared.cap
             torch.cuda.current_stream(feats.device).wait_stream(prepared.stream)
-            fwd = lib.b2c_decoder_forward_prepared
+            fwd = "prepared"
         else:
             cap = captions.detach().to(device=feats.device, dtype=torch.int64).contiguous()
             ws = torch.empty(workspace_bytes(shape, code, B2C_WS_TRAIN), dtype=torch.uint8, device=feats.device)
-            fwd = lib.b2c_decoder_forward
+            fwd = "plain"
         prm = _fill_struct(B2CParams(), master, L)
         if init_state is not None:
             # reference LSTMDecoder.forward(..., hidden=(h0, c0)): the split forward with the state written between its halves
@@ -370,15 +392,20 @@ class DecoderFunction(torch.autograd.Function):
                        "b2c_decoder_prepare")
             _check(lib.b2c_decoder_set_initial_state(ctypes.byref(shape), h0.data_ptr(), c0.data_ptr(), ws.data_ptr(), ws.numel(), code, _stream()),
                    "b2c_decoder_set_initial_state")
-            fwd = lib.b2c_decoder_forward_prepared
+            fwd = "prepared"
         logits = torch.empty(T, B, V, dtype=compute_dtype, device=feats.device)
         hid = torch.empty(T, B, H, dtype=compute_dtype, device=feats.device)
         attw = torch.empty(T, B, S, dtype=torch.float32, device=feats.device)
         drop = _dropout(dropout_p, seed, opts)
-        _check(fwd(ctypes.byref(shape), ctypes.byref(prm), f.data_ptr(), cap.data_ptr(), logits.data_ptr(),
-                   hid.data_ptr(), attw.data_ptr(), ws.data_ptr(), ws.numel(), code, ctypes.byref(drop), _stream()),
-               "b2c_decoder_forward")
-        ctx.b2c = (shape, code, drop, L, ws, f, cap, master, hid, attw, feats.dtype, [p.dtype for p in params], opts)
+        steps = _steps_arg(opts.steps_dev)
+        args = (ctypes.byref(shape), ctypes.byref(prm), f.data_ptr(), cap.data_ptr(), logits.data_ptr(), hid.data_ptr(), attw.data_ptr(),
+                ws.data_ptr(), ws.numel(), code, ctypes.byref(drop))
+        if steps is None:
+            _check((lib.b2c_decoder_forward if fwd == "plain" else lib.b2c_decoder_forward_prepared)(*args, _stream()), "b2c_decoder_forward")
+        else:                                            # variable-length batch: the device step count of opts.steps_dev
+            _check((lib.b2c_decoder_forward_steps if fwd == "plain" else lib.b2c_decoder_forward_prepared_steps)(*args, steps, _stream()),
+                   "b2c_decoder_forward_steps")
+        ctx.b2c = (shape, code, drop, L, ws, f, cap, master, hid, attw, feats.dtype, [p.dtype for p in params], opts, steps)
         ctx.b2c_params = params
         ctx.mark_non_differentiable(attw)
         return logits, hid, attw
@@ -386,7 +413,7 @@ class DecoderFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dlogits, dhid, _dattw):
         lib = load_library()
-        shape, code, drop, L, ws, f, cap, master, hid, attw, feats_dtype, pdtypes, opts = ctx.b2c
+        shape, code, drop, L, ws, f, cap, master, hid, attw, feats_dtype, pdtypes, opts, steps = ctx.b2c
         cdt = f.dtype
         if dlogits is None:
             dlogits = torch.zeros(shape.T, shape.B, shape.V, dtype=cdt, device=f.device)
@@ -403,7 +430,13 @@ class DecoderFunction(torch.autograd.Function):
         prm = _fill_struct(B2CParams(), master, L)
         grd = _fill_struct(B2CGrads(), grads, L)
         flags = B2C_BWD_DEFER_JOIN if defer else 0
-        if ld is None:
+        if steps is not None:                            # the rows past the step count of dlogits / dhid are zeros (KDLossFunction)
+            _check(lib.b2c_decoder_backward_steps(ctypes.byref(shape), ctypes.byref(prm), f.data_ptr(), cap.data_ptr(), hid.data_ptr(),
+                                                  attw.data_ptr(), dlogits.data_ptr(), shape.V if ld is None else ld, _ptr(dhid),
+                                                  ctypes.byref(grd), dfeats.data_ptr(), ws.data_ptr(), ws.numel(), code, ctypes.byref(drop),
+                                                  flags, steps, _stream()),
+                   "b2c_decoder_backward_steps")
+        elif ld is None:
             _check(lib.b2c_decoder_backward(ctypes.byref(shape), ctypes.byref(prm), f.data_ptr(), cap.data_ptr(), hid.data_ptr(), attw.data_ptr(),
                                             dlogits.data_ptr(), _ptr(dhid), ctypes.byref(grd), dfeats.data_ptr(), ws.data_ptr(), ws.numel(),
                                             code, ctypes.byref(drop), flags, _stream()),
@@ -482,8 +515,10 @@ class KDLossFunction(torch.autograd.Function):
     def forward(ctx, logits, teacher_logits, targets, feats_s, feats_t, hid_s, hid_t, cfg):
         lib = load_library()
         _require_cuda(logits, "student logits")
-        alpha, beta, gamma, temperature, w_ce, ce_mult, group, nval_global, unit_grad = cfg
+        alpha, beta, gamma, temperature, w_ce, ce_mult, group, nval_global, unit_grad = cfg[:9]
         T, B, V = logits.shape
+        # cfg[9]: CallOptions.steps_dev -- a variable-length batch of the first steps_dev[0] of T steps (its targets past them are PAD)
+        steps = _steps_arg(cfg[9] if len(cfg) > 9 else None)
         N = T * B
         dev = logits.device
         cdt = logits.dtype if logits.dtype in (torch.float32, torch.bfloat16) else torch.float32
@@ -504,12 +539,19 @@ class KDLossFunction(torch.autograd.Function):
             # view: DecoderFunction.backward hands the pitch on, and the vocabulary head's backward contractions stay on tensor cores
             Vp = (V + 7) // 8 * 8
             dlogits_buf = torch.empty(T, B, Vp, dtype=cdt, device=dev)
+            dlogits = dlogits_buf[..., :V]
+        else:
+            Vp = V
+            dlogits = dlogits_buf = torch.empty_like(y)
+        if steps is not None:                      # variable-length batch: rows past the step count get zero losses and gradients
+            _check(lib.b2c_kd_token_loss_steps(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), float(alpha), float(w_ce),
+                                               float(ce_mult), nval.data_ptr(), dlogits_buf.data_ptr(), Vp, rows[0].data_ptr(),
+                                               rows[1].data_ptr(), code, steps, B, st), "b2c_kd_token_loss_steps")
+        elif Vp != V:
             _check(lib.b2c_kd_token_loss_pitched(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), float(alpha), float(w_ce),
                                                  float(ce_mult), nval.data_ptr(), dlogits_buf.data_ptr(), Vp, rows[0].data_ptr(), rows[1].data_ptr(),
                                                  code, st), "b2c_kd_token_loss_pitched")
-            dlogits = dlogits_buf[..., :V]
         else:
-            dlogits = dlogits_buf = torch.empty_like(y)
             _check(lib.b2c_kd_token_loss(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), float(alpha), float(w_ce),
                                          float(ce_mult), nval.data_ptr(), dlogits.data_ptr(), rows[0].data_ptr(), rows[1].data_ptr(), code, st),
                    "b2c_kd_token_loss")
@@ -533,13 +575,19 @@ class KDLossFunction(torch.autograd.Function):
             dhs = torch.empty_like(hs)
             hid_part = torch.empty(Th * B, 2, dtype=torch.float32, device=dev)
         if fs is not None or hs is not None:
-            _check(lib.b2c_aux_loss(_ptr(fs), _ptr(ft), B, Ss, St, E, _ptr(hs), _ptr(ht), hs.shape[0] if hs is not None else 0, Th, H,
-                                    float(beta), float(gamma), _ptr(dfs), _ptr(dft), _ptr(dhs), _ptr(feat_part), _ptr(hid_part), code, fcode, st),
-                   "b2c_aux_loss")
+            aux = (_ptr(fs), _ptr(ft), B, Ss, St, E, _ptr(hs), _ptr(ht), hs.shape[0] if hs is not None else 0, Th, H,
+                   float(beta), float(gamma), _ptr(dfs), _ptr(dft), _ptr(dhs), _ptr(feat_part), _ptr(hid_part), code, fcode)
+            if steps is None:
+                _check(lib.b2c_aux_loss(*aux, st), "b2c_aux_loss")
+            else:
+                _check(lib.b2c_aux_loss_steps(*aux, steps, st), "b2c_aux_loss_steps")
         out5 = torch.empty(5, dtype=torch.float32, device=dev)
-        _check(lib.b2c_loss_finalize(rows[0].data_ptr(), rows[1].data_ptr(), N, nval.data_ptr(), float(ce_mult), _ptr(feat_part), B, E,
-                                     _ptr(hid_part), Th, H, float(temperature), float(alpha), float(beta), float(gamma), float(w_ce),
-                                     out5.data_ptr(), st), "b2c_loss_finalize")
+        fin = (rows[0].data_ptr(), rows[1].data_ptr(), N, nval.data_ptr(), float(ce_mult), _ptr(feat_part), B, E,
+               _ptr(hid_part), Th, H, float(temperature), float(alpha), float(beta), float(gamma), float(w_ce), out5.data_ptr())
+        if steps is None:
+            _check(lib.b2c_loss_finalize(*fin, st), "b2c_loss_finalize")
+        else:
+            _check(lib.b2c_loss_finalize_steps(*fin, steps, st), "b2c_loss_finalize_steps")
         ctx.b2c = dict(dlogits=dlogits, dlogits_buf=dlogits_buf, dfs=dfs, dft=dft, dhs=dhs, code=code, used=False, unit_grad=bool(unit_grad),
                        dtypes=(logits.dtype, None if feats_s is None else feats_s.dtype,
                                None if feats_t is None else feats_t.dtype, None if hid_s is None else hid_s.dtype))

@@ -204,11 +204,22 @@ template <typename T> struct DecodeWs {
 
 
 // ------------------------------------------------------------------ launch helpers
+// Variable-length recurrences: the contractions issued inside a StepScope belong to step `t` of a recurrence with the device step
+// count `steps` and do nothing when t >= *steps (GemmArgs::steps).  Thread-local and scoped, like GemmCapScope.
+struct StepGate { const int* steps; int t; };
+inline StepGate& step_gate() { static thread_local StepGate g{nullptr, 0}; return g; }
+struct StepScope {
+  StepGate saved;
+  StepScope(const int* steps, int t) : saved(step_gate()) { step_gate() = StepGate{steps, t}; }
+  ~StepScope() { step_gate() = saved; }
+};
+
 template <typename T, typename TC>
 int gemm(cudaStream_t st, int M, int N, int K, const T* A, long lda, int a_mn, const T* B, long ldb, int b_mn,
          TC* C, long ldc, float beta, const float* bias, int relu, float alpha, int row_unperm_h) {
   GemmArgs g{M, N, K, alpha, beta, A, lda, a_mn, B, ldb, b_mn, C, ldc, bias, relu};
   g.row_unperm_h = row_unperm_h;
+  g.steps = step_gate().steps; g.step = step_gate().t;
   return Gemm<T, TC>::run(g, st);
 }
 // gate contraction with the LSTM cell fused into the epilogue (no C is written)
@@ -216,8 +227,22 @@ template <typename T>
 int gemm_lstm(cudaStream_t st, int M, int H, int K, const T* A, long lda, const T* Wcat, long ldb, const LstmEpi& le) {
   GemmArgs g{M, 4 * H, K, 1.f, 0.f, A, lda, 0, Wcat, ldb, 0, nullptr, 4 * H, nullptr, 0};
   g.lstm = &le;
+  g.steps = step_gate().steps; g.step = step_gate().t;
   return Gemm<T, float>::run(g, st);
 }
+
+// zero the rows of steps >= *steps of up to TAIL_MAX_SEGS (Tn, B, .) buffers in one launch (decoder_kernels.cuh tail_zero_kernel);
+// each buffer: base, bytes per step (a multiple of 4), steps
+struct TailFill {
+  TailTable tab; TailFill() { tab.n = 0; }
+  void add(void* base, size_t step_bytes, int n_steps) { tab.seg[tab.n++] = TailSeg{base, (long)(step_bytes / 4), n_steps}; }
+  int launch(const int* steps, cudaStream_t st) {
+    if (tab.n == 0) return 0;
+    tail_zero_kernel<<<dim3(2 * 148, tab.n), 256, 0, st>>>(tab, steps);
+    B2C_LAUNCH_CHECK("tail_zero_kernel");
+    return 0;
+  }
+};
 
 inline int ew_grid(long n) { long g = (n + 255) / 256; if (g > 148 * 8) g = 148 * 8; if (g < 1) g = 1; return (int)g; }
 
@@ -261,14 +286,14 @@ template <typename K> int set_smem(K kern, size_t bytes) {
 // started -- callers issue pdl_full_dependency_next() once between the producers of P / F and that kernel.
 template <typename T>
 int attn_fwd(cudaStream_t st, const B2CShape& s, const float* P, const T* F, const float* u, T* ctx, long ldctx, float* attw,
-             long ldu = 0, float* u_save = nullptr) {
+             long ldu = 0, float* u_save = nullptr, const int* steps = nullptr, int t = 0) {
   if (ldu == 0) ldu = s.E;
   const size_t smem = (size_t)s.S * s.E * sizeof(T) + (size_t)(s.E + s.S) * 4;
   const int nq = s.S <= ATT_MAXTOK * (ATT_THREADS / 32) ? cdiv(s.E / 4, 32) : 4;       // more tokens than the register rows hold: generic kernel
   // E <= 256: 4 of the <= 7 token rows per warp are fetched in the prologue, the kernel fits 64 registers and all B = 512 CTAs
   // are resident in one wave (measured on B200: 3.23 ms / step vs 3.28 with all 7 rows up front at 80 registers, 3 CTAs / SM)
 #define B2C_ATT_(NQ, KA) do { B2C_TRY(set_smem(attn_step_fwd_kernel<T, NQ, KA>, smem)); \
-    B2C_CUDA(launch_pdl(attn_step_fwd_kernel<T, NQ, KA>, dim3(s.B), dim3(ATT_THREADS), smem, st, P, F, u, ldu, s.S, s.E, ctx, ldctx, attw, u_save)); } while (0)
+    B2C_CUDA(launch_pdl(attn_step_fwd_kernel<T, NQ, KA>, dim3(s.B), dim3(ATT_THREADS), smem, st, P, F, u, ldu, s.S, s.E, ctx, ldctx, attw, u_save, steps, t)); } while (0)
   if (nq == 1) B2C_ATT_(1, 4); else if (nq == 2) B2C_ATT_(2, 4); else if (nq == 3) B2C_ATT_(3, ATT_MAXTOK); else B2C_ATT_(0, ATT_MAXTOK);
 #undef B2C_ATT_
   B2C_LAUNCH_CHECK("attn_step_fwd_kernel");
@@ -277,11 +302,11 @@ int attn_fwd(cudaStream_t st, const B2CShape& s, const float* P, const T* F, con
 
 template <typename T>
 int attn_bwd(cudaStream_t st, int B, int S, int E, const float* P, const T* F, const float* u, const float* attw, const float* dctx, long lddctx,
-             float* ds, T* du) {
+             float* ds, T* du, const int* steps = nullptr, int t = 0) {
   const size_t smem = (size_t)S * E * sizeof(T) + (size_t)(E + 2 * S) * 4;
   constexpr int PB = 13;            // P rows per batch of the du phase (measured: 8 -> 3.25, 13 -> 3.23, 25 -> 3.32 ms / step)
 #define B2C_ATTB(PB, SMALL) do { B2C_TRY(set_smem(attn_step_bwd_kernel<T, PB, SMALL>, smem)); \
-    B2C_CUDA(launch_pdl(attn_step_bwd_kernel<T, PB, SMALL>, dim3(B), dim3(ATT_THREADS), smem, st, P, F, u, (long)E, attw, dctx, lddctx, S, E, ds, du, (long)E)); } while (0)
+    B2C_CUDA(launch_pdl(attn_step_bwd_kernel<T, PB, SMALL>, dim3(B), dim3(ATT_THREADS), smem, st, P, F, u, (long)E, attw, dctx, lddctx, S, E, ds, du, (long)E, steps, t)); } while (0)
   if (E <= 256) B2C_ATTB(PB, true); else B2C_ATTB(PB, false);
 #undef B2C_ATTB
   B2C_LAUNCH_CHECK("attn_step_bwd_kernel");
@@ -342,8 +367,8 @@ inline int pick_sub_batches(int B) {
   return 1;
 }
 struct SubPlan { int ns; cudaStream_t st[MAX_SUB]; int b0[MAX_SUB]; int bn[MAX_SUB]; SubStreams* ss; cudaStream_t main; };
-int fork_subs(SubPlan& sp, int B, cudaStream_t st) {
-  sp.ns = pick_sub_batches(B); sp.main = st; sp.ss = nullptr;
+int fork_subs(SubPlan& sp, int B, cudaStream_t st, bool allow_split = true) {
+  sp.ns = allow_split ? pick_sub_batches(B) : 1; sp.main = st; sp.ss = nullptr;
   if (sp.ns == 1) { sp.st[0] = st; sp.b0[0] = 0; sp.bn[0] = B; return 0; }
   B2C_TRY(get_substreams(&sp.ss));
   B2C_CUDA(cudaEventRecord(sp.ss->fork, st));
@@ -490,7 +515,7 @@ struct EvalOut { const float* teacher; const int64_t* targets; float temperature
 template <typename T>
 int decoder_forward_impl(const B2CShape& s, const B2CParams& p, const T* feats, const int64_t* cap, T* logits, T* hid_top,
                          float* attw, void* ws, size_t ws_bytes, const B2CDropout& dr, cudaStream_t st, bool prepared,
-                         const EvalOut* ev = nullptr) {
+                         const EvalOut* ev = nullptr, const int* steps = nullptr) {
   TrainWs<T> W; W.carve(ws, s);
   B2C_CHECK_ARG(ws_bytes >= W.bytes, "workspace too small: %zu < %zu", ws_bytes, W.bytes);
   const int B = s.B, Tn = s.T, S = s.S, E = s.E, H = s.H, L = s.L, V = s.V;
@@ -499,8 +524,10 @@ int decoder_forward_impl(const B2CShape& s, const B2CParams& p, const T* feats, 
   // time-invariant half of the attention projection: P = F W_f^T + b_a
   B2C_TRY((gemm<T, float>(st, B * S, E, E, feats, E, 0, W.w.Wf, E, 0, W.P, E, 0.f, p.attn_b)));
   const int inL = in_dim(s, L - 1), ldL = inL + H;
+  // A device step count (variable-length batch) takes the per-step kernels, which skip the steps past it; the whole-sequence kernels
+  // (B2C_PERSISTENT, B2C_CLUSTER) and sub-batch streams (B2C_SUB_BATCHES) are not used then.
   SubPlan sp;
-  B2C_TRY(fork_subs(sp, B, st));
+  B2C_TRY(fork_subs(sp, B, st, steps == nullptr));
   pdl_full_dependency_next();        // P / F are final before any kernel of the recurrence can start (attention prologues read them early)
   // bf16 mode: the whole T loop as ONE persistent cooperative kernel when the shape fits its plan (recurrent.cuh); the
   // per-step kernels below remain for fp32 parity mode, other shapes and B2C_PERSISTENT=0 (A/B)
@@ -508,10 +535,10 @@ int decoder_forward_impl(const B2CShape& s, const B2CParams& p, const T* feats, 
   RecurPlan rplan{}; rplan.ok = false;
   // first choice: independent 8-CTA clusters, one per row slice (recur_cluster.cuh); no inter-layer dropout in that kernel yet
   int ncl = 0;
-  if (sizeof(T) == 2 && sp.ns == 1 && !(dr.p > 0.f)) ncl = cluster_plan(s);
+  if (sizeof(T) == 2 && sp.ns == 1 && !(dr.p > 0.f) && !steps) ncl = cluster_plan(s);
   if (ncl > 0) { B2C_TRY(cluster_forward<T>(st, s, ncl, W, feats, hid_top, attw)); rplan.ok = true; }
   else {
-  if (sizeof(T) == 2 && sp.ns == 1) rplan = recur_plan(s);
+  if (sizeof(T) == 2 && sp.ns == 1 && !steps) rplan = recur_plan(s);
   if (rplan.ok) B2C_TRY(recur_forward<T>(st, s, rplan, W, feats, hid_top, attw, dr));
   }
   for (int t = 0; t < (rplan.ok ? 0 : Tn); ++t) {
@@ -519,6 +546,7 @@ int decoder_forward_impl(const B2CShape& s, const B2CParams& p, const T* feats, 
       cudaStream_t ss = sp.st[i];
       const long b0 = sp.b0[i];
       B2CShape sh = s; sh.B = sp.bn[i];
+      StepScope gate(steps, t);              // every kernel of this step does nothing when t >= *steps
       const long row = (long)t * B + b0;                       // first row of this sub-batch at step t in a (T,B,.) buffer
       const T* q = W.xh[L - 1] + row * ldL + inL;
       float* u_t = W.u + row * E;
@@ -531,10 +559,10 @@ int decoder_forward_impl(const B2CShape& s, const B2CParams& p, const T* feats, 
       float* ur = W.UR + b0 * ldur;
       if (merged) {
         B2C_TRY((gemm<T, float>(ss, sh.B, E + 4 * H, H, q, ldL, 0, W.w.Wuh, H, 0, ur, ldur)));
-        B2C_TRY(attn_fwd<T>(ss, sh, W.P + b0 * S * E, feats + b0 * S * E, ur, W.xh[0] + row * (E + H), E + H, attw + row * S, ldur, u_t));
+        B2C_TRY(attn_fwd<T>(ss, sh, W.P + b0 * S * E, feats + b0 * S * E, ur, W.xh[0] + row * (E + H), E + H, attw + row * S, ldur, u_t, steps, t));
       } else {
         B2C_TRY((gemm<T, float>(ss, sh.B, E, H, q, ldL, 0, W.w.Wh, H, 0, u_t, E)));
-        B2C_TRY(attn_fwd<T>(ss, sh, W.P + b0 * S * E, feats + b0 * S * E, u_t, W.xh[0] + row * (E + H), E + H, attw + row * S));
+        B2C_TRY(attn_fwd<T>(ss, sh, W.P + b0 * S * E, feats + b0 * S * E, u_t, W.xh[0] + row * (E + H), E + H, attw + row * S, 0, nullptr, steps, t));
       }
       for (int k = 0; k < L; ++k) {
         const int in = in_dim(s, k), ld = in + H;
@@ -548,6 +576,17 @@ int decoder_forward_impl(const B2CShape& s, const B2CParams& p, const T* feats, 
     }
   }
   B2C_TRY(join_subs(sp));
+  if (steps) {
+    // Invariant I2 (variable-length batch): the time-batched work below and in the backward keeps M / K = Tn*B, and multiplies
+    // the rows of the skipped steps by exact zeros (their logits and hidden-state gradients are zero, invariant I3).  Those rows of
+    // the saves it reads must be finite for that (0 x NaN = NaN), and the workspace may hold anything: zero them.
+    TailFill f;
+    f.add(hid_top, (size_t)B * H * sizeof(T), Tn);
+    f.add(attw, (size_t)B * S * sizeof(float), Tn);
+    f.add(W.u, (size_t)B * E * sizeof(float), Tn);
+    for (int k = 0; k < L; ++k) f.add(W.xh[k], (size_t)B * (in_dim(s, k) + H) * sizeof(T), Tn);
+    B2C_TRY(f.launch(steps, st));
+  }
   // output head, time-batched: y = W2 Drop(ReLU(W1 h + b1)) + b2
   B2C_TRY((gemm<T, T>(st, (int)TB, E, H, hid_top, H, 0, W.w.W1, H, 0, W.o1, E, 0.f, p.out0_b, 1)));
   if (dr.p > 0.f) {
@@ -586,7 +625,8 @@ inline int wgrad_chunks() { static int v = -1; if (v < 0) { const char* e = gete
 template <typename T>
 int decoder_backward_impl(const B2CShape& s, const B2CParams& p, const T* feats, const int64_t* cap, const T* hid_top,
                           const float* attw, const T* dlogits, const T* dhid, const B2CGrads& g, float* dfeats,
-                          void* ws, size_t ws_bytes, const B2CDropout& dr, cudaStream_t st, int flags, long ld_dl = 0 /* 0 = V */) {
+                          void* ws, size_t ws_bytes, const B2CDropout& dr, cudaStream_t st, int flags, long ld_dl = 0 /* 0 = V */,
+                          const int* steps = nullptr) {
   TrainWs<T> W; W.carve(ws, s);
   B2C_CHECK_ARG(ws_bytes >= W.bytes, "workspace too small: %zu < %zu", ws_bytes, W.bytes);
   B2C_CHECK_ARG(g.embedding && g.attn_w && g.attn_b && g.comb_w && g.comb_b && g.out0_w && g.out0_b && g.out3_w && g.out3_b && dfeats, "NULL gradient pointer");
@@ -604,6 +644,16 @@ int decoder_backward_impl(const B2CShape& s, const B2CParams& p, const T* feats,
   B2C_CUDA(cudaStreamWaitEvent(side, hs->ev[3], 0));
   B2C_CUDA(cudaMemsetAsync(W.dxh0, 0, (size_t)TB * (E + H) * sizeof(float), side));
   for (int k = 1; k < L; ++k) B2C_CUDA(cudaMemsetAsync(W.dxh[k], 0, (size_t)TB * 2 * H * sizeof(float), side));
+  if (steps) {
+    // Invariant I3 (variable-length batch): the skipped steps write no gate, u or score gradients, and the post-loop contractions
+    // read Tn*B rows of them: zero those rows.  (dxh0 / dxh[k] are zeroed above; the dlogits / dhidden_top rows of the skipped
+    // steps are zeros by the caller's contract, so d(o1) and dH_ext are too.)
+    TailFill f;
+    for (int k = 0; k < L; ++k) f.add(W.dgates[k], (size_t)B * 4 * H * sizeof(T), Tn);
+    f.add(W.du, (size_t)B * E * sizeof(T), Tn);
+    f.add(W.ds, (size_t)B * S * sizeof(float), Tn);
+    B2C_TRY(f.launch(steps, side));
+  }
   B2C_CUDA(cudaEventRecord(hs->ev[3], side));
   // ---- output head (time-batched).  Only d(o1) -> dH_ext feeds the time loop; the head's weight gradients run on a side
   // stream underneath the (latency-bound) recurrence and are joined after it.
@@ -624,7 +674,7 @@ int decoder_backward_impl(const B2CShape& s, const B2CParams& p, const T* feats,
   // ---- reverse time loop
   B2C_CUDA(cudaStreamWaitEvent(st, hs->ev[3], 0));                 // the zeroed dxh slots
   SubPlan sp;
-  B2C_TRY(fork_subs(sp, B, st));
+  B2C_TRY(fork_subs(sp, B, st, steps == nullptr));       // a device step count: no sub-batch streams (as in the forward)
   // Time-batched LSTM weight gradients over rows [r0, r1) of the (T*B, .) buffers (4H-sized rows come out interleaved and are
   // written gate-major).  They run on the side stream after the recurrence, next to the attn_post -> dF chain on the main one.
   // (Measured on B200: contracting the finished half of the steps on the side stream UNDER the recurrence slowed the chain by
@@ -643,17 +693,22 @@ int decoder_backward_impl(const B2CShape& s, const B2CParams& p, const T* feats,
   };
   // LSTM weight gradients of the steps already traversed, contracted in chunks on the side stream while the loop goes on (capped
   // grid, see gemm_cta_cap): the side branch that used to end ~70 us after the main chain is mostly done when the loop ends.
-  const int n_chunks = (sp.ns == 1 && bg_ctas() > 0) ? wgrad_chunks() : 0;
+  const int n_chunks = (sp.ns == 1 && bg_ctas() > 0 && !steps) ? wgrad_chunks() : 0;      // not with a device step count (steps unknown here)
   const int chunk_steps = n_chunks > 0 ? cdiv(Tn, n_chunks) : 0;
   long wg_done_from = TB;              // rows [wg_done_from, TB) have been contracted
   bool wg_any = false;
   pdl_full_dependency_next();        // the forward's saves (P, u, attention weights) are final before the reverse recurrence starts
+  // Variable-length batch: every kernel of step t >= *steps does nothing but its griddepcontrol.launch_dependents / wait (invariant
+  // I1: without the wait, a skipped grid could complete before its predecessors, and the post-loop kernels, which wait for the last
+  // grid of the chain only, would race with step *steps - 1).  The cell adjoint of step *steps - 1 treats itself as the last step
+  // (invariant I4: no carry, no dq, no dc from the skipped steps or an earlier call).
   for (int t = Tn - 1; t >= 0; --t) {
     const bool last = (t == Tn - 1);
     for (int i = 0; i < sp.ns; ++i) {
       cudaStream_t ss = sp.st[i];
       const long b0 = sp.b0[i];
       const int Bh = sp.bn[i];
+      StepScope gate(steps, t);
       const long row = (long)t * B + b0;
       for (int k = L - 1; k >= 0; --k) {
         const int in = in_dim(s, k), ld = in + H;
@@ -663,7 +718,8 @@ int decoder_backward_impl(const B2CShape& s, const B2CParams& p, const T* feats,
         B2C_CUDA(launch_pdl(lstm_pointwise_bwd_kernel<T>, dim3(ew_grid((long)Bh * H)), dim3(256), 0, ss,
             (const T*)(W.gates[k] + row * 4 * H), (const float*)(W.c[k] + row * H), (const float*)(W.c[k] + (row + B) * H), W.dc[k] + b0 * H, last ? 1 : 0,
             carry, (long)ld, above, (long)(2 * H), (const float*)(top ? W.dHext + row * H : nullptr), (const T*)((top && dhid) ? dhid + row * H : nullptr),
-            (const T*)((top && !last) ? W.dq + b0 * H : nullptr), (long)H, W.dgates[k] + row * 4 * H, Bh, H, dr.p, dr.seed, (uint32_t)k, row, (const unsigned long long*)dr.seed_dev));
+            (const T*)((top && !last) ? W.dq + b0 * H : nullptr), (long)H, W.dgates[k] + row * 4 * H, Bh, H, dr.p, dr.seed, (uint32_t)k, row, (const unsigned long long*)dr.seed_dev,
+            steps, t));
         B2C_LAUNCH_CHECK("lstm_pointwise_bwd_kernel");
         float* out = (k == 0) ? W.dxh0 + row * (E + H) : W.dxh[k] + row * 2 * H;
         B2C_TRY((gemm<T, float>(ss, Bh, ld, 4 * H, W.dgates[k] + row * 4 * H, 4 * H, 0, W.w.Wcat[k], ld, 1, out, ld, 1.f)));
@@ -671,7 +727,7 @@ int decoder_backward_impl(const B2CShape& s, const B2CParams& p, const T* feats,
       // layer 0's input gradient IS d(ctx_t): no context GEMM on the chain
       const float* dctx_t = W.dxh0 + row * (E + H);
       T* du_t = W.du + row * E;
-      B2C_TRY(attn_bwd<T>(ss, Bh, S, E, W.P + b0 * S * E, feats + b0 * S * E, W.u + row * E, attw + row * S, dctx_t, (long)(E + H), W.ds + row * S, du_t));
+      B2C_TRY(attn_bwd<T>(ss, Bh, S, E, W.P + b0 * S * E, feats + b0 * S * E, W.u + row * E, attw + row * S, dctx_t, (long)(E + H), W.ds + row * S, du_t, steps, t));
       if (t > 0) B2C_TRY((gemm<T, T>(ss, Bh, H, E, du_t, E, 0, W.w.Wh, H, 1, W.dq + b0 * H, H)));
     }
     if (chunk_steps > 0 && t > 0 && (Tn - t) % chunk_steps == 0 && t >= chunk_steps) {
@@ -1079,13 +1135,14 @@ int projector_backward_impl(const B2CShape& s, const B2CProjParams& p, const flo
 template <typename TS>
 int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, int V, float temperature, float alpha,
                        float w_ce_eff, const int* n_valid, TS* dy, float* row_kl, float* row_ce, cudaStream_t st, int* argmax_out = nullptr,
-                       long ld = 0 /* dy pitch; 0 = V */) {
+                       long ld = 0 /* dy pitch; 0 = V */, const int* steps = nullptr, long rows_per_step = 0) {
   if (ld == 0) ld = V;
   const bool eval = (dy == nullptr) || (argmax_out != nullptr);      // losses only (+ predictions): the row-in-smem kernel
   const bool vec = (V % 8 == 0) && (ld == V) && ((uintptr_t)y % 16 == 0) && ((uintptr_t)z % 16 == 0) && ((uintptr_t)dy % 16 == 0);
   const bool t4 = (temperature == 4.0f);
   const size_t smem = align_up((size_t)V * 4, 16) + align_up((size_t)V * sizeof(TS), 16);
   const float inv_temp = 1.0f / temperature, kd_coef = alpha * temperature / (float)N;
+  const float kd_num = alpha * temperature;        // with a device step count the kernels form kd_coef = kd_num / (*steps * rows_per_step)
   // default: persistent CTAs, TMA double-buffered row prefetch, register-resident math (V % 8 == 0, V <= 16384)
   const size_t psmem = 2 * ((size_t)V * 4 + (size_t)V * sizeof(TS));     // double-buffered row pair; larger rows take the row-in-smem kernel
   if (vec && V <= 8 * KDR_THREADS * 8 && !eval && psmem <= 200 * 1024) {
@@ -1097,7 +1154,7 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
 #define B2C_KDP(NCH, T4)                                                                                                   \
   do {                                                                                                                     \
     B2C_TRY(set_smem(kd_token_loss_pipe_kernel<TS, NCH, T4>, psmem));                                                      \
-    kd_token_loss_pipe_kernel<TS, NCH, T4><<<(unsigned)grid, KDR_THREADS, psmem, st>>>(y, z, tgt, N, V, inv_temp, temperature, kd_coef, w_ce_eff, n_valid, dy, row_kl, row_ce); \
+    kd_token_loss_pipe_kernel<TS, NCH, T4><<<(unsigned)grid, KDR_THREADS, psmem, st>>>(y, z, tgt, N, V, inv_temp, temperature, kd_coef, w_ce_eff, n_valid, dy, row_kl, row_ce, steps, rows_per_step, kd_num); \
   } while (0)
 #define B2C_KDP2(NCH) do { if (t4) B2C_KDP(NCH, true); else B2C_KDP(NCH, false); } while (0)
     switch (need) {
@@ -1124,7 +1181,7 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
 #define B2C_KDU(NCH, T4)                                                                                                   \
   do {                                                                                                                     \
     B2C_TRY(set_smem(kd_token_loss_pipe_unaligned_kernel<NCH, T4>, usmem));                                                \
-    kd_token_loss_pipe_unaligned_kernel<NCH, T4><<<(unsigned)grid, KDR_THREADS, usmem, st>>>(yb, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce_eff, n_valid, dyb, row_kl, row_ce); \
+    kd_token_loss_pipe_unaligned_kernel<NCH, T4><<<(unsigned)grid, KDR_THREADS, usmem, st>>>(yb, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce_eff, n_valid, dyb, row_kl, row_ce, steps, rows_per_step, kd_num); \
   } while (0)
 #define B2C_KDU2(NCH) do { if (t4) B2C_KDU(NCH, true); else B2C_KDU(NCH, false); } while (0)
     switch (need) {
@@ -1140,7 +1197,7 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
 #define B2C_KD_LAUNCH(G, T4)                                                                                             \
   do {                                                                                                                   \
     B2C_TRY(set_smem(kd_token_loss_kernel<TS, G, T4>, smem));                                                            \
-    kd_token_loss_kernel<TS, G, T4><<<(unsigned)N, KD_THREADS, smem, st>>>(y, z, tgt, V, inv_temp, kd_coef, w_ce_eff, n_valid, dy, row_kl, row_ce, argmax_out); \
+    kd_token_loss_kernel<TS, G, T4><<<(unsigned)N, KD_THREADS, smem, st>>>(y, z, tgt, V, inv_temp, kd_coef, w_ce_eff, n_valid, dy, row_kl, row_ce, argmax_out, steps, rows_per_step, kd_num); \
   } while (0)
   if (vec && t4) B2C_KD_LAUNCH(8, true);
   else if (vec) B2C_KD_LAUNCH(8, false);
@@ -1153,7 +1210,8 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
 
 template <typename TF, typename TH>
 int aux_loss_impl(const TF* fs, const float* ft, int B, int Ss, int St, int E, const TH* hs, const float* ht, int Tn, int Th, int H,
-                  float beta, float gamma, float* dfs, float* dft, TH* dhs, float* feat_part, float* hid_part, cudaStream_t st) {
+                  float beta, float gamma, float* dfs, float* dft, TH* dhs, float* feat_part, float* hid_part, cudaStream_t st,
+                  const int* steps = nullptr) {
   const int nfb = fs ? B : 0;
   const long all_rows = hs ? (long)Tn * B : 0;
   const int hid_blocks = (int)((all_rows + 7) / 8);
@@ -1161,7 +1219,7 @@ int aux_loss_impl(const TF* fs, const float* ft, int B, int Ss, int St, int E, c
   const size_t smem = fs ? (size_t)(2 * Ss + 2 * St + 2 * E + 8 * 2 * E + 8) * 4 : 0;       // + per-warp column partials [8][2][E]
   B2C_TRY(set_smem(aux_loss_kernel<TF, TH>, smem));
   aux_loss_kernel<TF, TH><<<nfb + hid_blocks, 256, smem, st>>>(fs, ft, nfb, B, Ss, St, E, hs, ht, (int)((long)Th * B), (int)all_rows, H, Th, beta, gamma,
-                                                               dfs, dft, dhs, feat_part, hid_part);
+                                                               dfs, dft, dhs, feat_part, hid_part, steps);
   B2C_LAUNCH_CHECK("aux_loss_kernel");
   return 0;
 }
@@ -1201,14 +1259,14 @@ size_t b2c_workspace_bytes(const B2CShape* shape, int dtype, int mode) {
 
 static int decoder_forward_entry(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
                                  void* logits, void* hidden_top, float* attn_w, void* workspace, size_t ws_bytes,
-                                 int dtype, const B2CDropout* dropout, void* stream, bool prepared) {
+                                 int dtype, const B2CDropout* dropout, void* stream, bool prepared, const int32_t* steps = nullptr) {
   B2C_TRY(check_shape(shape)); B2C_TRY(check_device());
   B2C_CHECK_ARG(params && feats && captions && logits && hidden_top && attn_w && workspace, "NULL argument");
   const B2CDropout dr = dropout ? *dropout : B2CDropout{0.f, 0, nullptr};
   B2C_CHECK_ARG(dr.p >= 0.f && dr.p < 1.f, "dropout p=%f outside [0,1)", dr.p);
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B2C_F32) return decoder_forward_impl<float>(*shape, *params, (const float*)feats, captions, (float*)logits, (float*)hidden_top, attn_w, workspace, ws_bytes, dr, st, prepared);
-  if (dtype == B2C_BF16) return decoder_forward_impl<bf16>(*shape, *params, (const bf16*)feats, captions, (bf16*)logits, (bf16*)hidden_top, attn_w, workspace, ws_bytes, dr, st, prepared);
+  if (dtype == B2C_F32) return decoder_forward_impl<float>(*shape, *params, (const float*)feats, captions, (float*)logits, (float*)hidden_top, attn_w, workspace, ws_bytes, dr, st, prepared, nullptr, steps);
+  if (dtype == B2C_BF16) return decoder_forward_impl<bf16>(*shape, *params, (const bf16*)feats, captions, (bf16*)logits, (bf16*)hidden_top, attn_w, workspace, ws_bytes, dr, st, prepared, nullptr, steps);
   return set_err(B2C_EINVAL, "bad dtype %d", dtype);
 }
 int b2c_decoder_forward(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
@@ -1220,6 +1278,16 @@ int b2c_decoder_forward_prepared(const B2CShape* shape, const B2CParams* params,
                                  void* logits, void* hidden_top, float* attn_w, void* workspace, size_t ws_bytes,
                                  int dtype, const B2CDropout* dropout, void* stream) {
   return decoder_forward_entry(shape, params, feats, captions, logits, hidden_top, attn_w, workspace, ws_bytes, dtype, dropout, stream, true);
+}
+int b2c_decoder_forward_steps(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                              void* logits, void* hidden_top, float* attn_w, void* workspace, size_t ws_bytes,
+                              int dtype, const B2CDropout* dropout, const int32_t* steps, void* stream) {
+  return decoder_forward_entry(shape, params, feats, captions, logits, hidden_top, attn_w, workspace, ws_bytes, dtype, dropout, stream, false, steps);
+}
+int b2c_decoder_forward_prepared_steps(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                                       void* logits, void* hidden_top, float* attn_w, void* workspace, size_t ws_bytes,
+                                       int dtype, const B2CDropout* dropout, const int32_t* steps, void* stream) {
+  return decoder_forward_entry(shape, params, feats, captions, logits, hidden_top, attn_w, workspace, ws_bytes, dtype, dropout, stream, true, steps);
 }
 int b2c_decoder_forward_eval(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
                              const float* teacher_logits, const int64_t* targets, float temperature,
@@ -1279,6 +1347,20 @@ int b2c_decoder_backward_pitched(const B2CShape* shape, const B2CParams* params,
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == B2C_F32) return decoder_backward_impl<float>(*shape, *params, (const float*)feats, captions, (const float*)hidden_top, attn_w, (const float*)dlogits, (const float*)dhidden_top, *grads, dfeats, workspace, ws_bytes, dr, st, flags, (long)ld_dlogits);
   if (dtype == B2C_BF16) return decoder_backward_impl<bf16>(*shape, *params, (const bf16*)feats, captions, (const bf16*)hidden_top, attn_w, (const bf16*)dlogits, (const bf16*)dhidden_top, *grads, dfeats, workspace, ws_bytes, dr, st, flags, (long)ld_dlogits);
+  return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+}
+
+int b2c_decoder_backward_steps(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                               const void* hidden_top, const float* attn_w, const void* dlogits, int64_t ld_dlogits, const void* dhidden_top,
+                               const B2CGrads* grads, float* dfeats, void* workspace, size_t ws_bytes,
+                               int dtype, const B2CDropout* dropout, int flags, const int32_t* steps, void* stream) {
+  B2C_TRY(check_shape(shape)); B2C_TRY(check_device());
+  B2C_CHECK_ARG(params && feats && captions && hidden_top && attn_w && dlogits && grads && workspace, "NULL argument");
+  B2C_CHECK_ARG(ld_dlogits >= shape->V, "ld_dlogits=%ld < V=%d", (long)ld_dlogits, shape->V);
+  const B2CDropout dr = dropout ? *dropout : B2CDropout{0.f, 0, nullptr};
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == B2C_F32) return decoder_backward_impl<float>(*shape, *params, (const float*)feats, captions, (const float*)hidden_top, attn_w, (const float*)dlogits, (const float*)dhidden_top, *grads, dfeats, workspace, ws_bytes, dr, st, flags, (long)ld_dlogits, steps);
+  if (dtype == B2C_BF16) return decoder_backward_impl<bf16>(*shape, *params, (const bf16*)feats, captions, (const bf16*)hidden_top, attn_w, (const bf16*)dlogits, (const bf16*)dhidden_top, *grads, dfeats, workspace, ws_bytes, dr, st, flags, (long)ld_dlogits, steps);
   return set_err(B2C_EINVAL, "bad dtype %d", dtype);
 }
 
@@ -1426,6 +1508,21 @@ int b2c_kd_token_loss_pitched(const void* student_logits, const float* teacher_l
   return set_err(B2C_EINVAL, "bad dtype %d", dtype);
 }
 
+int b2c_kd_token_loss_steps(const void* student_logits, const float* teacher_logits, const int64_t* targets,
+                            int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
+                            const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype,
+                            const int32_t* steps, int64_t rows_per_step, void* stream) {
+  B2C_TRY(check_device());
+  B2C_CHECK_ARG(student_logits && teacher_logits && targets && n_valid && dlogits && row_kl && row_ce, "NULL argument");
+  B2C_CHECK_ARG(N > 0 && N < 2147483647L && V > 1 && temperature > 0.f, "bad N=%ld V=%d temperature=%f", (long)N, V, temperature);
+  B2C_CHECK_ARG(ld_dlogits >= V, "ld_dlogits=%ld < V=%d", (long)ld_dlogits, V);
+  B2C_CHECK_ARG(steps == nullptr || (rows_per_step > 0 && N % rows_per_step == 0), "rows_per_step=%ld must divide N=%ld", (long)rows_per_step, (long)N);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == B2C_F32) return kd_token_loss_impl<float>((const float*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (float*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits, steps, (long)rows_per_step);
+  if (dtype == B2C_BF16) return kd_token_loss_impl<bf16>((const bf16*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (bf16*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits, steps, (long)rows_per_step);
+  return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+}
+
 int b2c_kd_token_eval(const void* student_logits, const float* teacher_logits, const int64_t* targets, int64_t N, int32_t V,
                       float temperature, const int32_t* n_valid, float* row_kl, float* row_ce, int32_t* argmax_out, int dtype, void* stream) {
   B2C_TRY(check_device());
@@ -1460,6 +1557,21 @@ int b2c_aux_loss(const void* feats_s, const float* feats_t, int32_t B, int32_t S
   return set_err(B2C_EINVAL, "bad dtype %d / feature dtype %d", dtype, feat_dtype);
 }
 
+int b2c_aux_loss_steps(const void* feats_s, const float* feats_t, int32_t B, int32_t Ss, int32_t St, int32_t E,
+                       const void* hid_s, const float* hid_t, int32_t T, int32_t Th, int32_t H,
+                       float beta, float gamma, float* dfeats_s, float* dfeats_t, void* dhid_s,
+                       float* feat_part, float* hid_part, int dtype, int feat_dtype, const int32_t* steps, void* stream) {
+  B2C_TRY(check_device());
+  B2C_CHECK_ARG(B > 0, "B=%d", B);
+  if (feats_s) B2C_CHECK_ARG(feats_t && feat_part && Ss > 0 && St > 0 && E > 0 && E % 8 == 0, "feature KD needs feats_t, feat_part, positive Ss/St and E a positive multiple of 8 (E=%d)", E);
+  if (hid_s) B2C_CHECK_ARG(hid_t && hid_part && T > 0 && Th > 0 && Th <= T && H > 0 && H % 8 == 0, "hidden KD needs hid_t, hid_part, 0 < Th <= T and H a positive multiple of 8 (H=%d)", H);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == B2C_F32 && feat_dtype == B2C_F32) return aux_loss_impl<float, float>((const float*)feats_s, feats_t, B, Ss, St, E, (const float*)hid_s, hid_t, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (float*)dhid_s, feat_part, hid_part, st, steps);
+  if (dtype == B2C_BF16 && feat_dtype == B2C_BF16) return aux_loss_impl<bf16, bf16>((const bf16*)feats_s, feats_t, B, Ss, St, E, (const bf16*)hid_s, hid_t, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (bf16*)dhid_s, feat_part, hid_part, st, steps);
+  if (dtype == B2C_BF16 && feat_dtype == B2C_F32) return aux_loss_impl<float, bf16>((const float*)feats_s, feats_t, B, Ss, St, E, (const bf16*)hid_s, hid_t, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (bf16*)dhid_s, feat_part, hid_part, st, steps);
+  return set_err(B2C_EINVAL, "bad dtype %d / feature dtype %d", dtype, feat_dtype);
+}
+
 int b2c_loss_finalize(const float* row_kl, const float* row_ce, int64_t N, const int32_t* n_valid, float ce_mult,
                       const float* feat_part, int32_t B, int32_t E, const float* hid_part, int32_t Th, int32_t H,
                       float temperature, float alpha, float beta, float gamma, float w_ce, float* out5, void* stream) {
@@ -1467,7 +1579,19 @@ int b2c_loss_finalize(const float* row_kl, const float* row_ce, int64_t N, const
   B2C_CHECK_ARG(row_kl && row_ce && n_valid && out5 && N > 0 && B > 0, "bad argument");
   loss_finalize_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(row_kl, row_ce, (long)N, n_valid, feat_part, B, E, feat_part ? 1 : 0,
                                                             hid_part, (long)Th * B, H, Th, hid_part ? 1 : 0,
-                                                            temperature, alpha, beta, gamma, w_ce, ce_mult, out5);
+                                                            temperature, alpha, beta, gamma, w_ce, ce_mult, out5, (const int*)nullptr);
+  B2C_LAUNCH_CHECK("loss_finalize_kernel");
+  return 0;
+}
+
+int b2c_loss_finalize_steps(const float* row_kl, const float* row_ce, int64_t N, const int32_t* n_valid, float ce_mult,
+                            const float* feat_part, int32_t B, int32_t E, const float* hid_part, int32_t Th, int32_t H,
+                            float temperature, float alpha, float beta, float gamma, float w_ce, float* out5, const int32_t* steps, void* stream) {
+  B2C_TRY(check_device());
+  B2C_CHECK_ARG(row_kl && row_ce && n_valid && out5 && N > 0 && B > 0, "bad argument");
+  loss_finalize_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(row_kl, row_ce, (long)N, n_valid, feat_part, B, E, feat_part ? 1 : 0,
+                                                            hid_part, (long)Th * B, H, Th, hid_part ? 1 : 0,
+                                                            temperature, alpha, beta, gamma, w_ce, ce_mult, out5, steps);
   B2C_LAUNCH_CHECK("loss_finalize_kernel");
   return 0;
 }

@@ -121,7 +121,8 @@ template <typename T, int NQ, int KA>  // NQ = float4 per lane per token (ceil(E
 __global__ void __launch_bounds__(ATT_THREADS, KA >= ATT_MAXTOK ? 1 : 4)
 attn_step_fwd_kernel(const float* __restrict__ P, const T* __restrict__ F, const float* __restrict__ u, long ldu,
                      int S, int E, T* __restrict__ ctx, long ldctx, float* __restrict__ attw /* (B,S) or null */,
-                     float* __restrict__ u_save /* (B,E) or null: dense copy of u (a forward save when u sits inside a wider row) */) {
+                     float* __restrict__ u_save /* (B,E) or null: dense copy of u (a forward save when u sits inside a wider row) */,
+                     const int* __restrict__ steps /* null, or the device step count: step `step` >= *steps does nothing */, int step) {
   extern __shared__ __align__(128) unsigned char att_smem[];
   const int SE = S * E;
   T* Fs = reinterpret_cast<T*>(att_smem);
@@ -131,6 +132,7 @@ attn_step_fwd_kernel(const float* __restrict__ P, const T* __restrict__ F, const
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarp = ATT_THREADS / 32;
   const int b = blockIdx.x;
   pdl_launch_dependents();
+  if (steps != nullptr && step >= __ldg(steps)) { pdl_wait(); return; }      // past the batch's length (invariant I1, api.cu)
   // ---- prologue: independent of the preceding kernel
   if (tid == 0) { mbar_init(&bar, 1); fence_barrier_init(); }
   const float4* Pb = reinterpret_cast<const float4*>(P + (long)b * SE);
@@ -236,7 +238,8 @@ template <typename T, int PB, bool E256 = false>       // E256: E <= 256 known a
 __global__ void __launch_bounds__(ATT_THREADS, 4)
 attn_step_bwd_kernel(const float* __restrict__ P, const T* __restrict__ F, const float* __restrict__ u, long ldu,
                      const float* __restrict__ attw, const float* __restrict__ dctx, long lddctx,
-                     int S, int E, float* __restrict__ ds_out, T* __restrict__ du, long lddu) {
+                     int S, int E, float* __restrict__ ds_out, T* __restrict__ du, long lddu,
+                     const int* __restrict__ steps /* null, or the device step count: step `step` >= *steps does nothing */, int step) {
   extern __shared__ __align__(128) unsigned char att_smem[];
   const int SE = S * E;
   T* Fs = reinterpret_cast<T*>(att_smem);
@@ -248,6 +251,7 @@ attn_step_bwd_kernel(const float* __restrict__ P, const T* __restrict__ F, const
   const int b = blockIdx.x;
   const float* Pb = P + (long)b * SE;
   pdl_launch_dependents();
+  if (steps != nullptr && step >= __ldg(steps)) { pdl_wait(); return; }      // past the batch's length (invariant I1, api.cu)
   // ---- prologue: F, P, u and the attention weights were written by the forward pass
   if (tid == 0) { mbar_init(&bar, 1); fence_barrier_init(); }
   for (int l = tid; l < S; l += ATT_THREADS) ws[l] = attw[(long)b * S + l];
@@ -489,8 +493,13 @@ lstm_pointwise_bwd_kernel(const T* __restrict__ gates, const float* __restrict__
                           const float* __restrict__ dh_carry, long ld_carry, const float* __restrict__ dh_above, long ld_above,
                           const float* __restrict__ dh_ext, const T* __restrict__ dh_hid, const T* __restrict__ dh_q, long ld_q,
                           T* __restrict__ dgates, int B, int H, float drop_p, uint64_t seed, uint32_t site, long row_base,
-                          const unsigned long long* __restrict__ seed_dev) {
+                          const unsigned long long* __restrict__ seed_dev, const int* __restrict__ steps, int step) {
   pdl_launch_dependents();
+  if (steps != nullptr) {                      // variable-length batch (api.cu, invariants I1 and I4)
+    const int n = __ldg(steps);
+    if (step >= n) { pdl_wait(); return; }
+    if (step == n - 1) { dc_is_zero = 1; dh_carry = nullptr; dh_q = nullptr; }   // the batch's last step: nothing flows back into it
+  }
   if (drop_p > 0.f) seed = drop_seed(seed, seed_dev);
   const long total = (long)B * H;
   const float inv_keep = drop_p > 0.f ? 1.0f / (1.0f - drop_p) : 1.0f;
@@ -523,6 +532,29 @@ lstm_pointwise_bwd_kernel(const T* __restrict__ gates, const float* __restrict__
     Gate4<T>::store(dgates + b * 4 * H + 4 * j, dg);
     dc[idx] = dcc * f;
   }
+}
+
+// ======================================================================================
+// Variable-length batches (b2c.h *_steps entry points): the rows of the steps at and past the device step count, in several
+// (steps, B, .) buffers, set to zero by one launch.  Segment y of the grid: step_words 4-byte words per step, n_steps steps.
+// ======================================================================================
+struct TailSeg { void* base; long step_words; int n_steps; };
+constexpr int TAIL_MAX_SEGS = 8;
+struct TailTable { TailSeg seg[TAIL_MAX_SEGS]; int n; };
+__global__ void __launch_bounds__(256) tail_zero_kernel(const __grid_constant__ TailTable tab, const int* __restrict__ steps) {
+  const TailSeg& s = tab.seg[blockIdx.y];
+  const int n = min(max(__ldg(steps), 0), s.n_steps);
+  uint32_t* p = reinterpret_cast<uint32_t*>(s.base);
+  const long w0 = (long)n * s.step_words, w1 = (long)s.n_steps * s.step_words;
+  // scalar words up to the first 16-byte boundary, 16-byte stores over the rest, scalar words after the last boundary
+  long v0 = w0 + (long)((16 - ((uintptr_t)(p + w0) & 15)) & 15) / 4;
+  if (v0 > w1) v0 = w1;
+  const long nv = (w1 - v0) / 4;
+  const long i0 = (long)blockIdx.x * blockDim.x + threadIdx.x, stride = (long)gridDim.x * blockDim.x;
+  for (long i = w0 + i0; i < v0; i += stride) p[i] = 0u;
+  uint4* q = reinterpret_cast<uint4*>(p + v0);
+  for (long i = i0; i < nv; i += stride) q[i] = make_uint4(0u, 0u, 0u, 0u);
+  for (long i = v0 + nv * 4 + i0; i < w1; i += stride) p[i] = 0u;
 }
 
 // ======================================================================================

@@ -37,6 +37,8 @@ struct LstmEpi {
   const unsigned long long* seed_dev;   // optional device step counter mixed into the seed (CUDA-graph replays)
   const float* addend32; long ld_addend32;   // optional fp32 addend (rows, >= 4H) with its own pitch: the recurrent half W_hh h_{t-1} of the
                                         // pre-activations when it was contracted ahead of time (tcgen05 path only)
+  const int* steps; int step;           // variable-length recurrences: the launch does nothing when step >= *steps (any flavour; steps
+                                        // null = always run).  Set from GemmArgs, see GemmStepScope.
 };
 
 // Validation (validate_student_model, reference src/train_student_kd.py:29-86) needs, per logits row, only the token-KD term, the CE
@@ -89,6 +91,7 @@ gemm_simt_kernel(int M, int N, int K, float alpha, const TA* __restrict__ A, lon
   __shared__ float Bs[SG_BK][SG_BN + 4];
   pdl_launch_dependents();
   pdl_wait();
+  if (le.steps != nullptr && le.step >= __ldg(le.steps)) return;      // a step past the batch's length (after the wait: invariant I1, api.cu)
   const int tid = threadIdx.x;
   const int m0 = blockIdx.y * SG_BM, n0 = blockIdx.x * SG_BN;
   const int tx = tid & 15, ty = tid >> 4;      // 16 x 16 threads, 4x4 outputs each
@@ -308,6 +311,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const bool split = splits > 1;
 
   pdl_launch_dependents();                   // the next kernel on the chain may begin its own prologue
+  // a step past the batch's length: no barrier, no TMEM, but still griddepcontrol.wait, so that this grid completes only after its
+  // predecessors did (invariant I1, api.cu).  The step count is read before the wait: it is written before the recurrence's first,
+  // fully serialised kernel starts, and nothing on the chain writes it.
+  if (le.steps != nullptr && le.step >= __ldg(le.steps)) { pdl_wait(); return; }
   if (warp == 0 && lane == 0) { tma_prefetch_desc(&tmA); tma_prefetch_desc(&tmB); }
   if (warp == 1) {
     if (lane == 0) {
@@ -807,6 +814,8 @@ struct GemmArgs {
   const LstmEpi* lstm = nullptr;     // fused LSTM-cell epilogue instead of writing C
   ArgmaxEpi* amax = nullptr;         // per-row partial argmax instead of writing C (tcgen05 path only; nparts / cols_per_part are filled in)
   EvalEpi* eval = nullptr;           // per-row partials of token KD / CE / argmax instead of writing C (tcgen05 path only; nparts filled in)
+  const int* steps = nullptr;        // != null: the launch is step `step` of a variable-length recurrence and does nothing when step >= *steps
+  int step = 0;
 };
 
 inline bool tc_eligible(const GemmArgs& g) {
@@ -906,6 +915,7 @@ int launch_tc(const GemmArgs& g, const TcPlan& plan, cudaStream_t st) {
     g.eval->nparts = cdiv(g.N, g.eval->cols_per_part);          // the caller sized `parts` for the smallest part (32 columns)
     epi = pack_eval(*g.eval);
   }
+  epi.steps = g.steps; epi.step = g.step;
   B2C_CUDA(launch_pdl(kern, dim3(grid), dim3(TC_THREADS), TcCfg<BN>::SMEM_BYTES, st, ta, tb, g.M, g.N, g.K, g.alpha, g.beta, (TC*)g.C, g.ldc,
                       g.bias, g.relu, kb_per_split, tiles_m, tiles_n, splits, g.row_unperm_h, epi));
   B2C_LAUNCH_CHECK("gemm_tc_kernel");
@@ -932,8 +942,10 @@ int gemm_bf16_tc(const GemmArgs& g, cudaStream_t st) {
 template <typename TA, typename TB, typename TC>
 int gemm_simt(const GemmArgs& g, cudaStream_t st) {
   dim3 grid(cdiv(g.N, SG_BN), cdiv(g.M, SG_BM));
+  LstmEpi le = g.lstm ? *g.lstm : LstmEpi{};
+  le.steps = g.steps; le.step = g.step;
   B2C_CUDA(launch_pdl(gemm_simt_kernel<TA, TB, TC>, grid, dim3(256), 0, st, g.M, g.N, g.K, g.alpha, (const TA*)g.A, g.lda, g.a_mn,
-                      (const TB*)g.B, g.ldb, g.b_mn, g.beta, (TC*)g.C, g.ldc, g.bias, g.relu, g.row_unperm_h, g.lstm ? *g.lstm : LstmEpi{}));
+                      (const TB*)g.B, g.ldb, g.b_mn, g.beta, (TC*)g.C, g.ldc, g.bias, g.relu, g.row_unperm_h, le));
   B2C_LAUNCH_CHECK("gemm_simt_kernel");
   return 0;
 }

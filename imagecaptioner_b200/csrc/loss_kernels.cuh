@@ -68,7 +68,20 @@ __global__ void __launch_bounds__(KD_THREADS)
 kd_token_loss_kernel(const TS* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
                      int V, float inv_temp, float kd_coef, float w_ce, const int* __restrict__ n_valid_ptr,
                      TS* __restrict__ dy /* NULL: losses only (evaluation) */, float* __restrict__ row_kl, float* __restrict__ row_ce,
-                     int* __restrict__ argmax_out /* NULL, or (N): argmax_v y[r, v], lowest index on ties like torch.argmax */) {
+                     int* __restrict__ argmax_out /* NULL, or (N): argmax_v y[r, v], lowest index on ties like torch.argmax */,
+                     const int* __restrict__ steps /* NULL, or the device step count of a variable-length batch */, long rows_per_step,
+                     float kd_num /* alpha * Temp: kd_coef = kd_num / (*steps * rows_per_step) when steps is set */) {
+  if (steps != nullptr) {
+    // variable-length batch: only the first n = *steps * rows_per_step rows exist.  A row past them reads nothing and leaves zero
+    // losses and a zero gradient row; the others use the KD scale of n rows.
+    const long n = min((long)gridDim.x, (long)__ldg(steps) * rows_per_step);
+    if ((long)blockIdx.x >= n) {
+      if (dy != nullptr) for (int v = threadIdx.x; v < V; v += KD_THREADS) dy[(long)blockIdx.x * V + v] = from_f<TS>(0.f);
+      if (threadIdx.x == 0) { row_kl[blockIdx.x] = 0.f; row_ce[blockIdx.x] = 0.f; }
+      return;
+    }
+    kd_coef = kd_num / (float)n;
+  }
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float* zs = reinterpret_cast<float*>(smem_raw);                             // V floats
   TS* ys = reinterpret_cast<TS*>(smem_raw + align_up((size_t)V * 4, 16)); // V TS
@@ -279,7 +292,7 @@ template <typename TS, int NCH, bool TEMP4, bool UNALIGNED>
 __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
                                                    long N, int V, long ld, float inv_temp, float temperature, float kd_coef, float w_ce,
                                                    const int* __restrict__ n_valid_ptr, TS* __restrict__ dy, float* __restrict__ row_kl,
-                                                   float* __restrict__ row_ce) {
+                                                   float* __restrict__ row_ce, const int* __restrict__ steps, long rows_per_step, float kd_num) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ __align__(8) uint64_t full_bar[KD_SLOTS];
   __shared__ float scratch[KDR_THREADS / 32 * 4];
@@ -291,6 +304,11 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int groups = UNALIGNED ? (Vp >> 3) : (V >> 3);
   const int n_valid = *n_valid_ptr;
+  // variable-length batch (steps != null): rows [n, N) are past the batch.  They are never fetched (the enclosing 16-byte range of
+  // row n - 1 in the unaligned form may reach into row n; those columns are replaced by the sentinel below and never used) and get
+  // zero losses and a zero gradient row; the KD scale is that of n rows.
+  long n = N;
+  if (steps != nullptr) { n = min(N, (long)__ldg(steps) * rows_per_step); kd_coef = kd_num / (float)n; }
   const uintptr_t y_end = (uintptr_t)(y + N * (long)V), z_end = (uintptr_t)(z + N * (long)V);
   // enclosing 16-byte range [lo, hi) of row `row` of y / z, and whether both lie inside their tensors
   auto y_lo = [&](long row) { return (uintptr_t)(y + row * (long)V) & ~(uintptr_t)15; };
@@ -320,11 +338,11 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
   __syncthreads();
   const long r0 = blockIdx.x, stride = gridDim.x;
   if (tid == 0) {
-    for (int i = 0; i < KD_SLOTS; ++i) if (r0 + i * stride < N) issue(r0 + i * stride, i);
+    for (int i = 0; i < KD_SLOTS; ++i) if (r0 + i * stride < n) issue(r0 + i * stride, i);
   }
 
   int it = 0;
-  for (long r = r0; r < N; r += stride, ++it) {
+  for (long r = r0; r < n; r += stride, ++it) {
     const int sidx = it % KD_SLOTS; const uint32_t ph = (it / KD_SLOTS) & 1;
     const float* zs = reinterpret_cast<const float*>(smem_raw + (size_t)sidx * slot);
     const TS* ys = reinterpret_cast<const TS*>(smem_raw + (size_t)sidx * slot + zbytes);
@@ -383,7 +401,7 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
       else { y_tgt = to_f<TS>(y[r * (long)V + t_idx]); z_tgt = z[r * (long)V + t_idx]; }
     }
     __syncthreads();                           // every thread has taken its groups out of the slot ...
-    if (tid == 0 && r + KD_SLOTS * stride < N) issue(r + KD_SLOTS * stride, sidx);      // ... so a later row can land in it
+    if (tid == 0 && r + KD_SLOTS * stride < n) issue(r + KD_SLOTS * stride, sidx);      // ... so a later row can land in it
 
     // phase 1: row maxima
     float my = -INFINITY, mz = -INFINITY;
@@ -465,14 +483,21 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
       }
     }
   }
+  for (long r = n + blockIdx.x; r < N; r += gridDim.x) {       // rows past a variable-length batch (none otherwise)
+    const float zero[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    for (int g = tid; g < groups; g += KDR_THREADS) RowS<TS>::store(dy + r * ld + g * 8, zero);
+    if (tid == 0) { row_kl[r] = 0.f; row_ce[r] = 0.f; }
+  }
 }
 
 template <typename TS, int NCH, bool TEMP4>
 __global__ void __launch_bounds__(KDR_THREADS, (NCH <= 3 ? 3 : (NCH <= 5 ? 2 : 1)))
 kd_token_loss_pipe_kernel(const TS* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
                           long N, int V, float inv_temp, float temperature, float kd_coef, float w_ce, const int* __restrict__ n_valid_ptr,
-                          TS* __restrict__ dy, float* __restrict__ row_kl, float* __restrict__ row_ce) {
-  kd_token_pipe_body<TS, NCH, TEMP4, false>(y, z, tgt, N, V, V, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce);
+                          TS* __restrict__ dy, float* __restrict__ row_kl, float* __restrict__ row_ce,
+                          const int* __restrict__ steps, long rows_per_step, float kd_num) {
+  kd_token_pipe_body<TS, NCH, TEMP4, false>(y, z, tgt, N, V, V, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce,
+                                            steps, rows_per_step, kd_num);
 }
 
 // The form for bf16 rows of any length (V % 8 != 0 or unaligned logits) with dlogits of pitch ld (ld % 8 == 0).
@@ -481,8 +506,9 @@ __global__ void __launch_bounds__(KDR_THREADS, (NCH <= 3 ? 3 : (NCH <= 5 ? 2 : 1
 kd_token_loss_pipe_unaligned_kernel(const bf16* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
                                     long N, int V, long ld, float inv_temp, float temperature, float kd_coef, float w_ce,
                                     const int* __restrict__ n_valid_ptr, bf16* __restrict__ dy, float* __restrict__ row_kl,
-                                    float* __restrict__ row_ce) {
-  kd_token_pipe_body<bf16, NCH, TEMP4, true>(y, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce);
+                                    float* __restrict__ row_ce, const int* __restrict__ steps, long rows_per_step, float kd_num) {
+  kd_token_pipe_body<bf16, NCH, TEMP4, true>(y, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce,
+                                             steps, rows_per_step, kd_num);
 }
 
 // validate_student_model's monitoring metric (reference src/distillation_utils.py:398-409, compute_bleu_score): per sample,
@@ -523,7 +549,8 @@ aux_loss_kernel(const TF* __restrict__ fs, const float* __restrict__ ft, int n_f
                 const TH* __restrict__ hs, const float* __restrict__ ht, int n_hid_rows /*Th*B*/, int n_all_rows /*T*B*/,
                 int H, int Th, float beta, float gamma,
                 float* __restrict__ dfs, float* __restrict__ dft, TH* __restrict__ dhs,
-                float* __restrict__ feat_part /*B*2*/, float* __restrict__ hid_part /*n_hid_rows*2*/) {
+                float* __restrict__ feat_part /*B*2*/, float* __restrict__ hid_part /*n_hid_rows*2*/,
+                const int* __restrict__ steps /* null, or the device step count of a variable-length batch */) {
   extern __shared__ __align__(16) float sm[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarp = blockDim.x >> 5;
   if ((int)blockIdx.x < n_feat_blocks) {
@@ -644,8 +671,13 @@ aux_loss_kernel(const TF* __restrict__ fs, const float* __restrict__ ft, int n_f
     if (row >= n_all_rows) return;
     const TH* s = hs + row * H;
     TH* d = dhs ? dhs + row * H : nullptr;
-    if (row >= n_hid_rows) {                     // student steps beyond the teacher's list: no loss, zero grad
+    // variable-length batch: the teacher's list and the student's steps end at *steps; the steps past it are not read, have no
+    // loss (zero partials) and a zero gradient, and the mean over steps divides by the steps that are left
+    int th = Th;
+    if (steps != nullptr) th = min(Th, max(__ldg(steps), 0));
+    if (row >= (long)th * B) {                   // student steps beyond the teacher's list: no loss, zero grad
       if (d) for (int h = lane; h < H; h += 32) d[h] = from_f<TH>(0.f);
+      if (row < n_hid_rows && lane == 0) { hid_part[row * 2] = 0.f; hid_part[row * 2 + 1] = 0.f; }
       return;
     }
     const float* t = ht + row * H;
@@ -673,8 +705,8 @@ aux_loss_kernel(const TF* __restrict__ fs, const float* __restrict__ ft, int n_f
     const float cosv = dot * inv_norm;
     if (lane == 0) { hid_part[row * 2] = sq; hid_part[row * 2 + 1] = 1.0f - cosv; }
     if (d) {
-      const float c_mse = gamma / (float)Th * 0.7f * 2.0f / ((float)B * (float)H);
-      const float c_cos = gamma / (float)Th * 0.3f / (float)B;
+      const float c_mse = gamma / (float)th * 0.7f * 2.0f / ((float)B * (float)H);
+      const float c_cos = gamma / (float)th * 0.3f / (float)B;
       if (in_regs) {
         const float k_a = cosv / nse;
 #pragma unroll
@@ -702,7 +734,8 @@ __global__ void __launch_bounds__(1024)
 loss_finalize_kernel(const float* __restrict__ row_kl, const float* __restrict__ row_ce, long N, const int* __restrict__ n_valid_ptr,
                      const float* __restrict__ feat_part, int B, int E, int has_feat,
                      const float* __restrict__ hid_part, long n_hid_rows, int H, int Th, int has_hid,
-                     float temperature, float alpha, float beta, float gamma, float w_ce, float ce_mult, float* __restrict__ out5) {
+                     float temperature, float alpha, float beta, float gamma, float w_ce, float ce_mult, float* __restrict__ out5,
+                     const int* __restrict__ steps /* null, or the device step count: token KD over steps*B rows, hidden KD over min(Th, steps) steps */) {
   __shared__ double red[32][5];
   double kl = 0, ce = 0, fg = 0, fa = 0, hm = 0, hc = 0;
   for (long i = threadIdx.x; i < N; i += blockDim.x) { kl += row_kl[i]; ce += row_ce[i]; }
@@ -716,10 +749,12 @@ loss_finalize_kernel(const float* __restrict__ row_kl, const float* __restrict__
     double s[5] = {0, 0, 0, 0, 0};
     for (int w = 0; w < (int)(blockDim.x >> 5); ++w) for (int k = 0; k < 5; ++k) s[k] += red[w][k];
     const int nv = *n_valid_ptr;
-    const double kd_l = (double)temperature * temperature * s[0] / (double)N;
+    long n = N; int th = Th;                   // the partials of rows / steps past a variable-length batch are zeros
+    if (steps != nullptr) { n = min(N, (long)*steps * B); th = min(Th, *steps); }
+    const double kd_l = (double)temperature * temperature * s[0] / (double)n;
     const double ce_l = s[1] * (double)ce_mult / (double)nv;                       // 0/0 -> NaN like the reference when every target is PAD
     const double ft_l = has_feat ? s[2] / ((double)B * E) : 0.0;
-    const double hd_l = has_hid ? (0.7 * s[3] / ((double)B * H) + 0.3 * s[4] / (double)B) / (double)Th : 0.0;
+    const double hd_l = has_hid ? (0.7 * s[3] / ((double)B * H) + 0.3 * s[4] / (double)B) / (double)th : 0.0;
     out5[0] = (float)((double)w_ce * ce_l + (double)alpha * kd_l + (double)beta * ft_l + (double)gamma * hd_l);
     out5[1] = (float)ce_l; out5[2] = (float)kd_l; out5[3] = (float)ft_l; out5[4] = (float)hd_l;
   }

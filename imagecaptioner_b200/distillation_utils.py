@@ -63,7 +63,9 @@ class DistillationLoss(nn.Module):
             hid_s = hid_t = None
         if feats_s is None or feats_t is None:
             feats_s = feats_t = None
-        cfg = (alpha, beta, gamma, temperature, w_ce, float(self.world_size), self.process_group, self.n_valid_global, self.assume_unit_grad)
+        opts = getattr(self, "b2c_options", None)           # GraphedKDStep(max_steps=...): the variable-length batch's step count
+        cfg = (alpha, beta, gamma, temperature, w_ce, float(self.world_size), self.process_group, self.n_valid_global, self.assume_unit_grad,
+               getattr(opts, "steps_dev", None))
         return _ops.KDLossFunction.apply(logits, teacher_logits, targets, feats_s, feats_t, hid_s, hid_t, cfg)
 
     def forward_device(self, student_outputs, teacher_outputs, targets):

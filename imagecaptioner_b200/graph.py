@@ -12,6 +12,11 @@ the whole flat buffer precedes ``optimizer.step()``).
 
 The step structure is the reference's training loop body (src/train_student_kd.py:262-303) with the encoders
 outside the path: the caller provides encoder features, captions, targets and the teacher's outputs.
+
+Variable-length batches (``max_steps=T_cap``): the reference's loader pads every batch to its own longest caption, so T changes
+from batch to batch.  The graph is then captured once with (T_cap, B, ...) buffers and a device step count; ``load()`` takes any
+batch with 1 <= T <= T_cap and the replay computes exactly the loss, gradients and update of that T-step batch (padding the batch
+to T_cap instead would not: token KD is a mean over all T*B rows and hidden KD a mean over steps).
 """
 from __future__ import annotations
 
@@ -26,10 +31,11 @@ from .ddp import FlatGradAllReducer
 
 class GraphedKDStep:
     INPUT_KEYS = ("encoder_features", "captions_input", "targets", "teacher_logits", "teacher_features", "teacher_hiddens")
+    TIME_KEYS = ("captions_input", "targets", "teacher_logits", "teacher_hiddens")      # (T, B, ...): the time axis first
 
     def __init__(self, model, projector, loss_module, optimizer, reducer: Optional[FlatGradAllReducer], example: Dict[str, torch.Tensor],
                  max_grad_norm: float = 1.0, autocast_dtype: Optional[torch.dtype] = torch.bfloat16, use_graph: bool = True,
-                 warmup_steps: int = 3, direct_grads: bool = True):
+                 warmup_steps: int = 3, direct_grads: bool = True, max_steps: Optional[int] = None):
         self.model, self.projector, self.loss_module = model, projector, loss_module
         self._native_opt = hasattr(optimizer, "flat_param") and hasattr(optimizer, "reducer")     # optim.FlatAdamW
         if self._native_opt:
@@ -44,7 +50,27 @@ class GraphedKDStep:
             optimizer.fold_average(reducer.world_size)
         self.max_grad_norm = max_grad_norm
         self.autocast_dtype = autocast_dtype
-        self.static = {k: example[k].clone() for k in self.INPUT_KEYS if example.get(k) is not None}
+        # max_steps: static (max_steps, B, ...) buffers and a device step count (steps[0] = T of the loaded batch) that the decoder
+        # and the loss read at replay time (CallOptions.steps_dev); None: buffers of the example's shape, every batch that shape
+        self.max_steps = max_steps
+        self.steps = None
+        if max_steps is None:
+            self.static = {k: example[k].clone() for k in self.INPUT_KEYS if example.get(k) is not None}
+        else:
+            T = example["captions_input"].shape[0]
+            if not 1 <= T <= max_steps:
+                raise ValueError(f"the example batch has T={T} steps, max_steps={max_steps}")
+            self.static = {}
+            for k in self.INPUT_KEYS:
+                src = example.get(k)
+                if src is None:
+                    continue
+                if k in self.TIME_KEYS:
+                    self.static[k] = torch.zeros((max_steps,) + tuple(src.shape[1:]), dtype=src.dtype, device=src.device)
+                else:
+                    self.static[k] = src.clone()
+            self.steps = torch.zeros(1, dtype=torch.int32, device=example["targets"].device)
+            self.load(example, non_blocking=False)
         self.static["encoder_features"].requires_grad_(True)
         self.out5 = None
         self.graph = None          # forward + loss + backward (+ clip + AdamW when there is a single rank)
@@ -67,7 +93,7 @@ class GraphedKDStep:
         # duration of this object's own forward/backward (see _fwd_bwd), so an eager loop on the same model is unaffected.
         dev = self.static["targets"].device
         self.step_counter = torch.zeros(1, dtype=torch.int64, device=dev)
-        self._opts = _ops.CallOptions(grad_dest=reducer.grad_views() if direct_grads else None, seed_dev=self.step_counter)
+        self._opts = _ops.CallOptions(grad_dest=reducer.grad_views() if direct_grads else None, seed_dev=self.step_counter, steps_dev=self.steps)
         # Data parallel: NCCL stays OUTSIDE the graphs (graph 1 = forward + loss + backward, graph 2 = clip + AdamW); the two
         # exchanges (non-PAD count, flat gradient buffer) are issued eagerly around / alongside graph 1, see overlap_comm below.
         # B2C_FAKE_DP=1: exercise the multi-rank control flow (two graphs, overlapped exchanges) on ONE GPU with an identity in
@@ -134,6 +160,8 @@ class GraphedKDStep:
         o.background_ctas = self.background_ctas if self._overlap else 0
         for m in self._modules():
             m.b2c_options = o
+        if self.steps is not None:
+            self.loss_module.b2c_options = o        # the KD loss reads steps_dev (rows / steps past it: no loss, zero gradient)
 
     def _after_decoder_backward(self):
         """Runs right behind b2c_decoder_backward (autograd thread, capture stream).  The communication stream may start the
@@ -154,6 +182,8 @@ class GraphedKDStep:
     def _detach_options(self):
         for m in self._modules():
             m.b2c_options = None
+        if self.steps is not None:
+            self.loss_module.b2c_options = None
 
     def release(self):
         """Drop the graphs and every hook this object attached (the model can then be trained eagerly, e.g. with gradient
@@ -277,13 +307,38 @@ class GraphedKDStep:
         self._capturing = False
 
     def load(self, batch: Dict[str, torch.Tensor], non_blocking: bool = True) -> int:
-        """Copy one step's inputs (host or device tensors) into the static buffers; returns the bytes copied."""
+        """Copy one step's inputs (host or device tensors) into the static buffers; returns the bytes copied.
+
+        With max_steps: a batch of any T <= max_steps steps (captions_input, targets, teacher_logits and teacher_hiddens all of T
+        steps).  It fills steps [0, T) of the time-indexed buffers, writes PAD (0) into the caption and target steps past T (they
+        then add nothing to the non-PAD count), leaves the teacher's steps past T as they are (never read) and sets the device step
+        count to T, all on the current stream."""
+        if self.max_steps is None:
+            n = 0
+            with torch.no_grad():
+                for k, dst in self.static.items():
+                    src = batch[k]
+                    dst.copy_(src, non_blocking=non_blocking)
+                    n += src.numel() * src.element_size()
+            return n
+        T = int(batch["captions_input"].shape[0])
+        if not 1 <= T <= self.max_steps:
+            raise ValueError(f"batch of T={T} steps: this GraphedKDStep takes 1 <= T <= max_steps={self.max_steps}")
+        for k in self.TIME_KEYS:
+            if k in self.static and batch[k].shape[0] != T:
+                raise ValueError(f"{k} has {batch[k].shape[0]} steps, captions_input {T}")
         n = 0
         with torch.no_grad():
             for k, dst in self.static.items():
                 src = batch[k]
-                dst.copy_(src, non_blocking=non_blocking)
+                if k in self.TIME_KEYS:
+                    dst[:T].copy_(src, non_blocking=non_blocking)
+                    if k in ("captions_input", "targets") and T < self.max_steps:
+                        dst[T:].zero_()
+                else:
+                    dst.copy_(src, non_blocking=non_blocking)
                 n += src.numel() * src.element_size()
+            self.steps.fill_(T)
         return n
 
     def step(self) -> torch.Tensor:

@@ -17,6 +17,8 @@
  *   b2c_count_valid       <- CrossEntropyLoss(ignore_index=0) normaliser  src/distillation_utils.py:22
  *   b2c_kd_token_loss     <- token_level_distillation :30-54 + CE term :154 (+ their gradient)
  *   b2c_kd_token_loss_pitched / b2c_decoder_backward_pitched <- the same two calls with the logits gradient at a padded row pitch
+ *   *_steps               <- the training calls for a batch of fewer steps than shape->T (data_loader.py pads each batch to its own
+ *                            longest caption): a device step count, so one CUDA graph serves every caption length
  *   b2c_kd_token_eval     <- validate_student_model: loss without gradients + logits.argmax(-1)   src/train_student_kd.py:29-86
  *   b2c_bleu1             <- compute_bleu_score (per sample, on the device)                       src/distillation_utils.py:398-409
  *   b2c_aux_loss          <- encoder_feature_distillation :56-94 + decoder_hidden_state_distillation :96-136
@@ -154,6 +156,28 @@ int b2c_decoder_backward_pitched(const B2CShape* shape, const B2CParams* params,
                                  const B2CGrads* grads, float* dfeats, void* workspace, size_t ws_bytes,
                                  int dtype, const B2CDropout* dropout, int flags, void* stream);
 
+/* ---- Variable-length batches.  The *_steps entry points take `steps`, a device int32 scalar with 1 <= *steps <= shape->T (NULL
+ * means shape->T): the buffers keep their shape->T-step layout, and the call computes what the plain call computes for a batch of
+ * the first *steps steps.  The value is read by the kernels when they run, so a CUDA graph captured once at a capacity T replays
+ * for any length up to it.  It must be written before the call on `stream` and not change until the call's work is complete.
+ *   - forward: the rows of steps >= *steps of logits are unspecified, those of hidden_top and attn_w are zeros;
+ *   - backward: the rows of steps >= *steps of dlogits and dhidden_top must be zeros (b2c_kd_token_loss_steps and b2c_aux_loss_steps
+ *     write them so); the gradients are those of the *steps-step batch;
+ *   - the recurrences launch their per-step kernels for all shape->T steps, and the ones past *steps return at once; the
+ *     whole-sequence recurrence kernels (B2C_PERSISTENT, B2C_CLUSTER), sub-batch streams (B2C_SUB_BATCHES) and weight-gradient
+ *     chunks under the reverse loop (B2C_WGRAD_CHUNKS) are not used. */
+int b2c_decoder_forward_steps(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                              void* logits, void* hidden_top, float* attn_w, void* workspace, size_t ws_bytes,
+                              int dtype, const B2CDropout* dropout, const int32_t* steps, void* stream);
+int b2c_decoder_forward_prepared_steps(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                                       void* logits, void* hidden_top, float* attn_w, void* workspace, size_t ws_bytes,
+                                       int dtype, const B2CDropout* dropout, const int32_t* steps, void* stream);
+/* b2c_decoder_backward_pitched with a step count (ld_dlogits == V: contiguous dlogits). */
+int b2c_decoder_backward_steps(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                               const void* hidden_top, const float* attn_w, const void* dlogits, int64_t ld_dlogits, const void* dhidden_top,
+                               const B2CGrads* grads, float* dfeats, void* workspace, size_t ws_bytes,
+                               int dtype, const B2CDropout* dropout, int flags, const int32_t* steps, void* stream);
+
 /* b2c_decoder_backward contracts every weight gradient on an internal (per-device) side stream next to the chain that produces
  * dfeats, and by default makes `stream` wait for that branch before it returns ("all work is enqueued on stream").  A caller that
  * does not read parameter gradients until later (an optimizer step after the rest of the backward) passes
@@ -237,6 +261,15 @@ int b2c_kd_token_loss_pitched(const void* student_logits, const float* teacher_l
                               int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
                               const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype, void* stream);
 
+/* b2c_kd_token_loss_pitched with a step count over N = T * rows_per_step rows (rows_per_step = B): the n = *steps * rows_per_step
+ * first rows are computed with the KD scale alpha*Temp/n; the rows past them are never used (a few bytes of row n may be fetched with
+ * the last row's enclosing 16-byte range), and get row_kl = row_ce = 0 and a dlogits row of zeros (padding columns included).
+ * The caller keeps the targets of those rows PAD (0), so n_valid (b2c_count_valid over all N rows) is that of the n rows. */
+int b2c_kd_token_loss_steps(const void* student_logits, const float* teacher_logits, const int64_t* targets,
+                            int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
+                            const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype,
+                            const int32_t* steps, int64_t rows_per_step, void* stream);
+
 /* Evaluation form of the token pass (validate_student_model, src/train_student_kd.py:29-86): the same per-row KL and CE partials,
  * NO gradient, plus (argmax_out != NULL) the teacher-forced prediction argmax_v student_logits[r, v] of every row (lowest index on
  * ties, like torch.argmax) from the same read of the logits -- `student_logits.argmax(dim=-1)` (:74) without a second pass. */
@@ -260,10 +293,22 @@ int b2c_aux_loss(const void* feats_s, const float* feats_t, int32_t B, int32_t S
                  float beta, float gamma, float* dfeats_s, float* dfeats_t, void* dhid_s,
                  float* feat_part, float* hid_part, int dtype, int feat_dtype, void* stream);
 
+/* b2c_aux_loss with a step count: hidden KD over the first min(Th, *steps) steps (the steps past them are not read, get zero
+ * partials and a zero dhid_s, and the mean over steps divides by min(Th, *steps)); feature KD is unchanged. */
+int b2c_aux_loss_steps(const void* feats_s, const float* feats_t, int32_t B, int32_t Ss, int32_t St, int32_t E,
+                       const void* hid_s, const float* hid_t, int32_t T, int32_t Th, int32_t H,
+                       float beta, float gamma, float* dfeats_s, float* dfeats_t, void* dhid_s,
+                       float* feat_part, float* hid_part, int dtype, int feat_dtype, const int32_t* steps, void* stream);
+
 /* out5 = { total, ce, token_kd, feature_kd, hidden_kd } (device, fp32); fixed-order fp64 reduction. */
 int b2c_loss_finalize(const float* row_kl, const float* row_ce, int64_t N, const int32_t* n_valid, float ce_mult,
                       const float* feat_part, int32_t B, int32_t E, const float* hid_part, int32_t Th, int32_t H,
                       float temperature, float alpha, float beta, float gamma, float w_ce, float* out5, void* stream);
+/* b2c_loss_finalize with a step count: token KD divided by *steps * B rows, hidden KD by min(Th, *steps) steps. */
+int b2c_loss_finalize_steps(const float* row_kl, const float* row_ce, int64_t N, const int32_t* n_valid, float ce_mult,
+                            const float* feat_part, int32_t B, int32_t E, const float* hid_part, int32_t Th, int32_t H,
+                            float temperature, float alpha, float beta, float gamma, float w_ce, float* out5, const int32_t* steps,
+                            void* stream);
 
 /* p[i] *= *scale for i < n  (scale is a device fp32 scalar: autograd's grad_output). */
 int b2c_scale_inplace(void* p, int64_t n, int dtype, const float* scale, void* stream);
