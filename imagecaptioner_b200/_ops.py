@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("B2C_LIB") or os.path.join(_HERE, "lib", "libb2c.so")      # B2C_LIB: A/B builds (development only)
 
 B2C_MAX_LAYERS = 4
-B2C_F32, B2C_BF16 = 0, 1
+B2C_F32, B2C_BF16, B2C_F16 = 0, 1, 2          # B2C_F16: teacher operands only
 B2C_WS_TRAIN, B2C_WS_DECODE, B2C_WS_ATTN, B2C_WS_REFINE, B2C_WS_PROJ = 0, 1, 2, 3, 4
 ABI_VERSION = 5
 B2C_BWD_DEFER_JOIN = 1
@@ -93,6 +93,8 @@ SYMBOLS = {
     "b2c_decoder_prepare": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _sz, ctypes.c_int, _vp]),
     "b2c_decoder_set_initial_state": (ctypes.c_int, [_SHP, _vp, _vp, _vp, _sz, ctypes.c_int, _vp]),
     "b2c_decoder_forward_eval": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp, _vp, _vp, _vp, _sz, ctypes.c_int, _vp]),
+    "b2c_decoder_forward_eval_teacher": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, ctypes.c_int, _vp, _f, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                                                        ctypes.c_int, _vp]),
     "b2c_decoder_forward_prepared": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _vp, _sz, ctypes.c_int, _DRP, _vp]),
     "b2c_decoder_backward": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _vp, _GRD, _vp, _vp, _sz, ctypes.c_int, _DRP, ctypes.c_int, _vp]),
     "b2c_decoder_backward_pitched": (ctypes.c_int, [_SHP, _PRM, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _GRD, _vp, _vp, _sz, ctypes.c_int, _DRP, ctypes.c_int, _vp]),
@@ -110,16 +112,22 @@ SYMBOLS = {
     "b2c_refinement_forward_dual": (ctypes.c_int, [_SHP, ctypes.POINTER(B2CRefineParams), _vp, _vp, _vp, _vp, _sz, ctypes.c_int, _DRP, _vp]),
     "b2c_refinement_backward": (ctypes.c_int, [_SHP, ctypes.POINTER(B2CRefineParams), _vp, _vp, ctypes.POINTER(B2CRefineGrads), _vp, _vp, _sz, ctypes.c_int, _DRP, _vp]),
     "b2c_projector_forward": (ctypes.c_int, [_SHP, ctypes.POINTER(B2CProjParams), _vp, _vp, _vp, _sz, ctypes.c_int, _DRP, _vp]),
+    "b2c_projector_forward_teacher": (ctypes.c_int, [_SHP, ctypes.POINTER(B2CProjParams), _vp, ctypes.c_int, _vp, _vp, _sz, ctypes.c_int, _DRP, _vp]),
     "b2c_projector_backward": (ctypes.c_int, [_SHP, ctypes.POINTER(B2CProjParams), _vp, ctypes.POINTER(B2CProjGrads), _vp, _sz, ctypes.c_int, _DRP, _vp]),
     "b2c_count_valid": (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp]),
     "b2c_kd_token_loss": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _f, _f, _f, _vp, _vp, _vp, _vp, ctypes.c_int, _vp]),
     "b2c_kd_token_loss_pitched": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _f, _f, _f, _vp, _vp, _i64, _vp, _vp, ctypes.c_int, _vp]),
     "b2c_kd_token_loss_steps": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _f, _f, _f, _vp, _vp, _i64, _vp, _vp, ctypes.c_int, _vp, _i64, _vp]),
+    "b2c_kd_token_loss_teacher": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _i64, _i32, _f, _f, _f, _f, _vp, _vp, _i64, _vp, _vp, ctypes.c_int,
+                                                 _vp, _i64, _vp]),
     "b2c_kd_token_eval": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _f, _vp, _vp, _vp, _vp, ctypes.c_int, _vp]),
+    "b2c_kd_token_eval_teacher": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _i64, _i32, _f, _vp, _vp, _vp, _vp, ctypes.c_int, _vp]),
     "b2c_bleu1": (ctypes.c_int, [_vp, _vp, _i32, _i32, _vp, _vp]),
     "b2c_aux_loss": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32, _i32, _f, _f, _vp, _vp, _vp, _vp, _vp, ctypes.c_int, ctypes.c_int, _vp]),
     "b2c_aux_loss_steps": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32, _i32, _f, _f, _vp, _vp, _vp, _vp, _vp, ctypes.c_int, ctypes.c_int,
                                           _vp, _vp]),
+    "b2c_aux_loss_teacher": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, ctypes.c_int, _i32, _i32, _i32, _f, _f, _vp, _vp, _vp, _vp, _vp,
+                                            ctypes.c_int, ctypes.c_int, _vp, _vp]),
     "b2c_loss_finalize": (ctypes.c_int, [_vp, _vp, _i64, _vp, _f, _vp, _i32, _i32, _vp, _i32, _i32, _f, _f, _f, _f, _f, _vp, _vp]),
     "b2c_loss_finalize_steps": (ctypes.c_int, [_vp, _vp, _i64, _vp, _f, _vp, _i32, _i32, _vp, _i32, _i32, _f, _f, _f, _f, _f, _vp, _vp, _vp]),
     "b2c_scale_inplace": (ctypes.c_int, [_vp, _i64, ctypes.c_int, _vp, _vp]),
@@ -177,6 +185,21 @@ def dtype_code(dt: torch.dtype) -> int:
     if dt == torch.bfloat16:
         return B2C_BF16
     raise ValueError(f"unsupported compute dtype {dt} (use torch.float32 or torch.bfloat16)")
+
+
+_TEACHER_CODES = {torch.float32: B2C_F32, torch.bfloat16: B2C_BF16, torch.float16: B2C_F16}
+
+
+def teacher_operand(t: torch.Tensor, device: torch.device):
+    """A teacher tensor (logits, hidden states, features for the projector) as the kernels read it -> (tensor, dtype code).
+    float32, bfloat16 and float16 are read in their own precision and widened exactly in registers, so a half-precision teacher
+    (autocast, or outputs cached in half precision) costs no fp32 copy; the tensor is made contiguous only if it is not.  Any other
+    dtype (float64, ...) is converted to float32."""
+    t = t.detach()
+    code = _TEACHER_CODES.get(t.dtype)
+    if code is None:
+        return t.to(device=device, dtype=torch.float32).contiguous(), B2C_F32
+    return t.to(device=device).contiguous(), code
 
 
 def param_order(L: int) -> List[str]:
@@ -524,7 +547,7 @@ class KDLossFunction(torch.autograd.Function):
         cdt = logits.dtype if logits.dtype in (torch.float32, torch.bfloat16) else torch.float32
         code = dtype_code(cdt)
         y = logits.detach().to(cdt).contiguous()
-        z = teacher_logits.detach().to(device=dev, dtype=torch.float32).contiguous()
+        z, zcode = teacher_operand(teacher_logits, dev)
         tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
         st = _stream()
         if nval_global is not None:                # the caller already holds the (global) non-PAD count on the device
@@ -543,21 +566,13 @@ class KDLossFunction(torch.autograd.Function):
         else:
             Vp = V
             dlogits = dlogits_buf = torch.empty_like(y)
-        if steps is not None:                      # variable-length batch: rows past the step count get zero losses and gradients
-            _check(lib.b2c_kd_token_loss_steps(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), float(alpha), float(w_ce),
-                                               float(ce_mult), nval.data_ptr(), dlogits_buf.data_ptr(), Vp, rows[0].data_ptr(),
-                                               rows[1].data_ptr(), code, steps, B, st), "b2c_kd_token_loss_steps")
-        elif Vp != V:
-            _check(lib.b2c_kd_token_loss_pitched(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), float(alpha), float(w_ce),
-                                                 float(ce_mult), nval.data_ptr(), dlogits_buf.data_ptr(), Vp, rows[0].data_ptr(), rows[1].data_ptr(),
-                                                 code, st), "b2c_kd_token_loss_pitched")
-        else:
-            _check(lib.b2c_kd_token_loss(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), float(alpha), float(w_ce),
-                                         float(ce_mult), nval.data_ptr(), dlogits.data_ptr(), rows[0].data_ptr(), rows[1].data_ptr(), code, st),
-                   "b2c_kd_token_loss")
+        # steps (variable-length batch): rows past the step count get zero losses and gradients; Vp != V: pitched dlogits
+        _check(lib.b2c_kd_token_loss_teacher(y.data_ptr(), z.data_ptr(), zcode, tg.data_ptr(), N, V, float(temperature), float(alpha),
+                                             float(w_ce), float(ce_mult), nval.data_ptr(), dlogits_buf.data_ptr(), Vp, rows[0].data_ptr(),
+                                             rows[1].data_ptr(), code, steps, B, st), "b2c_kd_token_loss_teacher")
         fs = ft = hs = ht = dfs = dft = dhs = feat_part = hid_part = None
         Ss = St = E = H = Th = 0
-        fcode = code
+        fcode, hcode = code, B2C_F32
         if feats_s is not None and feats_t is not None:
             # fp32 student features stay fp32 (the reference's encoder features reach the loss un-cast); otherwise the compute type
             fs = feats_s.detach().contiguous() if feats_s.dtype == torch.float32 else feats_s.detach().to(cdt).contiguous()
@@ -570,17 +585,14 @@ class KDLossFunction(torch.autograd.Function):
             feat_part = torch.empty(B, 2, dtype=torch.float32, device=dev)
         if hid_s is not None and hid_t is not None:
             hs = hid_s.detach().to(cdt).contiguous()
-            ht = hid_t.detach().to(device=dev, dtype=torch.float32).contiguous()
+            ht, hcode = teacher_operand(hid_t, dev)
             Th, H = ht.shape[0], ht.shape[2]
             dhs = torch.empty_like(hs)
             hid_part = torch.empty(Th * B, 2, dtype=torch.float32, device=dev)
         if fs is not None or hs is not None:
-            aux = (_ptr(fs), _ptr(ft), B, Ss, St, E, _ptr(hs), _ptr(ht), hs.shape[0] if hs is not None else 0, Th, H,
-                   float(beta), float(gamma), _ptr(dfs), _ptr(dft), _ptr(dhs), _ptr(feat_part), _ptr(hid_part), code, fcode)
-            if steps is None:
-                _check(lib.b2c_aux_loss(*aux, st), "b2c_aux_loss")
-            else:
-                _check(lib.b2c_aux_loss_steps(*aux, steps, st), "b2c_aux_loss_steps")
+            _check(lib.b2c_aux_loss_teacher(_ptr(fs), _ptr(ft), B, Ss, St, E, _ptr(hs), _ptr(ht), hcode, hs.shape[0] if hs is not None else 0,
+                                            Th, H, float(beta), float(gamma), _ptr(dfs), _ptr(dft), _ptr(dhs), _ptr(feat_part), _ptr(hid_part),
+                                            code, fcode, steps, st), "b2c_aux_loss_teacher")
         out5 = torch.empty(5, dtype=torch.float32, device=dev)
         fin = (rows[0].data_ptr(), rows[1].data_ptr(), N, nval.data_ptr(), float(ce_mult), _ptr(feat_part), B, E,
                _ptr(hid_part), Th, H, float(temperature), float(alpha), float(beta), float(gamma), float(w_ce), out5.data_ptr())
@@ -624,7 +636,7 @@ def _eval_finish(rows, nval, B, feats_s, feats_t, hid_s, hid_t, alpha, beta, gam
     N = rows.shape[1]
     fs = ft = hs = ht = feat_part = hid_part = None
     Ss = St = E = H = Th = 0
-    fcode = code
+    fcode, hcode = code, B2C_F32
     if feats_s is not None and feats_t is not None:
         fs = feats_s.detach().contiguous() if feats_s.dtype == torch.float32 else feats_s.detach().to(cdt).contiguous()
         fcode = dtype_code(fs.dtype)
@@ -634,12 +646,13 @@ def _eval_finish(rows, nval, B, feats_s, feats_t, hid_s, hid_t, alpha, beta, gam
         feat_part = torch.empty(B, 2, dtype=torch.float32, device=dev)
     if hid_s is not None and hid_t is not None:
         hs = hid_s.detach().to(cdt).contiguous()
-        ht = hid_t.detach().to(device=dev, dtype=torch.float32).contiguous()
+        ht, hcode = teacher_operand(hid_t, dev)
         Th, H = ht.shape[0], ht.shape[2]
         hid_part = torch.empty(Th * B, 2, dtype=torch.float32, device=dev)
     if fs is not None or hs is not None:
-        _check(lib.b2c_aux_loss(_ptr(fs), _ptr(ft), B, Ss, St, E, _ptr(hs), _ptr(ht), hs.shape[0] if hs is not None else 0, Th, H,
-                                float(beta), float(gamma), None, None, None, _ptr(feat_part), _ptr(hid_part), code, fcode, st), "b2c_aux_loss")
+        _check(lib.b2c_aux_loss_teacher(_ptr(fs), _ptr(ft), B, Ss, St, E, _ptr(hs), _ptr(ht), hcode, hs.shape[0] if hs is not None else 0, Th, H,
+                                        float(beta), float(gamma), None, None, None, _ptr(feat_part), _ptr(hid_part), code, fcode, None, st),
+               "b2c_aux_loss_teacher")
     out5 = torch.empty(5, dtype=torch.float32, device=dev)
     _check(lib.b2c_loss_finalize(rows[0].data_ptr(), rows[1].data_ptr(), N, nval.data_ptr(), float(ce_mult), _ptr(feat_part), B, E,
                                  _ptr(hid_part), Th, H, float(temperature), float(alpha), float(beta), float(gamma), float(w_ce),
@@ -659,13 +672,13 @@ def kd_eval(logits, teacher_logits, targets, feats_s, feats_t, hid_s, hid_t, alp
     cdt = logits.dtype if logits.dtype in (torch.float32, torch.bfloat16) else torch.float32
     code = dtype_code(cdt)
     y = logits.detach().to(cdt).contiguous()
-    z = teacher_logits.detach().to(device=dev, dtype=torch.float32).contiguous()
+    z, zcode = teacher_operand(teacher_logits, dev)
     tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
     nval = nval_global if nval_global is not None else count_valid(tg, V)
     rows = torch.empty(2, N, dtype=torch.float32, device=dev)
     pred = torch.empty(T, B, dtype=torch.int32, device=dev)
-    _check(lib.b2c_kd_token_eval(y.data_ptr(), z.data_ptr(), tg.data_ptr(), N, V, float(temperature), nval.data_ptr(), rows[0].data_ptr(),
-                                 rows[1].data_ptr(), pred.data_ptr(), code, _stream()), "b2c_kd_token_eval")
+    _check(lib.b2c_kd_token_eval_teacher(y.data_ptr(), z.data_ptr(), zcode, tg.data_ptr(), N, V, float(temperature), nval.data_ptr(),
+                                         rows[0].data_ptr(), rows[1].data_ptr(), pred.data_ptr(), code, _stream()), "b2c_kd_token_eval_teacher")
     out5 = _eval_finish(rows, nval, B, feats_s, feats_t, hid_s, hid_t, alpha, beta, gamma, temperature, w_ce, ce_mult, cdt, code, dev)
     return out5, pred
 
@@ -686,7 +699,7 @@ def decoder_forward_eval(feats: torch.Tensor, captions: torch.Tensor, teacher_lo
     code = B2C_BF16
     f = feats.detach().to(torch.bfloat16).contiguous()
     cap = captions.detach().to(device=dev, dtype=torch.int64).contiguous()
-    z = teacher_logits.detach().to(device=dev, dtype=torch.float32).contiguous()
+    z, zcode = teacher_operand(teacher_logits, dev)
     tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
     if tuple(z.shape) != (T, B, V) or tuple(tg.shape) != (T, B):
         raise ValueError(f"teacher logits {tuple(z.shape)} / targets {tuple(tg.shape)} do not match (T,B,V) = {(T, B, V)}")
@@ -697,9 +710,10 @@ def decoder_forward_eval(feats: torch.Tensor, captions: torch.Tensor, teacher_lo
     rows = torch.empty(2, T * B, dtype=torch.float32, device=dev)
     pred = torch.empty(T, B, dtype=torch.int32, device=dev)
     prm = _fill_struct(B2CParams(), master, L)
-    _check(lib.b2c_decoder_forward_eval(ctypes.byref(shape), ctypes.byref(prm), f.data_ptr(), cap.data_ptr(), z.data_ptr(), tg.data_ptr(),
-                                        float(temperature), hid.data_ptr(), attw.data_ptr(), rows[0].data_ptr(), rows[1].data_ptr(),
-                                        pred.data_ptr(), ws.data_ptr(), ws.numel(), code, _stream()), "b2c_decoder_forward_eval")
+    _check(lib.b2c_decoder_forward_eval_teacher(ctypes.byref(shape), ctypes.byref(prm), f.data_ptr(), cap.data_ptr(), z.data_ptr(), zcode,
+                                                tg.data_ptr(), float(temperature), hid.data_ptr(), attw.data_ptr(), rows[0].data_ptr(),
+                                                rows[1].data_ptr(), pred.data_ptr(), ws.data_ptr(), ws.numel(), code, _stream()),
+           "b2c_decoder_forward_eval_teacher")
     return hid, attw, rows, pred
 
 
@@ -794,15 +808,15 @@ class ProjectorFunction(torch.autograd.Function):
         B, St, Et = x.shape
         shape = B2CShape(B, out_tokens, St, Et, student_dim, 1, 2)
         code = dtype_code(compute_dtype)
-        xf = x.detach().to(torch.float32).contiguous()
+        xt, xcode = teacher_operand(x, x.device)
         master = _master(params)
         prm = _fill_flat(B2CProjParams(), master) if master else B2CProjParams()
         nbytes = workspace_bytes(shape, code, B2C_WS_PROJ) if master else 256
         ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
         out = torch.empty(B, out_tokens, student_dim, dtype=torch.float32, device=x.device)
         drop = _dropout(dropout_p, seed, opts)
-        _check(lib.b2c_projector_forward(ctypes.byref(shape), ctypes.byref(prm), xf.data_ptr(), out.data_ptr(), ws.data_ptr(), ws.numel(),
-                                         code, ctypes.byref(drop), _stream()), "b2c_projector_forward")
+        _check(lib.b2c_projector_forward_teacher(ctypes.byref(shape), ctypes.byref(prm), xt.data_ptr(), xcode, out.data_ptr(), ws.data_ptr(),
+                                                 ws.numel(), code, ctypes.byref(drop), _stream()), "b2c_projector_forward_teacher")
         ctx.b2c = (shape, code, drop, ws, master, [p.dtype for p in params], opts)
         ctx.b2c_params = params
         return out

@@ -510,7 +510,7 @@ int set_initial_state_impl(const B2CShape& s, const float* h0, const float* c0, 
   return 0;
 }
 
-struct EvalOut { const float* teacher; const int64_t* targets; float temperature; float* row_kl; float* row_ce; int* argmax; };
+struct EvalOut { const void* teacher; int teacher_dtype; const int64_t* targets; float temperature; float* row_kl; float* row_ce; int* argmax; };
 
 template <typename T>
 int decoder_forward_impl(const B2CShape& s, const B2CParams& p, const T* feats, const int64_t* cap, T* logits, T* hid_top,
@@ -598,7 +598,7 @@ int decoder_forward_impl(const B2CShape& s, const B2CParams& p, const T* feats, 
     // logits (no logits tensor is written or read back), merged by one small kernel
     GemmArgs gv{(int)TB, V, E, 1.f, 0.f, W.o1, (long)E, 0, W.w.W2, (long)E, 0, nullptr, (long)V, p.out3_b, 0};
     B2C_CHECK_ARG(sizeof(T) == 2 && tc_eligible(gv), "the logits-free validation forward needs bf16 mode and a TMA-describable vocabulary head");
-    EvalEpi ee{ev->teacher, ev->targets, W.evalp, 1.0f / ev->temperature, 0, 0};
+    EvalEpi ee{ev->teacher, ev->targets, W.evalp, 1.0f / ev->temperature, 0, 0, ev->teacher_dtype};
     gv.eval = &ee;
     B2C_TRY((Gemm<T, float>::run(gv, st)));
     kd_eval_combine_kernel<<<cdiv(TB, 8), 256, 0, st>>>(W.evalp, ee.nparts, TB, V, ev->targets, 1.0f / ev->temperature, ev->row_kl, ev->row_ce, ev->argmax);
@@ -1079,15 +1079,15 @@ int check_proj_shape(const B2CShape* s) {
   return 0;
 }
 
-template <typename T>
-int projector_forward_impl(const B2CShape& s, const B2CProjParams& p, const float* x, float* out, void* ws, size_t ws_bytes,
+template <typename T, typename TZ>          // TZ: the teacher features' type (float, bf16 or f16)
+int projector_forward_impl(const B2CShape& s, const B2CProjParams& p, const TZ* x, float* out, void* ws, size_t ws_bytes,
                            const B2CDropout& dr, cudaStream_t st) {
   const bool identity = (p.w == nullptr);
   const int B = s.B, St = s.S, Et = s.E, Es = s.H, So = s.T;
   const long R = (long)B * St;
   if (identity) {
     B2C_CHECK_ARG(Et == Es && !p.b && !p.ln_w && !p.ln_b, "identity projection needs Et == Es and no parameters");
-    pool_fwd_kernel<float><<<ew_grid((long)B * So * Es), 256, 0, st>>>(x, out, B, St, So, Es);
+    pool_fwd_kernel<TZ><<<ew_grid((long)B * So * Es), 256, 0, st>>>(x, out, B, St, So, Es);
     B2C_LAUNCH_CHECK("pool_fwd_kernel");
     return 0;
   }
@@ -1098,7 +1098,7 @@ int projector_forward_impl(const B2CShape& s, const B2CProjParams& p, const floa
   tab.seg[0] = PackSeg{p.w, W.Wp, nullptr, Es, Et, (long)Et, (long)Et, 0};
   pack_params_kernel<T><<<dim3(48, 1), 256, 0, st>>>(tab);
   B2C_LAUNCH_CHECK("pack_params_kernel");
-  cast_f32_kernel<T><<<ew_grid(R * Et / 4), 256, 0, st>>>(x, W.xb, R * Et);
+  cast_f32_kernel<T, TZ><<<ew_grid(R * Et / 4), 256, 0, st>>>(x, W.xb, R * Et);
   B2C_LAUNCH_CHECK("cast_f32_kernel");
   B2C_TRY((gemm<T, T>(st, (int)R, Es, Et, W.xb, Et, 0, W.Wp, Et, 0, W.h, Es, 0.f, p.b, 1)));
   if (dr.p > 0.f) {
@@ -1132,8 +1132,8 @@ int projector_backward_impl(const B2CShape& s, const B2CProjParams& p, const flo
   return 0;
 }
 
-template <typename TS>
-int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, int V, float temperature, float alpha,
+template <typename TS, typename TZ>         // TZ: the teacher logits' type (float, bf16 or f16)
+int kd_token_loss_impl(const TS* y, const TZ* z, const int64_t* tgt, long N, int V, float temperature, float alpha,
                        float w_ce_eff, const int* n_valid, TS* dy, float* row_kl, float* row_ce, cudaStream_t st, int* argmax_out = nullptr,
                        long ld = 0 /* dy pitch; 0 = V */, const int* steps = nullptr, long rows_per_step = 0) {
   if (ld == 0) ld = V;
@@ -1144,7 +1144,7 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
   const float inv_temp = 1.0f / temperature, kd_coef = alpha * temperature / (float)N;
   const float kd_num = alpha * temperature;        // with a device step count the kernels form kd_coef = kd_num / (*steps * rows_per_step)
   // default: persistent CTAs, TMA double-buffered row prefetch, register-resident math (V % 8 == 0, V <= 16384)
-  const size_t psmem = 2 * ((size_t)V * 4 + (size_t)V * sizeof(TS));     // double-buffered row pair; larger rows take the row-in-smem kernel
+  const size_t psmem = 2 * ((size_t)V * sizeof(TZ) + (size_t)V * sizeof(TS));     // double-buffered row pair; larger rows take the row-in-smem kernel
   if (vec && V <= 8 * KDR_THREADS * 8 && !eval && psmem <= 200 * 1024) {
     const int need = cdiv(V / 8, KDR_THREADS);
     int per_sm = (int)((200 * 1024) / (psmem + 1024)); if (per_sm < 1) per_sm = 1;
@@ -1153,8 +1153,8 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
     long grid = (long)sm_count() * per_sm; if (grid > N) grid = N;
 #define B2C_KDP(NCH, T4)                                                                                                   \
   do {                                                                                                                     \
-    B2C_TRY(set_smem(kd_token_loss_pipe_kernel<TS, NCH, T4>, psmem));                                                      \
-    kd_token_loss_pipe_kernel<TS, NCH, T4><<<(unsigned)grid, KDR_THREADS, psmem, st>>>(y, z, tgt, N, V, inv_temp, temperature, kd_coef, w_ce_eff, n_valid, dy, row_kl, row_ce, steps, rows_per_step, kd_num); \
+    B2C_TRY(set_smem(kd_token_loss_pipe_kernel<TS, TZ, NCH, T4>, psmem));                                                  \
+    kd_token_loss_pipe_kernel<TS, TZ, NCH, T4><<<(unsigned)grid, KDR_THREADS, psmem, st>>>(y, z, tgt, N, V, inv_temp, temperature, kd_coef, w_ce_eff, n_valid, dy, row_kl, row_ce, steps, rows_per_step, kd_num); \
   } while (0)
 #define B2C_KDP2(NCH) do { if (t4) B2C_KDP(NCH, true); else B2C_KDP(NCH, false); } while (0)
     switch (need) {
@@ -1169,7 +1169,7 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
   // bf16 rows of any length / alignment with a 16-byte-aligned dy of pitch ld % 8 == 0: the same pipeline on the rows'
   // enclosing 16-byte ranges (slot = the ranges plus one word of read-ahead)
   const int Vp = (V + 7) & ~7;
-  const size_t usmem = 2 * ((size_t)(Vp + 4) * 4 + (size_t)(Vp + 8) * sizeof(TS));
+  const size_t usmem = 2 * ((size_t)(Vp + 16 / sizeof(TZ)) * sizeof(TZ) + (size_t)(Vp + 8) * sizeof(TS));
   if constexpr (sizeof(TS) == 2) if (!vec && !eval && ld % 8 == 0 && ld >= Vp && (uintptr_t)dy % 16 == 0 && V <= 8 * KDR_THREADS * 8 && usmem <= 200 * 1024) {
     const int need = cdiv(Vp / 8, KDR_THREADS);
     int per_sm = (int)((200 * 1024) / (usmem + 1024)); if (per_sm < 1) per_sm = 1;
@@ -1180,8 +1180,8 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
     bf16* dyb = reinterpret_cast<bf16*>(dy);
 #define B2C_KDU(NCH, T4)                                                                                                   \
   do {                                                                                                                     \
-    B2C_TRY(set_smem(kd_token_loss_pipe_unaligned_kernel<NCH, T4>, usmem));                                                \
-    kd_token_loss_pipe_unaligned_kernel<NCH, T4><<<(unsigned)grid, KDR_THREADS, usmem, st>>>(yb, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce_eff, n_valid, dyb, row_kl, row_ce, steps, rows_per_step, kd_num); \
+    B2C_TRY(set_smem(kd_token_loss_pipe_unaligned_kernel<TZ, NCH, T4>, usmem));                                            \
+    kd_token_loss_pipe_unaligned_kernel<TZ, NCH, T4><<<(unsigned)grid, KDR_THREADS, usmem, st>>>(yb, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce_eff, n_valid, dyb, row_kl, row_ce, steps, rows_per_step, kd_num); \
   } while (0)
 #define B2C_KDU2(NCH) do { if (t4) B2C_KDU(NCH, true); else B2C_KDU(NCH, false); } while (0)
     switch (need) {
@@ -1196,8 +1196,8 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
   B2C_CHECK_ARG(ld == V, "dlogits pitch %ld != V=%d needs bf16, a 16-byte-aligned dlogits with pitch %% 8 == 0 and >= roundup(V, 8), and V <= 16384", ld, V);
 #define B2C_KD_LAUNCH(G, T4)                                                                                             \
   do {                                                                                                                   \
-    B2C_TRY(set_smem(kd_token_loss_kernel<TS, G, T4>, smem));                                                            \
-    kd_token_loss_kernel<TS, G, T4><<<(unsigned)N, KD_THREADS, smem, st>>>(y, z, tgt, V, inv_temp, kd_coef, w_ce_eff, n_valid, dy, row_kl, row_ce, argmax_out, steps, rows_per_step, kd_num); \
+    B2C_TRY(set_smem(kd_token_loss_kernel<TS, TZ, G, T4>, smem));                                                        \
+    kd_token_loss_kernel<TS, TZ, G, T4><<<(unsigned)N, KD_THREADS, smem, st>>>(y, z, tgt, V, inv_temp, kd_coef, w_ce_eff, n_valid, dy, row_kl, row_ce, argmax_out, steps, rows_per_step, kd_num); \
   } while (0)
   if (vec && t4) B2C_KD_LAUNCH(8, true);
   else if (vec) B2C_KD_LAUNCH(8, false);
@@ -1208,8 +1208,8 @@ int kd_token_loss_impl(const TS* y, const float* z, const int64_t* tgt, long N, 
   return 0;
 }
 
-template <typename TF, typename TH>
-int aux_loss_impl(const TF* fs, const float* ft, int B, int Ss, int St, int E, const TH* hs, const float* ht, int Tn, int Th, int H,
+template <typename TF, typename TH, typename TZ>
+int aux_loss_impl(const TF* fs, const float* ft, int B, int Ss, int St, int E, const TH* hs, const TZ* ht, int Tn, int Th, int H,
                   float beta, float gamma, float* dfs, float* dft, TH* dhs, float* feat_part, float* hid_part, cudaStream_t st,
                   const int* steps = nullptr) {
   const int nfb = fs ? B : 0;
@@ -1217,11 +1217,20 @@ int aux_loss_impl(const TF* fs, const float* ft, int B, int Ss, int St, int E, c
   const int hid_blocks = (int)((all_rows + 7) / 8);
   if (nfb + hid_blocks == 0) return 0;
   const size_t smem = fs ? (size_t)(2 * Ss + 2 * St + 2 * E + 8 * 2 * E + 8) * 4 : 0;       // + per-warp column partials [8][2][E]
-  B2C_TRY(set_smem(aux_loss_kernel<TF, TH>, smem));
-  aux_loss_kernel<TF, TH><<<nfb + hid_blocks, 256, smem, st>>>(fs, ft, nfb, B, Ss, St, E, hs, ht, (int)((long)Th * B), (int)all_rows, H, Th, beta, gamma,
+  B2C_TRY(set_smem(aux_loss_kernel<TF, TH, TZ>, smem));
+  aux_loss_kernel<TF, TH, TZ><<<nfb + hid_blocks, 256, smem, st>>>(fs, ft, nfb, B, Ss, St, E, hs, ht, (int)((long)Th * B), (int)all_rows, H, Th, beta, gamma,
                                                                dfs, dft, dhs, feat_part, hid_part, steps);
   B2C_LAUNCH_CHECK("aux_loss_kernel");
   return 0;
+}
+
+// Calls f with the teacher data `p` as a pointer to its element type: B2C_F32, B2C_BF16 or B2C_F16.
+template <typename F>
+int with_teacher(const void* p, int teacher_dtype, F&& f) {
+  if (teacher_dtype == B2C_F32) return f(static_cast<const float*>(p));
+  if (teacher_dtype == B2C_BF16) return f(static_cast<const bf16*>(p));
+  if (teacher_dtype == B2C_F16) return f(static_cast<const f16*>(p));
+  return set_err(B2C_EINVAL, "bad teacher dtype %d (B2C_F32, B2C_BF16 or B2C_F16)", teacher_dtype);
 }
 
 }  // namespace
@@ -1293,12 +1302,21 @@ int b2c_decoder_forward_eval(const B2CShape* shape, const B2CParams* params, con
                              const float* teacher_logits, const int64_t* targets, float temperature,
                              void* hidden_top, float* attn_w, float* row_kl, float* row_ce, int32_t* argmax_out,
                              void* workspace, size_t ws_bytes, int dtype, void* stream) {
+  return b2c_decoder_forward_eval_teacher(shape, params, feats, captions, teacher_logits, B2C_F32, targets, temperature, hidden_top, attn_w,
+                                          row_kl, row_ce, argmax_out, workspace, ws_bytes, dtype, stream);
+}
+int b2c_decoder_forward_eval_teacher(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                                     const void* teacher_logits, int teacher_dtype, const int64_t* targets, float temperature,
+                                     void* hidden_top, float* attn_w, float* row_kl, float* row_ce, int32_t* argmax_out,
+                                     void* workspace, size_t ws_bytes, int dtype, void* stream) {
   B2C_TRY(check_shape(shape)); B2C_TRY(check_device());
   B2C_CHECK_ARG(params && feats && captions && teacher_logits && targets && hidden_top && attn_w && row_kl && row_ce && workspace, "NULL argument");
   B2C_CHECK_ARG(temperature > 0.f, "temperature %f", temperature);
   B2C_CHECK_ARG(dtype == B2C_BF16, "the logits-free validation forward is a bf16-mode path (fp32 parity mode keeps the logits)");
+  B2C_CHECK_ARG(teacher_dtype == B2C_F32 || teacher_dtype == B2C_BF16 || teacher_dtype == B2C_F16,
+                "bad teacher dtype %d (B2C_F32, B2C_BF16 or B2C_F16)", teacher_dtype);
   const B2CDropout dr{0.f, 0, nullptr};
-  const EvalOut ev{teacher_logits, targets, temperature, row_kl, row_ce, argmax_out};
+  const EvalOut ev{teacher_logits, teacher_dtype, targets, temperature, row_kl, row_ce, argmax_out};
   return decoder_forward_impl<bf16>(*shape, *params, (const bf16*)feats, captions, (bf16*)nullptr, (bf16*)hidden_top, attn_w, workspace, ws_bytes, dr,
                                     (cudaStream_t)stream, false, &ev);
 }
@@ -1454,14 +1472,20 @@ int b2c_refinement_backward(const B2CShape* shape, const B2CRefineParams* params
 
 int b2c_projector_forward(const B2CShape* shape, const B2CProjParams* params, const float* x, float* out,
                           void* workspace, size_t ws_bytes, int dtype, const B2CDropout* dropout, void* stream) {
+  return b2c_projector_forward_teacher(shape, params, x, B2C_F32, out, workspace, ws_bytes, dtype, dropout, stream);
+}
+int b2c_projector_forward_teacher(const B2CShape* shape, const B2CProjParams* params, const void* x, int teacher_dtype, float* out,
+                                  void* workspace, size_t ws_bytes, int dtype, const B2CDropout* dropout, void* stream) {
   B2C_TRY(check_proj_shape(shape)); B2C_TRY(check_device());
   B2C_CHECK_ARG(params && x && out && workspace, "NULL argument");
   const B2CDropout dr = dropout ? *dropout : B2CDropout{0.f, 0, nullptr};
   B2C_CHECK_ARG(dr.p >= 0.f && dr.p < 1.f, "dropout p=%f outside [0,1)", dr.p);
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B2C_F32) return projector_forward_impl<float>(*shape, *params, x, out, workspace, ws_bytes, dr, st);
-  if (dtype == B2C_BF16) return projector_forward_impl<bf16>(*shape, *params, x, out, workspace, ws_bytes, dr, st);
-  return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+  return with_teacher(x, teacher_dtype, [&](auto xt) {
+    if (dtype == B2C_F32) return projector_forward_impl<float>(*shape, *params, xt, out, workspace, ws_bytes, dr, st);
+    if (dtype == B2C_BF16) return projector_forward_impl<bf16>(*shape, *params, xt, out, workspace, ws_bytes, dr, st);
+    return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+  });
 }
 
 int b2c_projector_backward(const B2CShape* shape, const B2CProjParams* params, const float* dout, const B2CProjGrads* grads,
@@ -1486,52 +1510,60 @@ int b2c_count_valid(const int64_t* targets, int64_t n, int32_t V, int32_t* n_val
 int b2c_kd_token_loss(const void* student_logits, const float* teacher_logits, const int64_t* targets,
                       int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
                       const int32_t* n_valid, void* dlogits, float* row_kl, float* row_ce, int dtype, void* stream) {
-  B2C_TRY(check_device());
-  B2C_CHECK_ARG(student_logits && teacher_logits && targets && n_valid && dlogits && row_kl && row_ce, "NULL argument");
-  B2C_CHECK_ARG(N > 0 && N < 2147483647L && V > 1 && temperature > 0.f, "bad N=%ld V=%d temperature=%f", (long)N, V, temperature);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B2C_F32) return kd_token_loss_impl<float>((const float*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (float*)dlogits, row_kl, row_ce, st);
-  if (dtype == B2C_BF16) return kd_token_loss_impl<bf16>((const bf16*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (bf16*)dlogits, row_kl, row_ce, st);
-  return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+  return b2c_kd_token_loss_teacher(student_logits, teacher_logits, B2C_F32, targets, N, V, temperature, alpha, w_ce, ce_mult, n_valid,
+                                   dlogits, V, row_kl, row_ce, dtype, nullptr, 0, stream);
 }
 
 int b2c_kd_token_loss_pitched(const void* student_logits, const float* teacher_logits, const int64_t* targets,
                               int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
                               const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype, void* stream) {
-  B2C_TRY(check_device());
-  B2C_CHECK_ARG(student_logits && teacher_logits && targets && n_valid && dlogits && row_kl && row_ce, "NULL argument");
-  B2C_CHECK_ARG(N > 0 && N < 2147483647L && V > 1 && temperature > 0.f, "bad N=%ld V=%d temperature=%f", (long)N, V, temperature);
-  B2C_CHECK_ARG(ld_dlogits >= V, "ld_dlogits=%ld < V=%d", (long)ld_dlogits, V);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B2C_F32) return kd_token_loss_impl<float>((const float*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (float*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits);
-  if (dtype == B2C_BF16) return kd_token_loss_impl<bf16>((const bf16*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (bf16*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits);
-  return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+  return b2c_kd_token_loss_teacher(student_logits, teacher_logits, B2C_F32, targets, N, V, temperature, alpha, w_ce, ce_mult, n_valid,
+                                   dlogits, ld_dlogits, row_kl, row_ce, dtype, nullptr, 0, stream);
 }
 
 int b2c_kd_token_loss_steps(const void* student_logits, const float* teacher_logits, const int64_t* targets,
                             int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
                             const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype,
                             const int32_t* steps, int64_t rows_per_step, void* stream) {
+  return b2c_kd_token_loss_teacher(student_logits, teacher_logits, B2C_F32, targets, N, V, temperature, alpha, w_ce, ce_mult, n_valid,
+                                   dlogits, ld_dlogits, row_kl, row_ce, dtype, steps, rows_per_step, stream);
+}
+
+int b2c_kd_token_loss_teacher(const void* student_logits, const void* teacher_logits, int teacher_dtype, const int64_t* targets,
+                              int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
+                              const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype,
+                              const int32_t* steps, int64_t rows_per_step, void* stream) {
   B2C_TRY(check_device());
   B2C_CHECK_ARG(student_logits && teacher_logits && targets && n_valid && dlogits && row_kl && row_ce, "NULL argument");
   B2C_CHECK_ARG(N > 0 && N < 2147483647L && V > 1 && temperature > 0.f, "bad N=%ld V=%d temperature=%f", (long)N, V, temperature);
   B2C_CHECK_ARG(ld_dlogits >= V, "ld_dlogits=%ld < V=%d", (long)ld_dlogits, V);
   B2C_CHECK_ARG(steps == nullptr || (rows_per_step > 0 && N % rows_per_step == 0), "rows_per_step=%ld must divide N=%ld", (long)rows_per_step, (long)N);
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B2C_F32) return kd_token_loss_impl<float>((const float*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (float*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits, steps, (long)rows_per_step);
-  if (dtype == B2C_BF16) return kd_token_loss_impl<bf16>((const bf16*)student_logits, teacher_logits, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (bf16*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits, steps, (long)rows_per_step);
-  return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+  return with_teacher(teacher_logits, teacher_dtype, [&](auto z) {
+    if (dtype == B2C_F32) return kd_token_loss_impl<float>((const float*)student_logits, z, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (float*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits, steps, (long)rows_per_step);
+    if (dtype == B2C_BF16) return kd_token_loss_impl<bf16>((const bf16*)student_logits, z, targets, (long)N, V, temperature, alpha, w_ce * ce_mult, n_valid, (bf16*)dlogits, row_kl, row_ce, st, nullptr, (long)ld_dlogits, steps, (long)rows_per_step);
+    return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+  });
 }
 
 int b2c_kd_token_eval(const void* student_logits, const float* teacher_logits, const int64_t* targets, int64_t N, int32_t V,
                       float temperature, const int32_t* n_valid, float* row_kl, float* row_ce, int32_t* argmax_out, int dtype, void* stream) {
+  return b2c_kd_token_eval_teacher(student_logits, teacher_logits, B2C_F32, targets, N, V, temperature, n_valid, row_kl, row_ce, argmax_out,
+                                   dtype, stream);
+}
+
+int b2c_kd_token_eval_teacher(const void* student_logits, const void* teacher_logits, int teacher_dtype, const int64_t* targets, int64_t N,
+                              int32_t V, float temperature, const int32_t* n_valid, float* row_kl, float* row_ce, int32_t* argmax_out,
+                              int dtype, void* stream) {
   B2C_TRY(check_device());
   B2C_CHECK_ARG(student_logits && teacher_logits && targets && n_valid && row_kl && row_ce, "NULL argument");
   B2C_CHECK_ARG(N > 0 && N < 2147483647L && V > 1 && temperature > 0.f, "bad N=%ld V=%d temperature=%f", (long)N, V, temperature);
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B2C_F32) return kd_token_loss_impl<float>((const float*)student_logits, teacher_logits, targets, (long)N, V, temperature, 0.f, 0.f, n_valid, (float*)nullptr, row_kl, row_ce, st, argmax_out);
-  if (dtype == B2C_BF16) return kd_token_loss_impl<bf16>((const bf16*)student_logits, teacher_logits, targets, (long)N, V, temperature, 0.f, 0.f, n_valid, (bf16*)nullptr, row_kl, row_ce, st, argmax_out);
-  return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+  return with_teacher(teacher_logits, teacher_dtype, [&](auto z) {
+    if (dtype == B2C_F32) return kd_token_loss_impl<float>((const float*)student_logits, z, targets, (long)N, V, temperature, 0.f, 0.f, n_valid, (float*)nullptr, row_kl, row_ce, st, argmax_out);
+    if (dtype == B2C_BF16) return kd_token_loss_impl<bf16>((const bf16*)student_logits, z, targets, (long)N, V, temperature, 0.f, 0.f, n_valid, (bf16*)nullptr, row_kl, row_ce, st, argmax_out);
+    return set_err(B2C_EINVAL, "bad dtype %d", dtype);
+  });
 }
 
 int b2c_bleu1(const int32_t* predicted, const int64_t* targets, int32_t T, int32_t B, float* bleu_out, void* stream) {
@@ -1546,30 +1578,33 @@ int b2c_aux_loss(const void* feats_s, const float* feats_t, int32_t B, int32_t S
                  const void* hid_s, const float* hid_t, int32_t T, int32_t Th, int32_t H,
                  float beta, float gamma, float* dfeats_s, float* dfeats_t, void* dhid_s,
                  float* feat_part, float* hid_part, int dtype, int feat_dtype, void* stream) {
-  B2C_TRY(check_device());
-  B2C_CHECK_ARG(B > 0, "B=%d", B);
-  if (feats_s) B2C_CHECK_ARG(feats_t && feat_part && Ss > 0 && St > 0 && E > 0 && E % 8 == 0, "feature KD needs feats_t, feat_part, positive Ss/St and E a positive multiple of 8 (E=%d)", E);
-  if (hid_s) B2C_CHECK_ARG(hid_t && hid_part && T > 0 && Th > 0 && Th <= T && H > 0 && H % 8 == 0, "hidden KD needs hid_t, hid_part, 0 < Th <= T and H a positive multiple of 8 (H=%d)", H);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B2C_F32 && feat_dtype == B2C_F32) return aux_loss_impl<float, float>((const float*)feats_s, feats_t, B, Ss, St, E, (const float*)hid_s, hid_t, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (float*)dhid_s, feat_part, hid_part, st);
-  if (dtype == B2C_BF16 && feat_dtype == B2C_BF16) return aux_loss_impl<bf16, bf16>((const bf16*)feats_s, feats_t, B, Ss, St, E, (const bf16*)hid_s, hid_t, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (bf16*)dhid_s, feat_part, hid_part, st);
-  if (dtype == B2C_BF16 && feat_dtype == B2C_F32) return aux_loss_impl<float, bf16>((const float*)feats_s, feats_t, B, Ss, St, E, (const bf16*)hid_s, hid_t, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (bf16*)dhid_s, feat_part, hid_part, st);
-  return set_err(B2C_EINVAL, "bad dtype %d / feature dtype %d", dtype, feat_dtype);
+  return b2c_aux_loss_teacher(feats_s, feats_t, B, Ss, St, E, hid_s, hid_t, B2C_F32, T, Th, H, beta, gamma, dfeats_s, dfeats_t, dhid_s,
+                              feat_part, hid_part, dtype, feat_dtype, nullptr, stream);
 }
 
 int b2c_aux_loss_steps(const void* feats_s, const float* feats_t, int32_t B, int32_t Ss, int32_t St, int32_t E,
                        const void* hid_s, const float* hid_t, int32_t T, int32_t Th, int32_t H,
                        float beta, float gamma, float* dfeats_s, float* dfeats_t, void* dhid_s,
                        float* feat_part, float* hid_part, int dtype, int feat_dtype, const int32_t* steps, void* stream) {
+  return b2c_aux_loss_teacher(feats_s, feats_t, B, Ss, St, E, hid_s, hid_t, B2C_F32, T, Th, H, beta, gamma, dfeats_s, dfeats_t, dhid_s,
+                              feat_part, hid_part, dtype, feat_dtype, steps, stream);
+}
+
+int b2c_aux_loss_teacher(const void* feats_s, const float* feats_t, int32_t B, int32_t Ss, int32_t St, int32_t E,
+                         const void* hid_s, const void* hid_t, int hid_t_dtype, int32_t T, int32_t Th, int32_t H,
+                         float beta, float gamma, float* dfeats_s, float* dfeats_t, void* dhid_s,
+                         float* feat_part, float* hid_part, int dtype, int feat_dtype, const int32_t* steps, void* stream) {
   B2C_TRY(check_device());
   B2C_CHECK_ARG(B > 0, "B=%d", B);
   if (feats_s) B2C_CHECK_ARG(feats_t && feat_part && Ss > 0 && St > 0 && E > 0 && E % 8 == 0, "feature KD needs feats_t, feat_part, positive Ss/St and E a positive multiple of 8 (E=%d)", E);
   if (hid_s) B2C_CHECK_ARG(hid_t && hid_part && T > 0 && Th > 0 && Th <= T && H > 0 && H % 8 == 0, "hidden KD needs hid_t, hid_part, 0 < Th <= T and H a positive multiple of 8 (H=%d)", H);
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B2C_F32 && feat_dtype == B2C_F32) return aux_loss_impl<float, float>((const float*)feats_s, feats_t, B, Ss, St, E, (const float*)hid_s, hid_t, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (float*)dhid_s, feat_part, hid_part, st, steps);
-  if (dtype == B2C_BF16 && feat_dtype == B2C_BF16) return aux_loss_impl<bf16, bf16>((const bf16*)feats_s, feats_t, B, Ss, St, E, (const bf16*)hid_s, hid_t, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (bf16*)dhid_s, feat_part, hid_part, st, steps);
-  if (dtype == B2C_BF16 && feat_dtype == B2C_F32) return aux_loss_impl<float, bf16>((const float*)feats_s, feats_t, B, Ss, St, E, (const bf16*)hid_s, hid_t, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (bf16*)dhid_s, feat_part, hid_part, st, steps);
-  return set_err(B2C_EINVAL, "bad dtype %d / feature dtype %d", dtype, feat_dtype);
+  return with_teacher(hid_t, hid_t_dtype, [&](auto ht) {
+    if (dtype == B2C_F32 && feat_dtype == B2C_F32) return aux_loss_impl<float, float>((const float*)feats_s, feats_t, B, Ss, St, E, (const float*)hid_s, ht, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (float*)dhid_s, feat_part, hid_part, st, steps);
+    if (dtype == B2C_BF16 && feat_dtype == B2C_BF16) return aux_loss_impl<bf16, bf16>((const bf16*)feats_s, feats_t, B, Ss, St, E, (const bf16*)hid_s, ht, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (bf16*)dhid_s, feat_part, hid_part, st, steps);
+    if (dtype == B2C_BF16 && feat_dtype == B2C_F32) return aux_loss_impl<float, bf16>((const float*)feats_s, feats_t, B, Ss, St, E, (const bf16*)hid_s, ht, T, Th, H, beta, gamma, dfeats_s, dfeats_t, (bf16*)dhid_s, feat_part, hid_part, st, steps);
+    return set_err(B2C_EINVAL, "bad dtype %d / feature dtype %d", dtype, feat_dtype);
+  });
 }
 
 int b2c_loss_finalize(const float* row_kl, const float* row_ce, int64_t N, const int32_t* n_valid, float ce_mult,

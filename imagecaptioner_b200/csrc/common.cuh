@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -15,6 +16,7 @@
 namespace b2c {
 
 typedef __nv_bfloat16 bf16;
+typedef __half f16;          // teacher operands only (B2C_F16): the student never computes in fp16
 
 // ------------------------------------------------------------------ errors
 // Thread-local message; every entry point returns 0 or a negative B2C_E* code and never aborts.
@@ -34,6 +36,7 @@ inline unsigned long long& launch_counter() { static unsigned long long n = 0; r
 template <typename T> __device__ __forceinline__ float to_f(T v);
 template <> __device__ __forceinline__ float to_f<float>(float v) { return v; }
 template <> __device__ __forceinline__ float to_f<bf16>(bf16 v) { return __bfloat162float(v); }
+template <> __device__ __forceinline__ float to_f<f16>(f16 v) { return __half2float(v); }
 template <typename T> __device__ __forceinline__ T from_f(float v);
 template <> __device__ __forceinline__ float from_f<float>(float v) { return v; }
 template <> __device__ __forceinline__ bf16 from_f<bf16>(float v) { return __float2bfloat16_rn(v); }
@@ -178,6 +181,15 @@ __device__ __forceinline__ void st_na_v4(void* p, const uint4& v) {
 
 __device__ __forceinline__ float bf16_lo(uint32_t u) { return __uint_as_float(u << 16); }
 __device__ __forceinline__ float bf16_hi(uint32_t u) { return __uint_as_float(u & 0xffff0000u); }
+__device__ __forceinline__ float f16_lo(uint32_t u) { return __half2float(__ushort_as_half((unsigned short)(u & 0xffffu))); }
+__device__ __forceinline__ float f16_hi(uint32_t u) { return __half2float(__ushort_as_half((unsigned short)(u >> 16))); }
+// the two elements of a 32-bit word of a 2-byte type, widened exactly to fp32
+template <typename T> __device__ __forceinline__ float lo_f(uint32_t u);
+template <typename T> __device__ __forceinline__ float hi_f(uint32_t u);
+template <> __device__ __forceinline__ float lo_f<bf16>(uint32_t u) { return bf16_lo(u); }
+template <> __device__ __forceinline__ float hi_f<bf16>(uint32_t u) { return bf16_hi(u); }
+template <> __device__ __forceinline__ float lo_f<f16>(uint32_t u) { return f16_lo(u); }
+template <> __device__ __forceinline__ float hi_f<f16>(uint32_t u) { return f16_hi(u); }
 __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
   __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
   return *reinterpret_cast<uint32_t*>(&v);
@@ -193,6 +205,13 @@ template <> struct Vec8<bf16> {
   }
   static __device__ __forceinline__ void store(bf16* p, const float (&v)[8]) {
     *reinterpret_cast<uint4*>(p) = make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
+  }
+};
+template <> struct Vec8<f16> {                // load only: fp16 is a teacher operand type
+  static __device__ __forceinline__ void load(const f16* p, float (&v)[8]) {
+    const uint4 a = *reinterpret_cast<const uint4*>(p);
+    v[0] = f16_lo(a.x); v[1] = f16_hi(a.x); v[2] = f16_lo(a.y); v[3] = f16_hi(a.y);
+    v[4] = f16_lo(a.z); v[5] = f16_hi(a.z); v[6] = f16_lo(a.w); v[7] = f16_hi(a.w);
   }
 };
 template <> struct Vec8<float> {

@@ -16,6 +16,7 @@
 //                         tcgen05.mma (cta_group::1, M=128, N=64/128/256, K=16) accumulating fp32 in TMEM,
 //                         tcgen05.ld epilogue with fused alpha / bias / ReLU / beta.
 #pragma once
+#include <type_traits>
 #include "common.cuh"
 
 namespace b2c {
@@ -48,8 +49,9 @@ struct LstmEpi {
 //   my, s1 = sum e^{y-my}, sT = sum e^{(y-my)/Temp};  mz, sZ = sum e^{(z-mz)/Temp}, sA = sum e^{(z-mz)/Temp} ((z-mz) - (y-my))/Temp;
 //   y[target] if the target column lies in the part; the part's argmax column (lowest index among equals).
 // kd_eval_combine_kernel (loss_kernels.cuh) merges the parts of a row.  The descriptor travels in the LstmEpi slot: enabled == 3.
+// The teacher logits are fp32 (epilogue flavour 3), bf16 (6) or f16 (7), each its own instantiation (see gemm_tc_kernel).
 constexpr int EVAL_PART_FLOATS = 8;
-struct EvalEpi { const float* teacher; const int64_t* targets; float* parts; float inv_temp; int nparts; int cols_per_part; };
+struct EvalEpi { const void* teacher; const int64_t* targets; float* parts; float inv_temp; int nparts; int cols_per_part; int teacher_dtype; };
 
 // Greedy decoding needs argmax_n C[m, n] only: the vocabulary-head GEMM can reduce every accumulator tile to per-row partial
 // (max, index) pairs in its epilogue instead of writing the logits (41 MB per step at B = 2048, V = 5000, read again by the argmax
@@ -282,7 +284,7 @@ __device__ __forceinline__ uint4 epi_combine_f32(uint4 acc, uint4 old, float bet
 // kernels instead of one with both keep each one's code small: the recurrence's kernels are short and run back to back with
 // other kernels, so every launch starts with a cold instruction cache.
 // EPI selects ONE epilogue flavour per instantiation: 0 = the general store epilogues, 1 = fused LSTM cell, 2 = argmax partials (greedy
-// decode), 3 = validation partials.  Each flavour is its own kernel so none of them carries the others' code: these kernels run back to back
+// decode), 3 = validation partials (6 / 7: the same with bf16 / f16 teacher logits).  Each flavour is its own kernel so none of them carries the others' code: these kernels run back to back
 // with cold instruction caches, and code that is never executed still costs (round 1: 66 -> 23-32 KB per kernel bought 40 us per step;
 // round 2: ~300 inlined instructions of a dropout hash in the general epilogue cost 8 % of the whole step).
 template <int BN, bool A_MN, bool B_MN, typename TC, int EPI = 0>
@@ -518,9 +520,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     } else {
     constexpr int NCHUNK = BN / CH;                      // 128-byte column chunks per tile row
     constexpr int C_PER = (NCHUNK + 1) / 2;
-    if constexpr (EPI == 3) {
+    if constexpr (EPI == 3 || EPI == 6 || EPI == 7) {
       // ---- validation epilogue (EvalEpi): this thread owns one logits row and C_PER * CH columns of it
-      const float* zt = reinterpret_cast<const float*>(le.addend);
+      using TZ = typename std::conditional<EPI == 3, float, typename std::conditional<EPI == 6, bf16, f16>::type>::type;
+      const TZ* zt = reinterpret_cast<const TZ*>(le.addend);
       const int64_t* tg = reinterpret_cast<const int64_t*>(le.h_rec);
       float* parts = le.c_out;
       const int nparts = le.H, grow = m0 + q * 32 + lane;
@@ -537,13 +540,23 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           float v[32], z[32];
           tmem_ld32(tacc + (uint32_t)(ci * CH + h * 32), v);
           const bool full = colb + 32 <= N;
-          const float* zr = zt + (long)(row_ok ? grow : 0) * N + colb;
+          const TZ* zr = zt + (long)(row_ok ? grow : 0) * N + colb;
           if (full && ((((uintptr_t)zr) & 15) == 0)) {
+            if constexpr (sizeof(TZ) == 4) {
 #pragma unroll
-            for (int j = 0; j < 8; ++j) { const float4 t4 = __ldg(reinterpret_cast<const float4*>(zr) + j); z[4 * j] = t4.x; z[4 * j + 1] = t4.y; z[4 * j + 2] = t4.z; z[4 * j + 3] = t4.w; }
+              for (int j = 0; j < 8; ++j) { const float4 t4 = __ldg(reinterpret_cast<const float4*>(zr) + j); z[4 * j] = t4.x; z[4 * j + 1] = t4.y; z[4 * j + 2] = t4.z; z[4 * j + 3] = t4.w; }
+            } else {
+#pragma unroll
+              for (int j = 0; j < 4; ++j) {
+                const uint4 t4 = __ldg(reinterpret_cast<const uint4*>(zr) + j);
+                const uint32_t w[4] = {t4.x, t4.y, t4.z, t4.w};
+#pragma unroll
+                for (int k = 0; k < 4; ++k) { z[8 * j + 2 * k] = lo_f<TZ>(w[k]); z[8 * j + 2 * k + 1] = hi_f<TZ>(w[k]); }
+              }
+            }
           } else {
 #pragma unroll
-            for (int j = 0; j < 32; ++j) z[j] = (colb + j < N) ? __ldg(zr + j) : -INFINITY;
+            for (int j = 0; j < 32; ++j) z[j] = (colb + j < N) ? to_f<TZ>(__ldg(zr + j)) : -INFINITY;
           }
 #pragma unroll
           for (int j = 0; j < 32; ++j) v[j] = (colb + j < N) ? fmaf(alpha, v[j], bias != nullptr ? __ldg(bias + colb + j) : 0.f) : -INFINITY;
@@ -878,6 +891,7 @@ int launch_tc(const GemmArgs& g, const TcPlan& plan, cudaStream_t st) {
   void (*kern)(const CUtensorMap, const CUtensorMap, int, int, int, float, float, TC*, long, const float*, int, int, int, int, int, int, const LstmEpi) =
       gemm_tc_kernel<BN, A_MN, B_MN, TC, 0>;
   int flavour = g.lstm ? ((g.lstm->drop_p > 0.f && g.lstm->h_next) ? 1 : 5) : (g.amax ? 2 : (g.eval ? 3 : 0));
+  if (g.eval && g.eval->teacher_dtype != B2C_F32) flavour = g.eval->teacher_dtype == B2C_BF16 ? 6 : 7;
   if (flavour == 0 && fast_only_enabled() && g.M % TC_BM == 0 && g.N % BN == 0 && (plan.splits > 1 ? sizeof(TC) == 4 : g.beta == 0.f) &&
       ((uintptr_t)g.C) % 16 == 0 && (g.ldc * (long)sizeof(TC)) % 16 == 0 && (((uintptr_t)g.bias) & 15) == 0) {
     flavour = 4;                       // every tile takes the straight-line epilogue: the kernel without the generic path
@@ -886,10 +900,11 @@ int launch_tc(const GemmArgs& g, const TcPlan& plan, cudaStream_t st) {
   if (flavour != 0 && flavour != 4) {
     if constexpr (CAN_LSTM) {
       kern = flavour == 1 ? gemm_tc_kernel<BN, A_MN, B_MN, TC, 1> : (flavour == 5 ? gemm_tc_kernel<BN, A_MN, B_MN, TC, 5> :
-             (flavour == 2 ? gemm_tc_kernel<BN, A_MN, B_MN, TC, 2> : gemm_tc_kernel<BN, A_MN, B_MN, TC, 3>));
+             (flavour == 2 ? gemm_tc_kernel<BN, A_MN, B_MN, TC, 2> : (flavour == 6 ? gemm_tc_kernel<BN, A_MN, B_MN, TC, 6> :
+             (flavour == 7 ? gemm_tc_kernel<BN, A_MN, B_MN, TC, 7> : gemm_tc_kernel<BN, A_MN, B_MN, TC, 3>))));
     } else return set_err(B2C_EINVAL, "the fused LSTM / argmax / validation epilogues need K-major operands and the fp32 instantiation");
   }
-  static bool attr_set[6] = {false, false, false, false, false, false};      // per template instantiation and epilogue flavour
+  static bool attr_set[8] = {false, false, false, false, false, false, false, false};      // per template instantiation and epilogue flavour
   if (!attr_set[flavour]) {
     B2C_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcCfg<BN>::SMEM_BYTES));
     attr_set[flavour] = true;

@@ -63,9 +63,11 @@ __device__ __forceinline__ float block_reduce_sum4(float& a, float& b, float& c,
 //   CE_r  = logsumexp(y) - y[tgt]                       (tgt != PAD)
 //   dy_v  = kd_coef (pS_v - pT_v) + ce_coef (softmax(y)_v - [v == tgt])
 // with kd_coef = alpha*Temp/N and ce_coef = w_ce / n_valid (0 on PAD rows).
-template <typename TS, int G, bool TEMP4>
+// TZ (teacher logits): float, bf16 or f16; a half-precision row is widened exactly to fp32 on its way into shared memory, so the
+// arithmetic is that of the fp32 row.
+template <typename TS, typename TZ, int G, bool TEMP4>
 __global__ void __launch_bounds__(KD_THREADS)
-kd_token_loss_kernel(const TS* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
+kd_token_loss_kernel(const TS* __restrict__ y, const TZ* __restrict__ z, const int64_t* __restrict__ tgt,
                      int V, float inv_temp, float kd_coef, float w_ce, const int* __restrict__ n_valid_ptr,
                      TS* __restrict__ dy /* NULL: losses only (evaluation) */, float* __restrict__ row_kl, float* __restrict__ row_ce,
                      int* __restrict__ argmax_out /* NULL, or (N): argmax_v y[r, v], lowest index on ties like torch.argmax */,
@@ -91,19 +93,29 @@ kd_token_loss_kernel(const TS* __restrict__ y, const float* __restrict__ z, cons
   const int tid = threadIdx.x;
   const long r = blockIdx.x;
   const TS* yg = y + r * (long)V;
-  const float* zg = z + r * (long)V;
+  const TZ* zg = z + r * (long)V;
 
   if (G == 8) {
     if (tid == 0) { mbar_init(&bar, 1); fence_barrier_init(); }
     __syncthreads();
-    if (tid == 0) {
-      mbar_arrive_expect_tx(&bar, (uint32_t)(V * 4 + V * sizeof(TS)));
-      bulk_g2s(zs, zg, (uint32_t)(V * 4), &bar);
-      bulk_g2s(ys, yg, (uint32_t)(V * sizeof(TS)), &bar);
+    if constexpr (sizeof(TZ) == 4) {
+      if (tid == 0) {
+        mbar_arrive_expect_tx(&bar, (uint32_t)(V * 4 + V * sizeof(TS)));
+        bulk_g2s(zs, zg, (uint32_t)(V * 4), &bar);
+        bulk_g2s(ys, yg, (uint32_t)(V * sizeof(TS)), &bar);
+      }
+    } else {
+      // half-precision teacher row: 16-byte loads widened into the fp32 row while the student row's bulk copy is in flight
+      if (tid == 0) {
+        mbar_arrive_expect_tx(&bar, (uint32_t)(V * sizeof(TS)));
+        bulk_g2s(ys, yg, (uint32_t)(V * sizeof(TS)), &bar);
+      }
+      for (int g = tid; g < V / 8; g += KD_THREADS) { float v[8]; Vec8<TZ>::load(zg + g * 8, v); RowIO<float, 8>::store_s(zs, g * 8, v); }
+      __syncthreads();
     }
     mbar_wait(&bar, 0);
   } else {
-    for (int v = tid; v < V; v += KD_THREADS) { zs[v] = zg[v]; ys[v] = yg[v]; }
+    for (int v = tid; v < V; v += KD_THREADS) { zs[v] = to_f<TZ>(zg[v]); ys[v] = yg[v]; }
     __syncthreads();
   }
 
@@ -244,6 +256,13 @@ template <> struct RowS<bf16> {
     st_na_v4(p, make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7])));
   }
 };
+template <> struct RowS<f16> {          // teacher rows only
+  static __device__ __forceinline__ void load(const f16* p, float (&v)[8]) {
+    const uint4 a = *reinterpret_cast<const uint4*>(p);
+    v[0] = f16_lo(a.x); v[1] = f16_hi(a.x); v[2] = f16_lo(a.y); v[3] = f16_hi(a.y);
+    v[4] = f16_lo(a.z); v[5] = f16_hi(a.z); v[6] = f16_lo(a.w); v[7] = f16_hi(a.w);
+  }
+};
 template <> struct RowS<float> {
   static __device__ __forceinline__ void load(const float* p, float (&v)[8]) {
     const float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + 4);
@@ -259,12 +278,13 @@ constexpr int KD_SLOTS = 2;              // row slots per CTA: the TMA prefetch 
 
 // Unaligned rows (V % 8 != 0): row r of y / z starts anywhere inside a 16-byte word.  The bulk copy takes the enclosing
 // 16-byte-aligned byte range, so element v of the row sits at slot index sh + v with sh = the row start's offset inside its
-// word (0..7 bf16, 0..3 fp32).  These rebuild the 8 elements of column group g from the two (bf16) or three (fp32) 16-byte
-// words that hold them; the shift is uniform over the CTA, so the selects below never diverge.
+// word (0..7 bf16 / f16, 0..3 fp32).  These rebuild the 8 elements of column group g from the two (2-byte types) or three (fp32)
+// 16-byte words that hold them; the shift is uniform over the CTA, so the selects below never diverge.
 __device__ __forceinline__ uint32_t pick_word(const uint32_t (&u)[8], int q, int j) {      // u[q + j], q in 0..3
   return q == 0 ? u[j] : (q == 1 ? u[j + 1] : (q == 2 ? u[j + 2] : u[j + 3]));
 }
-__device__ __forceinline__ void load_shifted_bf16(const bf16* slot, int sh, int g, float (&v)[8]) {
+template <typename T>          // bf16 or f16
+__device__ __forceinline__ void load_shifted_h(const T* slot, int sh, int g, float (&v)[8]) {
   const uint4 a = reinterpret_cast<const uint4*>(slot)[g], b = reinterpret_cast<const uint4*>(slot)[g + 1];
   const uint32_t u[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
   const int q = sh >> 1, bits = (sh & 1) * 16;
@@ -272,7 +292,7 @@ __device__ __forceinline__ void load_shifted_bf16(const bf16* slot, int sh, int 
 #pragma unroll
   for (int j = 0; j < 4; ++j) w[j] = __funnelshift_r(pick_word(u, q, j), pick_word(u, q, j + 1), bits);
 #pragma unroll
-  for (int j = 0; j < 4; ++j) { v[2 * j] = bf16_lo(w[j]); v[2 * j + 1] = bf16_hi(w[j]); }
+  for (int j = 0; j < 4; ++j) { v[2 * j] = lo_f<T>(w[j]); v[2 * j + 1] = hi_f<T>(w[j]); }
 }
 __device__ __forceinline__ void load_shifted_f32(const float* slot, int sh, int g, float (&v)[8]) {
   const float4 a = reinterpret_cast<const float4*>(slot)[2 * g], b = reinterpret_cast<const float4*>(slot)[2 * g + 1],
@@ -281,6 +301,9 @@ __device__ __forceinline__ void load_shifted_f32(const float* slot, int sh, int 
 #pragma unroll
   for (int k = 0; k < 8; ++k) v[k] = sh == 0 ? f[k] : (sh == 1 ? f[k + 1] : (sh == 2 ? f[k + 2] : f[k + 3]));
 }
+__device__ __forceinline__ void load_shifted(const bf16* slot, int sh, int g, float (&v)[8]) { load_shifted_h(slot, sh, g, v); }
+__device__ __forceinline__ void load_shifted(const f16* slot, int sh, int g, float (&v)[8]) { load_shifted_h(slot, sh, g, v); }
+__device__ __forceinline__ void load_shifted(const float* slot, int sh, int g, float (&v)[8]) { load_shifted_f32(slot, sh, g, v); }
 
 // Body of kernel (3)'s default form.  UNALIGNED = false: V % 8 == 0, 16-byte aligned y / z / dy, dy pitch V (ld == V).
 // UNALIGNED = true (bf16 student logits, any V): y and z keep pitch V and any alignment; each row is fetched by bulk copies of
@@ -288,8 +311,10 @@ __device__ __forceinline__ void load_shifted_f32(const float* slot, int sh, int 
 // (the first / last row or two): that one is read with guarded plain loads.  Columns >= V are left out of the maxima, the
 // sums and the CE term.  dy has pitch ld (ld % 8 == 0, 16-byte aligned): 16-byte stores, columns V..roundup(V,8)-1 written
 // as exact zeros.
-template <typename TS, int NCH, bool TEMP4, bool UNALIGNED>
-__device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
+// TZ: the teacher logits' type (float, bf16 or f16).  A slot holds V * sizeof(TZ) teacher bytes; each 16-byte word of a
+// half-precision row gives 8 logits, widened exactly to fp32 in registers.
+template <typename TS, typename TZ, int NCH, bool TEMP4, bool UNALIGNED>
+__device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, const TZ* __restrict__ z, const int64_t* __restrict__ tgt,
                                                    long N, int V, long ld, float inv_temp, float temperature, float kd_coef, float w_ce,
                                                    const int* __restrict__ n_valid_ptr, TS* __restrict__ dy, float* __restrict__ row_kl,
                                                    float* __restrict__ row_ce, const int* __restrict__ steps, long rows_per_step, float kd_num) {
@@ -298,7 +323,7 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
   __shared__ float scratch[KDR_THREADS / 32 * 4];
   const int Vp = (V + 7) & ~7;
   // slot bytes: both multiples of 16; the unaligned form holds the enclosing ranges plus the word the last group reads past them
-  const size_t zbytes = UNALIGNED ? (size_t)(Vp + 4) * 4 : (size_t)V * 4;
+  const size_t zbytes = UNALIGNED ? (size_t)(Vp + 16 / sizeof(TZ)) * sizeof(TZ) : (size_t)V * sizeof(TZ);
   const size_t ybytes = UNALIGNED ? (size_t)(Vp + 8) * sizeof(TS) : (size_t)V * sizeof(TS);
   const size_t slot = zbytes + ybytes;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -344,7 +369,7 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
   int it = 0;
   for (long r = r0; r < n; r += stride, ++it) {
     const int sidx = it % KD_SLOTS; const uint32_t ph = (it / KD_SLOTS) & 1;
-    const float* zs = reinterpret_cast<const float*>(smem_raw + (size_t)sidx * slot);
+    const TZ* zs = reinterpret_cast<const TZ*>(smem_raw + (size_t)sidx * slot);
     const TS* ys = reinterpret_cast<const TS*>(smem_raw + (size_t)sidx * slot + zbytes);
     mbar_wait(&full_bar[sidx], ph);
     float yv[NCH][8], zv[NCH][8];
@@ -354,18 +379,18 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
 #pragma unroll
       for (int i = 0; i < NCH; ++i) {
         const int g = tid + i * KDR_THREADS;
-        if (i < NCH - 1 || g < groups) { RowS<TS>::load(ys + g * 8, yv[i]); RowS<float>::load(zs + g * 8, zv[i]); }
+        if (i < NCH - 1 || g < groups) { RowS<TS>::load(ys + g * 8, yv[i]); RowS<TZ>::load(zs + g * 8, zv[i]); }
       }
     } else {
       const TS* yr = y + r * (long)V;
-      const float* zr = z + r * (long)V;
+      const TZ* zr = z + r * (long)V;
       bulk = bulk_row(r);
       if (bulk) {
-        sy = (int)(((uintptr_t)yr & 15) / sizeof(TS)); sz = (int)(((uintptr_t)zr & 15) >> 2);
+        sy = (int)(((uintptr_t)yr & 15) / sizeof(TS)); sz = (int)(((uintptr_t)zr & 15) / sizeof(TZ));
 #pragma unroll
         for (int i = 0; i < NCH; ++i) {
           const int g = tid + i * KDR_THREADS;
-          if (i < NCH - 1 || g < groups) { load_shifted_bf16(ys, sy, g, yv[i]); load_shifted_f32(zs, sz, g, zv[i]); }
+          if (i < NCH - 1 || g < groups) { load_shifted(ys, sy, g, yv[i]); load_shifted(zs, sz, g, zv[i]); }
         }
       } else {
 #pragma unroll
@@ -375,7 +400,7 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
               const int c = g * 8 + j;
-              yv[i][j] = c < V ? to_f<TS>(yr[c]) : 0.f; zv[i][j] = c < V ? zr[c] : 0.f;
+              yv[i][j] = c < V ? to_f<TS>(yr[c]) : 0.f; zv[i][j] = c < V ? to_f<TZ>(zr[c]) : 0.f;
             }
           }
         }
@@ -397,8 +422,8 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
     const int t_idx = valid ? (int)t64 : -1;
     float y_tgt = 0.f, z_tgt = 0.f;
     if (valid) {
-      if (bulk) { y_tgt = to_f<TS>(ys[sy + t_idx]); z_tgt = zs[sz + t_idx]; }
-      else { y_tgt = to_f<TS>(y[r * (long)V + t_idx]); z_tgt = z[r * (long)V + t_idx]; }
+      if (bulk) { y_tgt = to_f<TS>(ys[sy + t_idx]); z_tgt = to_f<TZ>(zs[sz + t_idx]); }
+      else { y_tgt = to_f<TS>(y[r * (long)V + t_idx]); z_tgt = to_f<TZ>(z[r * (long)V + t_idx]); }
     }
     __syncthreads();                           // every thread has taken its groups out of the slot ...
     if (tid == 0 && r + KD_SLOTS * stride < n) issue(r + KD_SLOTS * stride, sidx);      // ... so a later row can land in it
@@ -490,24 +515,24 @@ __device__ __forceinline__ void kd_token_pipe_body(const TS* __restrict__ y, con
   }
 }
 
-template <typename TS, int NCH, bool TEMP4>
+template <typename TS, typename TZ, int NCH, bool TEMP4>
 __global__ void __launch_bounds__(KDR_THREADS, (NCH <= 3 ? 3 : (NCH <= 5 ? 2 : 1)))
-kd_token_loss_pipe_kernel(const TS* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
+kd_token_loss_pipe_kernel(const TS* __restrict__ y, const TZ* __restrict__ z, const int64_t* __restrict__ tgt,
                           long N, int V, float inv_temp, float temperature, float kd_coef, float w_ce, const int* __restrict__ n_valid_ptr,
                           TS* __restrict__ dy, float* __restrict__ row_kl, float* __restrict__ row_ce,
                           const int* __restrict__ steps, long rows_per_step, float kd_num) {
-  kd_token_pipe_body<TS, NCH, TEMP4, false>(y, z, tgt, N, V, V, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce,
+  kd_token_pipe_body<TS, TZ, NCH, TEMP4, false>(y, z, tgt, N, V, V, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce,
                                             steps, rows_per_step, kd_num);
 }
 
 // The form for bf16 rows of any length (V % 8 != 0 or unaligned logits) with dlogits of pitch ld (ld % 8 == 0).
-template <int NCH, bool TEMP4>
+template <typename TZ, int NCH, bool TEMP4>
 __global__ void __launch_bounds__(KDR_THREADS, (NCH <= 3 ? 3 : (NCH <= 5 ? 2 : 1)))
-kd_token_loss_pipe_unaligned_kernel(const bf16* __restrict__ y, const float* __restrict__ z, const int64_t* __restrict__ tgt,
+kd_token_loss_pipe_unaligned_kernel(const bf16* __restrict__ y, const TZ* __restrict__ z, const int64_t* __restrict__ tgt,
                                     long N, int V, long ld, float inv_temp, float temperature, float kd_coef, float w_ce,
                                     const int* __restrict__ n_valid_ptr, bf16* __restrict__ dy, float* __restrict__ row_kl,
                                     float* __restrict__ row_ce, const int* __restrict__ steps, long rows_per_step, float kd_num) {
-  kd_token_pipe_body<bf16, NCH, TEMP4, true>(y, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce,
+  kd_token_pipe_body<bf16, TZ, NCH, TEMP4, true>(y, z, tgt, N, V, ld, inv_temp, temperature, kd_coef, w_ce, n_valid_ptr, dy, row_kl, row_ce,
                                              steps, rows_per_step, kd_num);
 }
 
@@ -543,10 +568,12 @@ __global__ void count_valid_kernel(const int64_t* __restrict__ tgt, long n, int 
 }
 // Kernel (4).  blockIdx < n_feat_blocks : feature KD for sample b (256 threads);  above : hidden KD, one warp per
 // (t,b) row.  Gradients already carry beta / gamma; loss partials go to workspace for the finalize kernel.
-template <typename TF, typename TH>
+// TZ: the teacher hidden states' type (float, bf16 or f16), widened exactly to fp32 on load.  The teacher features ft stay fp32:
+// they are the projector's output, and dft flows back into it.
+template <typename TF, typename TH, typename TZ>
 __global__ void __launch_bounds__(256)
 aux_loss_kernel(const TF* __restrict__ fs, const float* __restrict__ ft, int n_feat_blocks /*B or 0*/, int B, int Ss, int St, int E,
-                const TH* __restrict__ hs, const float* __restrict__ ht, int n_hid_rows /*Th*B*/, int n_all_rows /*T*B*/,
+                const TH* __restrict__ hs, const TZ* __restrict__ ht, int n_hid_rows /*Th*B*/, int n_all_rows /*T*B*/,
                 int H, int Th, float beta, float gamma,
                 float* __restrict__ dfs, float* __restrict__ dft, TH* __restrict__ dhs,
                 float* __restrict__ feat_part /*B*2*/, float* __restrict__ hid_part /*n_hid_rows*2*/,
@@ -680,7 +707,7 @@ aux_loss_kernel(const TF* __restrict__ fs, const float* __restrict__ ft, int n_f
       if (row < n_hid_rows && lane == 0) { hid_part[row * 2] = 0.f; hid_part[row * 2 + 1] = 0.f; }
       return;
     }
-    const float* t = ht + row * H;
+    const TZ* t = ht + row * H;
     float sq = 0.f, dot = 0.f, ns = 0.f, nt = 0.f;
     constexpr int HC = 2;                                   // H <= 512: the row stays in registers between the two passes
     const bool in_regs = (H & 7) == 0 && H <= HC * 256;
@@ -690,13 +717,13 @@ aux_loss_kernel(const TF* __restrict__ fs, const float* __restrict__ ft, int n_f
       for (int c = 0; c < HC; ++c) {
         const int ch = lane + 32 * c;
         if (ch * 8 < H) {
-          Vec8<TH>::load(s + ch * 8, sa[c]); Vec8<float>::load(t + ch * 8, tc[c]);
+          Vec8<TH>::load(s + ch * 8, sa[c]); Vec8<TZ>::load(t + ch * 8, tc[c]);
 #pragma unroll
           for (int k = 0; k < 8; ++k) { const float a = sa[c][k], cc = tc[c][k], df = a - cc; sq += df * df; dot += a * cc; ns += a * a; nt += cc * cc; }
         }
       }
     } else {
-      for (int h = lane; h < H; h += 32) { const float a = to_f<TH>(s[h]), c = t[h]; const float df = a - c; sq += df * df; dot += a * c; ns += a * a; nt += c * c; }
+      for (int h = lane; h < H; h += 32) { const float a = to_f<TH>(s[h]), c = to_f<TZ>(t[h]); const float df = a - c; sq += df * df; dot += a * c; ns += a * a; nt += c * c; }
     }
     sq = warp_sum(sq); dot = warp_sum(dot); ns = warp_sum(ns); nt = warp_sum(nt);
     const float eps = 1e-12f;
@@ -721,7 +748,7 @@ aux_loss_kernel(const TF* __restrict__ fs, const float* __restrict__ ft, int n_f
         }
       } else {
         for (int h = lane; h < H; h += 32) {
-          const float a = to_f<TH>(s[h]), c = t[h];
+          const float a = to_f<TH>(s[h]), c = to_f<TZ>(t[h]);
           d[h] = from_f<TH>(c_mse * (a - c) - c_cos * (c * inv_norm - cosv * a / nse));
         }
       }

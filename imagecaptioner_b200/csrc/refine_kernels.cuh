@@ -12,10 +12,22 @@ __device__ __forceinline__ float4 ld_nc_f4(const float4* p) {
   asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
   return r;
 }
-template <typename T>
-__global__ void __launch_bounds__(256) cast_f32_kernel(const float* __restrict__ in, T* __restrict__ out, long n) {
+// Converting copy in -> out.  TI = float (the general case), or bf16 / f16 (teacher features handed to the projector in half
+// precision: 16-byte loads of 8 elements, widened exactly to fp32 and rounded to T like an fp32 input would be).
+template <typename T, typename TI = float>
+__global__ void __launch_bounds__(256) cast_f32_kernel(const TI* __restrict__ in, T* __restrict__ out, long n) {
   const long n8 = ((((uintptr_t)in) % 16 == 0) && (((uintptr_t)out) % 16 == 0)) ? (n >> 3) : 0;
   const long stride = (long)gridDim.x * blockDim.x;
+  if constexpr (sizeof(TI) == 2) {
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += stride) {
+      float v[8];
+      Vec8<TI>::load(in + i * 8, v);
+      if (sizeof(T) == 2) *reinterpret_cast<uint4*>(out + i * 8) = make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
+      else { reinterpret_cast<float4*>(out + i * 8)[0] = make_float4(v[0], v[1], v[2], v[3]); reinterpret_cast<float4*>(out + i * 8)[1] = make_float4(v[4], v[5], v[6], v[7]); }
+    }
+    for (long i = n8 * 8 + (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = from_f<T>(to_f<TI>(in[i]));
+    return;
+  }
   // two 8-element groups per thread and iteration, all four 16-byte loads issued before the stores
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += 2 * stride) {
     const long i2 = i + stride;

@@ -17,6 +17,11 @@ Variable-length batches (``max_steps=T_cap``): the reference's loader pads every
 from batch to batch.  The graph is then captured once with (T_cap, B, ...) buffers and a device step count; ``load()`` takes any
 batch with 1 <= T <= T_cap and the replay computes exactly the loss, gradients and update of that T-step batch (padding the batch
 to T_cap instead would not: token KD is a mean over all T*B rows and hidden KD a mean over steps).
+
+Half-precision teacher outputs: the static buffers take the example batch's dtypes.  With bf16 / fp16 teacher_logits,
+teacher_features and teacher_hiddens in the example, the captured kernels read them in that precision and widen them exactly to
+fp32 in registers (the same loss parts and gradients as for their fp32 upcasts), the graph holds no conversion of them, and load()
+copies half the teacher bytes.
 """
 from __future__ import annotations
 

@@ -35,6 +35,10 @@
  *   - Return 0 on success, a negative B2C_E* code otherwise; message via b2c_last_error() (thread local).
  *   - `dtype` selects the precision mode: B2C_F32 (parity mode: fp32 storage + FFMA contractions) or
  *     B2C_BF16 (throughput mode: bf16 storage, tcgen05 contractions, fp32 accumulation and cell state).
+ *   - `teacher_dtype` (the *_teacher entry points) is the element type of the teacher's outputs: B2C_F32, B2C_BF16 or B2C_F16, as
+ *     a teacher run under autocast or a half-precision cache of its outputs leaves them.  The kernels widen half-precision values
+ *     to fp32 exactly as they load them, so the results are bit-identical to those for the same values given as fp32.
+ *     Each entry point without the suffix is its _teacher form with teacher_dtype = B2C_F32.
  *   - Time-major layouts like the reference: captions/targets (T,B) int64, logits (T,B,V).
  *   - There is no CPU fallback.
  */
@@ -52,7 +56,7 @@ extern "C" {
 #define B2C_MAX_LAYERS 4
 
 enum { B2C_OK = 0, B2C_EINVAL = -1, B2C_EARCH = -2, B2C_ECUDA = -3, B2C_ENOMEM = -4 };
-enum { B2C_F32 = 0, B2C_BF16 = 1 };
+enum { B2C_F32 = 0, B2C_BF16 = 1, B2C_F16 = 2 };      /* B2C_F16: a teacher_dtype only, never a compute dtype */
 enum { B2C_WS_TRAIN = 0, B2C_WS_DECODE = 1, B2C_WS_ATTN = 2, B2C_WS_REFINE = 3, B2C_WS_PROJ = 4 };
 
 /* B batch (per GPU), T decode steps, S image tokens (49), E embed, H hidden, L LSTM layers, V vocab. */
@@ -120,6 +124,11 @@ int b2c_decoder_forward_eval(const B2CShape* shape, const B2CParams* params, con
                              const float* teacher_logits, const int64_t* targets, float temperature,
                              void* hidden_top, float* attn_w, float* row_kl, float* row_ce, int32_t* argmax_out,
                              void* workspace, size_t ws_bytes, int dtype, void* stream);
+/* b2c_decoder_forward_eval on teacher logits of element type teacher_dtype: the epilogue streams them in that type. */
+int b2c_decoder_forward_eval_teacher(const B2CShape* shape, const B2CParams* params, const void* feats, const int64_t* captions,
+                                     const void* teacher_logits, int teacher_dtype, const int64_t* targets, float temperature,
+                                     void* hidden_top, float* attn_w, float* row_kl, float* row_ce, int32_t* argmax_out,
+                                     void* workspace, size_t ws_bytes, int dtype, void* stream);
 
 /* The part of b2c_decoder_forward that does not read the image features: operand packing (compute-type copies of the weights,
  * attention_combine folded into layer 0), the embedding rows of `captions`, the time-batched embedding half of layer 0's
@@ -235,6 +244,10 @@ typedef struct B2CProjGrads { float *w, *b, *ln_w, *ln_b; } B2CProjGrads;
 /* x (B,St,Et) fp32 (teacher features, no gradient) -> out (B,So,Es) fp32 */
 int b2c_projector_forward(const B2CShape* shape, const B2CProjParams* params, const float* x, float* out,
                           void* workspace, size_t ws_bytes, int dtype, const B2CDropout* dropout, void* stream);
+/* b2c_projector_forward on teacher features x of element type teacher_dtype (in either compute mode).  The backward is unchanged:
+ * it reads the compute-type copy of x the forward keeps in the workspace. */
+int b2c_projector_forward_teacher(const B2CShape* shape, const B2CProjParams* params, const void* x, int teacher_dtype, float* out,
+                                  void* workspace, size_t ws_bytes, int dtype, const B2CDropout* dropout, void* stream);
 /* dout (B,So,Es) fp32 -> grads (fp32, overwritten) */
 int b2c_projector_backward(const B2CShape* shape, const B2CProjParams* params, const float* dout, const B2CProjGrads* grads,
                            void* workspace, size_t ws_bytes, int dtype, const B2CDropout* dropout, void* stream);
@@ -270,11 +283,23 @@ int b2c_kd_token_loss_steps(const void* student_logits, const float* teacher_log
                             const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype,
                             const int32_t* steps, int64_t rows_per_step, void* stream);
 
+/* The token pass on teacher logits of element type teacher_dtype: the arguments of b2c_kd_token_loss_steps, where steps == NULL is a
+ * batch of all N rows and ld_dlogits == V a contiguous dlogits, so this covers b2c_kd_token_loss, _pitched and _steps. */
+int b2c_kd_token_loss_teacher(const void* student_logits, const void* teacher_logits, int teacher_dtype, const int64_t* targets,
+                              int64_t N, int32_t V, float temperature, float alpha, float w_ce, float ce_mult,
+                              const int32_t* n_valid, void* dlogits, int64_t ld_dlogits, float* row_kl, float* row_ce, int dtype,
+                              const int32_t* steps, int64_t rows_per_step, void* stream);
+
 /* Evaluation form of the token pass (validate_student_model, src/train_student_kd.py:29-86): the same per-row KL and CE partials,
  * NO gradient, plus (argmax_out != NULL) the teacher-forced prediction argmax_v student_logits[r, v] of every row (lowest index on
  * ties, like torch.argmax) from the same read of the logits -- `student_logits.argmax(dim=-1)` (:74) without a second pass. */
 int b2c_kd_token_eval(const void* student_logits, const float* teacher_logits, const int64_t* targets, int64_t N, int32_t V,
                       float temperature, const int32_t* n_valid, float* row_kl, float* row_ce, int32_t* argmax_out, int dtype, void* stream);
+
+/* b2c_kd_token_eval on teacher logits of element type teacher_dtype. */
+int b2c_kd_token_eval_teacher(const void* student_logits, const void* teacher_logits, int teacher_dtype, const int64_t* targets, int64_t N,
+                              int32_t V, float temperature, const int32_t* n_valid, float* row_kl, float* row_ce, int32_t* argmax_out,
+                              int dtype, void* stream);
 
 /* compute_bleu_score (src/distillation_utils.py:398-409) for every sample of a batch on the device: predicted (T,B) int32,
  * targets (T,B) int64 -> bleu_out (B) = |set(pred) & set(target)| / |set(target)| over token ids outside {PAD=0, START=1, END=2}
@@ -299,6 +324,13 @@ int b2c_aux_loss_steps(const void* feats_s, const float* feats_t, int32_t B, int
                        const void* hid_s, const float* hid_t, int32_t T, int32_t Th, int32_t H,
                        float beta, float gamma, float* dfeats_s, float* dfeats_t, void* dhid_s,
                        float* feat_part, float* hid_part, int dtype, int feat_dtype, const int32_t* steps, void* stream);
+
+/* b2c_aux_loss_steps (steps may be NULL: all steps) with teacher hidden states hid_t of element type hid_t_dtype.  feats_t stays
+ * fp32: it is the projector's output, and dfeats_t flows back into the projector. */
+int b2c_aux_loss_teacher(const void* feats_s, const float* feats_t, int32_t B, int32_t Ss, int32_t St, int32_t E,
+                         const void* hid_s, const void* hid_t, int hid_t_dtype, int32_t T, int32_t Th, int32_t H,
+                         float beta, float gamma, float* dfeats_s, float* dfeats_t, void* dhid_s,
+                         float* feat_part, float* hid_part, int dtype, int feat_dtype, const int32_t* steps, void* stream);
 
 /* out5 = { total, ce, token_kd, feature_kd, hidden_kd } (device, fp32); fixed-order fp64 reduction. */
 int b2c_loss_finalize(const float* row_kl, const float* row_ce, int64_t N, const int32_t* n_valid, float ce_mult,
